@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the VBQ rate-distortion quantization step (BASELINE.json metric: coordinates quantized / second).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU)
 
 A "step" is one pass of the hot path over one batch: the Kodak-shaped bls2017 latent batch of BASELINE.json
@@ -290,6 +290,18 @@ def _time_steps(fn, steps, warmup, barrier, finish=None):
     return ev[0].elapsed_time(ev[1])
 
 
+def dump_outputs(directory, **arrays):
+    """Write each device tensor as <directory>/<name>.npy, integers as float32 (exact: code indices are < 2^24) and
+    floats at their own precision.  The headline outputs come to 2 x 27 MiB + 32 bytes, so they are written in full
+    rather than sampled."""
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        if a.dtype.kind != "f":
+            a = a.astype(np.float32)
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -338,7 +350,7 @@ def run_ours(args, rank, world, local_rank):
                                     qidx=b["qidx"], bits=b["bits"], totals=buckets[k][e], flags=args.flags,
                                     graph=args.graph) for b in sets] for e in range(every)] for k in range(n_buckets)]
         pending = [None] * n_buckets
-        last = {"i": -1}
+        last = {"i": -1, "totals": None}
 
         def step(i):
             last["i"] = i
@@ -346,7 +358,7 @@ def run_ours(args, rank, world, local_rank):
             if e == 0 and pending[k] is not None:
                 pending[k].wait()
                 pending[k] = None
-            plans[k][e][i % n_sets].run()
+            last["totals"] = plans[k][e][i % n_sets].run()
             if world > 1 and e == every - 1:
                 pending[k] = sharding.all_reduce_totals(buckets[k], async_op=True)
 
@@ -360,7 +372,7 @@ def run_ours(args, rank, world, local_rank):
                 if i >= 0 and i % every != every - 1:
                     sharding.all_reduce_totals(buckets[(i // every) % n_buckets])
                     last["i"] = -1
-        return step, drain
+        return step, drain, last
 
     # N > 1, headline: NO collective launch at all — while call i runs, an idle lane of its kernel writes the totals of call
     # i-1 into every rank's inbox over NVLink and collects (waits for + adds in rank order) the all-reduced totals of call
@@ -398,20 +410,24 @@ def run_ours(args, rank, world, local_rank):
         step, drain, peer, glob, local = headline_peer()
         variants["headline"] = "peer inboxes over NVLink: call i delivers the totals of call i-1 and collects those of call i-3 while it runs"
     else:
-        step, drain = headline(1)
+        step, drain, last = headline(1)
     with ClockSampler(local_rank) as clocks:
         total_ms = max_over_ranks(_time_steps(step, args.steps, args.warmup, barrier, drain))
     value = COORDS * world * args.steps / (total_ms * 1e-3)
     host_issue_us = _time_steps.host_issue_us
+    last_k = args.warmup + args.steps - 1      # call index of the last timed step
     if world > 1:
         # the exchanged totals are the NCCL all-reduce of the local ones (last call of the timed region)
         torch.cuda.synchronize()
-        last_k = (args.warmup + args.steps - 1)
         want = sharding.all_reduce_totals(local[last_k % n_sets].clone())
         got = glob[(args.steps - 1) % 8]
         assert torch.allclose(got, want, rtol=1e-12), (got, want)
+    if args.dump_outputs and rank == 0:
+        out = sets[last_k % n_sets]
+        dump_outputs(args.dump_outputs, qidx=out["qidx"], bits=out["bits"], totals=got if world > 1 else last["totals"])
+    if world > 1:
         for every in (1, n_sets):       # for comparison: the same steps with NCCL all-reduces (147 CTAs + 1 SM for NCCL)
-            stepn, drainn = headline(every)
+            stepn, drainn, _ = headline(every)
             msn = max_over_ranks(_time_steps(stepn, args.steps, args.warmup, barrier, drainn))
             variants["nccl_collective_every_%d" % every] = {"value": COORDS * world * args.steps / (msn * 1e-3), "unit": UNIT}
 
@@ -646,7 +662,12 @@ def main():
     ap.add_argument("--headline-only", action="store_true", help="skip the `corrected` and `configs` sections")
     ap.add_argument("--graph", action="store_true", help="replay one CUDA graph per step instead of the prebound eager "
                     "call (the eager launches overlap through programmatic dependent launch and measure faster)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned "
+                    "(rank 0: qidx, bits as float32 (1, rows, C); totals float64 (1, 4)) as DIR/<name>.npy; the inputs "
+                    "are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl ours and --steps >= 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
