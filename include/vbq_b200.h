@@ -236,7 +236,45 @@ int vbq_unpack_indices(const unsigned *d_words, long long n, int N, int *d_qidx,
 int vbq_symbol_histogram(const int *d_qidx, long long rows, int C, int N, unsigned long long *d_counts,
                          void *stream);
 
-/* ---- stand-alone operator forms ------------------------------------------------------------------------------- */
+/* ---- entropy coding of the sorted quantile indices: interleaved rANS (DESIGN.md §10) ------------------------------ */
+
+/* A PLANE is (items, item_rows, C) int32 symbols q in [0, Q), Q = 2^(N+1)-1, N <= 10, coded with one frequency table per
+ * (plane, channel) whose entries are >= 1 and sum to 2^prob_bits (12 <= prob_bits <= 16, Q <= 2^prob_bits).  Tables are
+ * passed as d_cum (n_planes, C, Q) uint16: cum[s] = f[0] + ... + f[s-1], with an implicit cum[Q] = 2^prob_bits.
+ * A GROUP is (item, segment of seg_rows rows, 32-channel group g); lane j of group g codes channel 32g+j over the
+ * segment's rows in increasing order.  The coder has a 32-bit state in [2^16, 2^32) and emits 16-bit words, at most one
+ * per symbol and lane.  The DECODER defines the format: read the active lanes' initial states (two words each, low half
+ * first); for each row and each active lane in increasing order: slot = x & (2^P-1), s the symbol with
+ * cum[s] <= slot < cum[s]+f[s], x = f[s] (x >> P) + slot - cum[s], and if x < 2^16 then x = (x << 16) | the group's
+ * next word.  After the last row every state is 2^16 and every word of the group has been read.
+ * PAYLOAD (uint16 words): per plane, the group end offset table (one uint32 per group as two words, low half first, in
+ * words from the start of the plane's group data; groups in (item, segment, channel group) order), then the groups
+ * (states, then words).  The planes' payloads follow each other.
+ *
+ * vbq_rans_workspace_bytes / vbq_rans_payload_bound: the encoder's workspace and the worst-case payload in bytes for a
+ * shape (every lane emitting a word per row); -1 for a bad shape.
+ * vbq_rans_encode codes n_planes planes (d_qidx (n_planes, items, item_rows, C)) in one launch into d_payload (at least
+ * vbq_rans_payload_bound bytes) and leaves the payload size in bytes in the device scalar *d_payload_size; no host
+ * synchronisation.  *d_status (device int) becomes nonzero (1) if a symbol was outside [0, Q).
+ * vbq_rans_decode reads groups of d_payload (payload_words words) at the word ranges d_group_bounds
+ * (n_planes * groups, 2) int64 [start, end), which the caller takes from the offset tables, and writes any of d_qidx
+ * (int32) and d_zhat (float32 = d_code_points[c][q], the caller's (C, Q) ascending code points) of shape
+ * (n_planes, items, item_rows, C).  A group never reads outside its range; *d_status (device int) receives 1 if a
+ * group ran out of words, 2 if a final state differs from 2^16 or words are left over, 4 if a range or initial state
+ * is invalid (0 = every group decoded and passed the integrity check).
+ * Status codes: VBQ_ERR_BAD_DEPTH for N > 10, VBQ_ERR_BAD_SHAPE for a bad shape or prob_bits. */
+long long vbq_rans_workspace_bytes(int n_planes, int items, long long item_rows, int C, long long seg_rows);
+long long vbq_rans_payload_bound(int n_planes, int items, long long item_rows, int C, long long seg_rows);
+int vbq_rans_encode(const int *d_qidx, int n_planes, int items, long long item_rows, int C, long long seg_rows, int N,
+                    int prob_bits, const unsigned short *d_cum, unsigned short *d_payload, long long payload_bytes,
+                    long long *d_payload_size, int *d_status, void *d_workspace, long long workspace_bytes,
+                    void *stream);
+int vbq_rans_decode(const unsigned short *d_payload, long long payload_words, const long long *d_group_bounds,
+                    int n_planes, int items, long long item_rows, int C, long long seg_rows, int N, int prob_bits,
+                    const unsigned short *d_cum, const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status,
+                    void *stream);
+
+/* ---- stand-alone operator forms------------------------------------------------------------------------------- */
 
 /* ChannelwisePriorCDFQuantizer.get_all_N_bit_intervals (quantizer.py:65-80): d_mu (rows, C) -> d_left, d_right
  * (C, N+1, rows): at every bit depth the largest code point below mu and the smallest one >= mu, with the edge

@@ -76,6 +76,10 @@ SIGNATURES = {
     "vbq_pack_indices": (_i, [_p, _ll, _i, _p, _p]),
     "vbq_unpack_indices": (_i, [_p, _ll, _i, _p, _p]),
     "vbq_symbol_histogram": (_i, [_p, _ll, _i, _i, _p, _p]),
+    "vbq_rans_workspace_bytes": (_ll, [_i, _i, _ll, _i, _ll]),
+    "vbq_rans_payload_bound": (_ll, [_i, _i, _ll, _i, _ll]),
+    "vbq_rans_encode": (_i, [_p, _i, _i, _ll, _i, _ll, _i, _i, _p, _p, _ll, _p, _p, _p, _ll, _p]),
+    "vbq_rans_decode": (_i, [_p, _ll, _p, _i, _i, _ll, _i, _ll, _i, _i, _p, _p, _p, _p, _p, _p]),
 }
 
 _lib = None

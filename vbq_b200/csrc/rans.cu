@@ -1,0 +1,419 @@
+// rans.cu — entropy coding of the sorted quantile indices: a 32-lane interleaved rANS coder with one frequency table
+// per (plane, channel).  The reference stops at ideal code lengths (-log2 of the fitted frequency, quantizer.py:226-228);
+// this turns the symbols of the search kernels into bytes and the bytes back into symbols and z_hat.
+//
+// Stream layout (normative; tests/rans_reference.py restates it in NumPy):
+//   * a plane is (items, item_rows, C) symbols q in [0, Q), Q = 2^(N+1)-1; a GROUP is (item, row segment of seg_rows
+//     rows, 32-channel group g); lane j of group g codes channel 32g+j (only lanes with 32g+j < C exist) over the
+//     segment's rows in increasing order;
+//   * rANS with a 32-bit state x in [2^16, 2^32), 16-bit words, probabilities of P = prob_bits <= 16 bits: a symbol
+//     moves at most one word per lane, so a warp finds every lane's word offset with one ballot and popc;
+//   * the decoder defines the format: read the active lanes' initial states (two words each, low half first); for each
+//     row, for each active lane in increasing order: slot = x & (2^P-1), s the symbol with cum[s] <= slot < cum[s]+f[s],
+//     x = f[s] (x >> P) + slot - cum[s], and if x < 2^16 then x = (x << 16) | next word of the group.  After the last
+//     row every state equals 2^16 and every word of the group has been read;
+//   * the payload of a plane is its group end offset table (uint32 per group, in 16-bit words from the start of the
+//     plane's group data, groups in (item, segment, channel group) order) followed by the groups, each its states and
+//     then its words.  The payload of a call is its planes' payloads back to back.
+#include "common.h"
+
+namespace {
+
+constexpr int kRansWarps = 8;
+constexpr unsigned kRansL = 1u << 16;
+constexpr int kRansBuckets = 256;   // coarse decode index: slot >> (P - 8) -> first candidate symbol
+
+struct RansShape {
+    int n_planes, items, C, CG, P, Q;
+    long long item_rows, seg_rows, n_segs, G;   // G = groups per plane
+};
+
+int rans_shape(const char *fn, int n_planes, int items, long long item_rows, int C, long long seg_rows, int N,
+               int prob_bits, RansShape *s) {
+    if (n_planes < 1 || n_planes > 65535 || items < 0 || item_rows < 0 || C < 1 || C > 32 * 65535 || seg_rows < 1)
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "%s: n_planes=%d items=%d item_rows=%lld C=%d seg_rows=%lld", fn, n_planes,
+                        items, item_rows, C, seg_rows);
+    if (N < 0 || N > 10) return vbq_fail(VBQ_ERR_BAD_DEPTH, "%s: N=%d (the coder holds N <= 10)", fn, N);
+    const int Q = (1 << (N + 1)) - 1;
+    if (prob_bits < 12 || prob_bits > 16 || Q > (1 << prob_bits))
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "%s: prob_bits=%d (12..16 with Q=%d <= 2^prob_bits)", fn, prob_bits, Q);
+    s->n_planes = n_planes; s->items = items; s->C = C; s->CG = (C + 31) / 32; s->P = prob_bits; s->Q = Q;
+    s->item_rows = item_rows; s->seg_rows = seg_rows;
+    s->n_segs = (item_rows + seg_rows - 1) / seg_rows;
+    s->G = (long long)items * s->n_segs * s->CG;
+    // worst-case words of a plane: every lane emits a word on every row, plus its state, plus the offset table
+    const double words = (double)items * s->n_segs * C * ((double)seg_rows + 2.0) + 2.0 * (double)s->G;
+    if (words >= 4294967296.0 || (double)items * s->n_segs >= 2147483647.0 * kRansWarps ||
+        (double)n_planes * s->G >= 2147483647.0)
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "%s: a plane of %d x %lld x %d symbols in segments of %lld rows exceeds "
+                        "the 32-bit offset table", fn, items, item_rows, C, seg_rows);
+    return VBQ_OK;
+}
+
+long long rans_plane_scratch_words(const RansShape &s) {
+    return (long long)s.items * s.n_segs * s.C * (s.seg_rows + 2);
+}
+
+long long align256(long long b) { return (b + 255) & ~255ll; }
+
+// The 32 channels of a group are consecutive rows of the (n_planes, C, Q) cum table: one linear copy.
+__device__ __forceinline__ void load_group_cum(unsigned short *sh_cum, const unsigned short *__restrict__ cum,
+                                               int plane, int cg, const RansShape &s) {
+    const int nact = min(32, s.C - 32 * cg);
+    const unsigned short *src = cum + ((size_t)plane * s.C + 32 * cg) * s.Q;
+    const int n = nact * s.Q;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) sh_cum[i] = __ldg(src + i);
+}
+
+__device__ __forceinline__ unsigned lanemask_lt() {
+    unsigned m;
+    asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
+    return m;
+}
+
+constexpr int kEncBlock = 16;   // rows whose symbols are loaded together (the next block's loads overlap the coding)
+
+// One warp per (item, segment) of the CTA's channel group: rows last to first, lanes high to low, words written back
+// to front into the group's scratch region [base, base + nact (seg_rows + 2)).
+__global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_encode_kernel(const int *__restrict__ qidx,
+                                                                         const unsigned short *__restrict__ cum,
+                                                                         RansShape s,
+                                                                         unsigned short *__restrict__ scratch,
+                                                                         long long *__restrict__ sizes,
+                                                                         int *__restrict__ status) {
+    extern __shared__ unsigned short sh_cum[];   // [nact][Q]
+    const int cg = blockIdx.y, plane = blockIdx.z;
+    load_group_cum(sh_cum, cum, plane, cg, s);
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const long long unit = (long long)blockIdx.x * kRansWarps + (threadIdx.x >> 5);   // item * n_segs + segment
+    if (unit >= (long long)s.items * s.n_segs) return;
+    const int item = (int)(unit / s.n_segs);
+    const long long r0 = (unit % s.n_segs) * s.seg_rows;
+    const long long len = min(s.seg_rows, s.item_rows - r0);
+    const int nact = min(32, s.C - 32 * cg);
+    const bool active = lane < nact;
+    const int c = 32 * cg + lane;
+    const int *src = qidx + (((long long)plane * s.items + item) * s.item_rows + r0) * s.C + c;
+    const unsigned short *tab = sh_cum + (active ? lane : 0) * s.Q;
+    const unsigned top = 1u << s.P;
+    const int fshift = 32 - s.P;
+    const long long base = ((long long)plane * s.items * s.n_segs + unit) * s.C * (s.seg_rows + 2) +
+                           32ll * cg * (s.seg_rows + 2);
+    const long long end = base + (long long)nact * (s.seg_rows + 2);
+    long long pos = end;
+    unsigned x = kRansL;
+    int bad = 0;
+    const unsigned lt = lanemask_lt();
+
+    int cur[kEncBlock], nxt[kEncBlock];
+#pragma unroll
+    for (int k = 0; k < kEncBlock; ++k) {
+        const long long t = len - 1 - k;
+        cur[k] = (active && t >= 0) ? __ldg(src + t * s.C) : 0;
+    }
+    for (long long t0 = len - 1; t0 >= 0; t0 -= kEncBlock) {
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) {
+            const long long t = t0 - kEncBlock - k;
+            nxt[k] = (active && t >= 0) ? __ldg(src + t * s.C) : 0;
+        }
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) {
+            if (t0 - k < 0) break;                         // warp-uniform
+            int sym = cur[k];
+            if (sym < 0 || sym >= s.Q) { bad = 1; sym = 0; }
+            const unsigned lo = tab[sym];
+            const unsigned f = (sym + 1 < s.Q ? (unsigned)tab[sym + 1] : top) - lo;
+            const bool emit = active && (unsigned long long)x >= ((unsigned long long)f << fshift);
+            const unsigned mask = __ballot_sync(0xffffffffu, emit);
+            pos -= __popc(mask);
+            if (emit) {
+                scratch[pos + __popc(mask & lt)] = (unsigned short)(x & 0xffffu);
+                x >>= 16;
+            }
+            if (active) x = ((x / f) << s.P) + (x % f) + lo;
+        }
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) cur[k] = nxt[k];
+    }
+    pos -= 2 * nact;
+    if (active) {
+        scratch[pos + 2 * lane] = (unsigned short)(x & 0xffffu);
+        scratch[pos + 2 * lane + 1] = (unsigned short)(x >> 16);
+    }
+    const long long g = (((long long)plane * s.items * s.n_segs + unit) * s.CG + cg);
+    if (lane == 0) sizes[g] = end - pos;
+    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, 1);
+}
+
+// Block-wide inclusive sum of one value per thread (blockDim.x a multiple of 32, at most 1024).
+__device__ long long block_inclusive_sum(long long v, long long *sh_warp, long long *total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const long long u = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v += u;
+    }
+    if (lane == 31) sh_warp[warp] = v;
+    __syncthreads();
+    if (warp == 0) {
+        long long w = lane < nw ? sh_warp[lane] : 0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const long long u = __shfl_up_sync(0xffffffffu, w, o);
+            if (lane >= o) w += u;
+        }
+        if (lane < nw) sh_warp[lane] = w;
+    }
+    __syncthreads();
+    if (warp > 0) v += sh_warp[warp - 1];
+    *total = sh_warp[nw - 1];
+    __syncthreads();
+    return v;
+}
+
+// One CTA: exclusive scan of the group sizes of every plane -> each group's destination, the planes' offset tables
+// and the payload size in bytes.
+__global__ void __launch_bounds__(1024) vbq_rans_scan_kernel(const long long *__restrict__ sizes,
+                                                            long long *__restrict__ dst, int n_planes, long long G,
+                                                            unsigned short *__restrict__ out,
+                                                            long long *__restrict__ out_bytes) {
+    __shared__ long long sh_warp[32];
+    long long plane_start = 0;   // in words
+    for (int p = 0; p < n_planes; ++p) {
+        long long carry = 0;
+        for (long long c0 = 0; c0 < G; c0 += blockDim.x) {
+            const long long i = c0 + threadIdx.x;
+            const long long v = i < G ? sizes[(long long)p * G + i] : 0;
+            long long chunk;
+            const long long incl = block_inclusive_sum(v, sh_warp, &chunk);
+            if (i < G) {
+                const unsigned long long e = (unsigned long long)(carry + incl);
+                out[plane_start + 2 * i] = (unsigned short)(e & 0xffffu);
+                out[plane_start + 2 * i + 1] = (unsigned short)(e >> 16);
+                dst[(long long)p * G + i] = plane_start + 2 * G + carry + incl - v;
+            }
+            carry += chunk;
+        }
+        plane_start += 2 * G + carry;
+    }
+    if (threadIdx.x == 0) *out_bytes = 2 * plane_start;
+}
+
+// One CTA per group: move its words from the end of its scratch region to their place in the payload.
+__global__ void vbq_rans_compact_kernel(const unsigned short *__restrict__ scratch, const long long *__restrict__ sizes,
+                                        const long long *__restrict__ dst, RansShape s,
+                                        unsigned short *__restrict__ out) {
+    const long long g = blockIdx.x;                  // (plane, item, segment, channel group)
+    const int cg = (int)(g % s.CG);
+    const long long unit = g / s.CG;                 // (plane, item, segment)
+    const int nact = min(32, s.C - 32 * cg);
+    const long long end = unit * s.C * (s.seg_rows + 2) + (32ll * cg + nact) * (s.seg_rows + 2);
+    const long long n = sizes[g];
+    const unsigned short *src = scratch + end - n;
+    unsigned short *d = out + dst[g];
+    for (long long i = threadIdx.x; i < n; i += blockDim.x) d[i] = src[i];
+}
+
+constexpr int kDecBlock = 8;   // rows per unrolled block; z_hat gathers of a block are stored one block later
+
+__device__ __forceinline__ unsigned short ld_word(const unsigned short *__restrict__ w, long long i, long long end) {
+    return i < end ? __ldg(w + i) : (unsigned short)0;
+}
+
+// Same CTA layout as the encoder.  Shared memory: the group's cum tables [nact][Q] and the coarse index [32][257].
+// A warp keeps the next 128 words of its group in registers (4 windows of 32, one word per lane) and reads each row's
+// words with shuffles; a window is refilled 64..96 words before it is needed.
+__global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_decode_kernel(const unsigned short *__restrict__ words,
+                                                                         long long n_words,
+                                                                         const long long *__restrict__ bounds,
+                                                                         const unsigned short *__restrict__ cum,
+                                                                         RansShape s,
+                                                                         const float *__restrict__ code_points,
+                                                                         int *__restrict__ qidx,
+                                                                         float *__restrict__ zhat,
+                                                                         int *__restrict__ status) {
+    extern __shared__ unsigned short sh_cum[];   // [32][Q] then [32][kRansBuckets + 1]
+    const int cg = blockIdx.y, plane = blockIdx.z;
+    unsigned short *sh_idx = sh_cum + 32 * s.Q;
+    load_group_cum(sh_cum, cum, plane, cg, s);
+    __syncthreads();
+    const int nact = min(32, s.C - 32 * cg);
+    const int bshift = s.P - 8;
+    const unsigned top = 1u << s.P;
+    // idx[j][b] = the symbol whose slot range holds b << bshift: every bucket start lies in exactly one symbol
+    for (int k = threadIdx.x; k < nact * s.Q; k += blockDim.x) {
+        const int j = k / s.Q, q = k - j * s.Q;
+        const unsigned lo = sh_cum[k], hi = q + 1 < s.Q ? (unsigned)sh_cum[k + 1] : top;
+        for (unsigned b = (lo + (1u << bshift) - 1) >> bshift; (b << bshift) < hi && b < kRansBuckets; ++b)
+            sh_idx[j * (kRansBuckets + 1) + b] = (unsigned short)q;
+    }
+    for (int j = threadIdx.x; j < nact; j += blockDim.x) sh_idx[j * (kRansBuckets + 1) + kRansBuckets] = (unsigned short)(s.Q - 1);
+    __syncthreads();
+
+    const int lane = threadIdx.x & 31;
+    const long long unit = (long long)blockIdx.x * kRansWarps + (threadIdx.x >> 5);
+    if (unit >= (long long)s.items * s.n_segs) return;
+    const int item = (int)(unit / s.n_segs);
+    const long long r0 = (unit % s.n_segs) * s.seg_rows;
+    const long long len = min(s.seg_rows, s.item_rows - r0);
+    const bool active = lane < nact;
+    const int c = 32 * cg + lane;
+    const unsigned short *tab = sh_cum + (active ? lane : 0) * s.Q;
+    const unsigned short *cidx = sh_idx + (active ? lane : 0) * (kRansBuckets + 1);
+    const long long g = (((long long)plane * s.items * s.n_segs + unit) * s.CG + cg);
+    long long start = bounds[2 * g], end = bounds[2 * g + 1];
+    int err = 0;
+    if (start < 0 || end > n_words || end - start < 2ll * nact) { err = 4; end = start = 0; }
+    const long long out0 = (((long long)plane * s.items + item) * s.item_rows + r0) * s.C + c;
+    const float *cp = code_points + (size_t)(active ? c : 0) * s.Q;
+    const unsigned lt = lanemask_lt();
+
+    unsigned x = kRansL;
+    if (!err && active) x = (unsigned)__ldg(words + start + 2 * lane) | ((unsigned)__ldg(words + start + 2 * lane + 1) << 16);
+    if (__any_sync(0xffffffffu, active && x < kRansL)) err |= 4;
+    long long pos = start + 2 * nact;
+    long long wbase = pos;
+    unsigned w0 = ld_word(words, wbase + lane, end), w1 = ld_word(words, wbase + 32 + lane, end);
+    unsigned w2 = ld_word(words, wbase + 64 + lane, end), w3 = ld_word(words, wbase + 96 + lane, end);
+
+    // z_hat of a block is gathered after the block and stored after the next one, so the gather's latency never stalls
+    // the state chain
+    float zprev[kDecBlock];
+    long long tprev = -1;
+    for (long long t0 = 0; t0 < len && !err; t0 += kDecBlock) {
+        int sy[kDecBlock];
+#pragma unroll
+        for (int k = 0; k < kDecBlock; ++k) {
+            sy[k] = 0;
+            if (t0 + k >= len) break;                      // warp-uniform
+            const unsigned slot = x & (top - 1);
+            int lo = min((int)cidx[slot >> bshift], s.Q - 1), hi = min((int)cidx[(slot >> bshift) + 1], s.Q - 1);
+            while (lo < hi) {
+                const int mid = (lo + hi + 1) >> 1;
+                if (tab[mid] <= slot) lo = mid; else hi = mid - 1;
+            }
+            const unsigned c0 = tab[lo];
+            const unsigned f = (lo + 1 < s.Q ? (unsigned)tab[lo + 1] : top) - c0;
+            x = f * (x >> s.P) + slot - c0;
+            const bool need = active && x < kRansL;
+            const unsigned mask = __ballot_sync(0xffffffffu, need);
+            const int n = __popc(mask);
+            if (pos + n > end) { err |= 1; break; }
+            const int rel = (int)(pos - wbase) + __popc(mask & lt);   // < 64 for the lanes that read
+            const unsigned a = __shfl_sync(0xffffffffu, w0, rel & 31), b = __shfl_sync(0xffffffffu, w1, rel & 31);
+            if (need) x = (x << 16) | (rel < 32 ? a : b);
+            pos += n;
+            if (pos - wbase >= 32) {
+                w0 = w1; w1 = w2; w2 = w3;
+                wbase += 32;
+                w3 = ld_word(words, wbase + 96 + lane, end);
+            }
+            sy[k] = lo;
+        }
+        if (zhat && tprev >= 0) {
+#pragma unroll
+            for (int k = 0; k < kDecBlock; ++k)
+                if (active) zhat[out0 + (tprev + k) * s.C] = zprev[k];   // a previous block is always full
+        }
+        if (err) break;
+#pragma unroll
+        for (int k = 0; k < kDecBlock; ++k) {
+            if (active && t0 + k < len) {
+                if (qidx) qidx[out0 + (t0 + k) * s.C] = sy[k];
+                if (zhat) zprev[k] = __ldg(cp + sy[k]);
+            }
+        }
+        tprev = t0;
+    }
+    if (zhat && tprev >= 0 && !err) {
+#pragma unroll
+        for (int k = 0; k < kDecBlock; ++k)
+            if (active && tprev + k < len) zhat[out0 + (tprev + k) * s.C] = zprev[k];
+    }
+    if (!err && (__any_sync(0xffffffffu, active && x != kRansL) || pos != end)) err |= 2;
+    if (err && lane == 0) atomicOr(status, err);
+}
+
+}  // namespace
+
+extern "C" long long vbq_rans_workspace_bytes(int n_planes, int items, long long item_rows, int C, long long seg_rows) {
+    RansShape s;
+    if (rans_shape("vbq_rans_workspace_bytes", n_planes, items, item_rows, C, seg_rows, 0, 16, &s) != VBQ_OK) return -1;
+    return 2 * align256(8ll * n_planes * s.G) + align256(2ll * n_planes * rans_plane_scratch_words(s));
+}
+
+extern "C" long long vbq_rans_payload_bound(int n_planes, int items, long long item_rows, int C, long long seg_rows) {
+    RansShape s;
+    if (rans_shape("vbq_rans_payload_bound", n_planes, items, item_rows, C, seg_rows, 0, 16, &s) != VBQ_OK) return -1;
+    return 2ll * n_planes * (2 * s.G + rans_plane_scratch_words(s));
+}
+
+extern "C" int vbq_rans_encode(const int *d_qidx, int n_planes, int items, long long item_rows, int C,
+                               long long seg_rows, int N, int prob_bits, const unsigned short *d_cum,
+                               unsigned short *d_payload, long long payload_bytes, long long *d_payload_size,
+                               int *d_status, void *d_workspace, long long workspace_bytes, void *stream) {
+    RansShape s;
+    RETURN_IF(rans_shape("vbq_rans_encode", n_planes, items, item_rows, C, seg_rows, N, prob_bits, &s));
+    if (!d_cum || !d_payload || !d_payload_size || !d_status || (s.G > 0 && (!d_qidx || !d_workspace)))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_encode: null pointer");
+    if (payload_bytes < vbq_rans_payload_bound(n_planes, items, item_rows, C, seg_rows))
+        return vbq_fail(VBQ_ERR_WORKSPACE, "vbq_rans_encode: payload capacity %lld < vbq_rans_payload_bound %lld",
+                        payload_bytes, vbq_rans_payload_bound(n_planes, items, item_rows, C, seg_rows));
+    const long long need = vbq_rans_workspace_bytes(n_planes, items, item_rows, C, seg_rows);
+    if (s.G > 0 && workspace_bytes < need)
+        return vbq_fail(VBQ_ERR_WORKSPACE, "vbq_rans_encode: workspace %lld < %lld bytes", workspace_bytes, need);
+    if (((uintptr_t)d_payload & 1) || ((uintptr_t)d_cum & 1) || ((uintptr_t)d_workspace & 7) || ((uintptr_t)d_qidx & 3))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_encode: misaligned pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int), st));
+    if (s.G == 0) {
+        CUDA_TRY(cudaMemsetAsync(d_payload_size, 0, sizeof(long long), st));
+        return VBQ_OK;
+    }
+    int dev = 0, sms = 0;
+    RETURN_IF(vbq_current_device(&dev, &sms));
+    char *ws = (char *)d_workspace;
+    long long *sizes = (long long *)ws;
+    long long *dst = (long long *)(ws + align256(8ll * n_planes * s.G));
+    unsigned short *scratch = (unsigned short *)(ws + 2 * align256(8ll * n_planes * s.G));
+    const long long units = (long long)s.items * s.n_segs;
+    const dim3 grid((unsigned)((units + kRansWarps - 1) / kRansWarps), s.CG, n_planes);
+    const size_t smem = (size_t)32 * s.Q * sizeof(unsigned short);
+    VBQ_ENSURE_MAX_SMEM(vbq_rans_encode_kernel, dev);
+    vbq_rans_encode_kernel<<<grid, kRansWarps * 32, smem, st>>>(d_qidx, d_cum, s, scratch, sizes, d_status);
+    CUDA_TRY(cudaGetLastError());
+    vbq_rans_scan_kernel<<<1, 1024, 0, st>>>(sizes, dst, n_planes, s.G, d_payload, d_payload_size);
+    CUDA_TRY(cudaGetLastError());
+    vbq_rans_compact_kernel<<<(unsigned)(n_planes * s.G), 256, 0, st>>>(scratch, sizes, dst, s, d_payload);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+extern "C" int vbq_rans_decode(const unsigned short *d_payload, long long payload_words,
+                               const long long *d_group_bounds, int n_planes, int items, long long item_rows, int C,
+                               long long seg_rows, int N, int prob_bits, const unsigned short *d_cum,
+                               const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status, void *stream) {
+    RansShape s;
+    RETURN_IF(rans_shape("vbq_rans_decode", n_planes, items, item_rows, C, seg_rows, N, prob_bits, &s));
+    if (payload_words < 0) return vbq_fail(VBQ_ERR_BAD_SHAPE, "vbq_rans_decode: payload_words=%lld", payload_words);
+    if (!d_cum || !d_status || (d_zhat && !d_code_points) || (s.G > 0 && (!d_payload || !d_group_bounds)))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_decode: null pointer");
+    if (((uintptr_t)d_payload & 1) || ((uintptr_t)d_cum & 1) || ((uintptr_t)d_group_bounds & 7) ||
+        ((uintptr_t)d_qidx & 3) || ((uintptr_t)d_zhat & 3) || ((uintptr_t)d_code_points & 3))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_decode: misaligned pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int), st));
+    if (s.G == 0) return VBQ_OK;
+    int dev = 0, sms = 0;
+    RETURN_IF(vbq_current_device(&dev, &sms));
+    const long long units = (long long)s.items * s.n_segs;
+    const dim3 grid((unsigned)((units + kRansWarps - 1) / kRansWarps), s.CG, n_planes);
+    const size_t smem = (size_t)32 * (s.Q + kRansBuckets + 1) * sizeof(unsigned short);
+    VBQ_ENSURE_MAX_SMEM(vbq_rans_decode_kernel, dev);
+    vbq_rans_decode_kernel<<<grid, kRansWarps * 32, smem, st>>>(d_payload, payload_words, d_group_bounds, d_cum, s,
+                                                                d_code_points, d_qidx, d_zhat, d_status);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}

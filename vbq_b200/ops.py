@@ -588,3 +588,60 @@ def symbol_histogram(qidx: torch.Tensor, max_bits: int, counts: Optional[torch.T
                                           _stream(qidx.device))
     _lib.check(st, "vbq_symbol_histogram")
     return counts
+
+
+# ------------------------------------------------------------------------------------------------------
+# entropy coding: interleaved rANS over (item, row segment, 32-channel group) groups (include/vbq_b200.h, csrc/rans.cu)
+# ------------------------------------------------------------------------------------------------------
+def rans_payload_bound(n_planes: int, items: int, item_rows: int, C: int, seg_rows: int) -> int:
+    return int(_lib.load().vbq_rans_payload_bound(n_planes, items, item_rows, C, seg_rows))
+
+
+def rans_encode(qidx: torch.Tensor, cum: torch.Tensor, max_bits: int, prob_bits: int, seg_rows: int):
+    """qidx (n_planes, items, item_rows, C) int32 and cum (n_planes, C, Q) int16 (the uint16 cum tables of
+    coding.cum_table) -> (payload int16 words of vbq_rans_payload_bound bytes, payload size in bytes as a 1-element
+    int64 tensor, status int32 tensor): one launch for all planes, no synchronisation."""
+    _need_cuda("qidx", qidx, torch.int32, 4)
+    _need_cuda("cum", cum, torch.int16, 3)
+    n_planes, items, item_rows, C = qidx.shape
+    lib = _lib.load()
+    bound = lib.vbq_rans_payload_bound(n_planes, items, item_rows, C, seg_rows)
+    ws_bytes = lib.vbq_rans_workspace_bytes(n_planes, items, item_rows, C, seg_rows)
+    if bound < 0 or ws_bytes < 0:
+        raise ValueError("vbq_b200: bad rANS shape: %s" % lib.vbq_last_error().decode())
+    dev = qidx.device
+    payload = torch.empty(max(1, bound // 2), dtype=torch.int16, device=dev)
+    size = torch.zeros(1, dtype=torch.int64, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    ws = torch.empty(max(1, ws_bytes), dtype=torch.uint8, device=dev)
+    st = lib.vbq_rans_encode(_ptr(qidx), n_planes, items, item_rows, C, seg_rows, max_bits, prob_bits, _ptr(cum),
+                             payload.data_ptr(), bound, size.data_ptr(), status.data_ptr(), ws.data_ptr(), ws_bytes,
+                             _stream(dev))
+    _lib.check(st, "vbq_rans_encode")
+    return payload, size, status
+
+
+def rans_decode(words: torch.Tensor, bounds: torch.Tensor, cum: torch.Tensor, items: int, item_rows: int,
+                seg_rows: int, max_bits: int, prob_bits: int, code_points: Optional[torch.Tensor] = None,
+                want_qidx: bool = True):
+    """words: the payload as int16 words; bounds (n_planes * groups, 2) int64 word ranges of the groups; cum
+    (n_planes, C, Q) int16.  Returns (qidx or None, zhat or None, status): (n_planes, items, item_rows, C) int32 symbols
+    and float32 code_points[c, q] (code_points (C, Q) ascending), and the int32 device status (0 = every group passed
+    the integrity check)."""
+    _need_cuda("words", words, torch.int16, 1)
+    _need_cuda("bounds", bounds, torch.int64, 2)
+    _need_cuda("cum", cum, torch.int16, 3)
+    n_planes, C, _ = cum.shape
+    dev = words.device
+    shape = (n_planes, items, item_rows, C)
+    q = torch.empty(shape, dtype=torch.int32, device=dev) if want_qidx else None
+    z = None
+    if code_points is not None:
+        _need_cuda("code_points", code_points, torch.float32, 2)
+        z = torch.empty(shape, dtype=torch.float32, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    st = _lib.load().vbq_rans_decode(_ptr(words), words.numel(), _ptr(bounds), n_planes, items, item_rows, C,
+                                     seg_rows, max_bits, prob_bits, _ptr(cum), _ptr(code_points), _ptr(q), _ptr(z),
+                                     status.data_ptr(), _stream(dev))
+    _lib.check(st, "vbq_rans_decode")
+    return q, z, status

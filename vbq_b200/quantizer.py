@@ -10,7 +10,7 @@ from __future__ import annotations
 import numpy as np
 import torch
 
-from . import ops, utils
+from . import coding, ops, serialize, utils
 
 
 _PINNED = {}   # (shape, dtype) -> pinned staging buffer for count tables (allocated once: cudaHostAlloc takes ~100 ms)
@@ -388,6 +388,52 @@ class ChannelwisePriorCDFQuantizer:
         self.entropy_models = entropy_models
         self._cache = {}
         return None
+
+    # ------------------------------------------------------------------------------------------------
+    # entropy coding: latents -> bytes -> z_hat (serialize.encode / decode, the rANS kernels of csrc/rans.cu)
+    # ------------------------------------------------------------------------------------------------
+    def rans_tables(self, lamb, prob_bits=coding.DEFAULT_PROB_BITS):
+        """(C, Q) int32 integer frequency table of entropy_models[lamb] (coding.frequency_tables), cached."""
+        key = ("rans", float(lamb), int(prob_bits))
+        if key not in self._cache:
+            self._cache[key] = coding.frequency_tables(self.entropy_models[lamb], prob_bits)
+        return self._cache[key]
+
+    def compress_to_bytes(self, posterior_means, posterior_logvars, lambs, prob_bits=coding.DEFAULT_PROB_BITS,
+                          seg_rows=None):
+        """Quantize (B, H', W', C) latents like `compress_latents` and entropy-code every image under the fitted
+        entropy models: {lambda: [bytes of image b for b in range(B)]}.  Every blob is a VBQ2 stream of one image and
+        one lambda that `decompress_from_bytes` turns back into its z_hat; the whole batch is coded in one launch."""
+        if self.entropy_models is None:
+            raise TypeError("'NoneType' object is not subscriptable: entropy_models not built "
+                            "(call build_entropy_models first)")
+        shape = tuple(posterior_means.shape)
+        assert shape[-1] == self.num_channels
+        B = shape[0] if len(shape) > 1 else 1
+        height = shape[1] if len(shape) == 4 else 0
+        m, lv = self._prep(posterior_means, posterior_logvars)
+        qidx = self.quantize(m, lv, lambs, logvar=True, outputs=ops.OUT_QIDX)['qidx']
+        tables = np.stack([self.rans_tables(l, prob_bits) for l in lambs])
+        blobs = serialize.encode_items(qidx, tables, self.max_bits_per_coord, items=B, seg_rows=seg_rows,
+                                       lambdas=lambs, height=height)
+        return {lamb: blobs[i] for i, lamb in enumerate(lambs)}
+
+    def decompress_from_bytes(self, blob):
+        """z_hat of a `compress_to_bytes` blob as a device tensor (1, H', W', C) (several items or planes stack on the
+        first axis).  The blob's lambda selects the entropy model by float equality, as the dict keys do."""
+        h = serialize.read_header(blob)
+        keys = []
+        for lam in h["lambdas"]:
+            k = [l for l in (self.entropy_models or {}) if float(l) == lam]
+            if not k:
+                raise KeyError(lam)
+            keys.append(k[0])
+        tables = [self.rans_tables(k, h["prob_bits"]) for k in keys]
+        out = serialize.decode(blob, tables=tables, code_points=self.code_points_by_channel, device=self.device,
+                               want_qidx=False)
+        z = out["zhat"]
+        Hp = out["height"] or out["item_rows"]
+        return z.reshape(-1, Hp, out["item_rows"] // max(1, Hp), self.num_channels)
 
     @property
     def lambs(self):

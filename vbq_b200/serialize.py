@@ -1,12 +1,20 @@
-"""Wire format for the emitted symbols (SURVEY §8 row f4; arithmetic coding itself stays out of scope).
+"""Wire formats for the emitted symbols (SURVEY §8 row f4).
 
 The reference stops at counting its sorted quantile indices per channel (quantizer.py:135-146) and reporting ideal
-code lengths (ipynb:452-455).  This module turns the kernel's `qidx` output into bytes an external entropy coder can
-consume: a fixed-width bit stream (max_bits_per_coord+1 bits per symbol, packed on the GPU) plus, optionally, the
-per-channel frequency tables the coder needs, and reads it back.
+code lengths (ipynb:452-455).  This module turns the kernel's `qidx` output into bytes and reads them back, in two
+formats:
 
-Layout (little endian):  magic b"VBQ1" | uint32 N, C, L, flags | uint64 rows | [flags & 1: L*C*Q uint32 counts]
-| L streams, each ceil(rows*C*(N+1)/32) uint32 words (symbols in (row, channel) order).
+VBQ1 (`dumps` / `loads`): a fixed-width bit stream (max_bits_per_coord+1 bits per symbol, packed on the GPU) plus,
+optionally, the per-channel counts an external entropy coder needs.  Layout (little endian):  magic b"VBQ1" |
+uint32 N, C, L, flags | uint64 rows | [flags & 1: L*C*Q uint32 counts] | L streams, each ceil(rows*C*(N+1)/32) uint32
+words (symbols in (row, channel) order).
+
+VBQ2 (`encode` / `decode`): entropy coded with the GPU rANS coder of csrc/rans.cu, one integer frequency table per
+(plane, channel) (`coding.frequency_tables`).  Layout (little endian):  magic b"VBQ2" | uint32 N, C, prob_bits,
+n_planes, items | uint64 item_rows, seg_rows | uint32 height, flags | per plane: float64 lambda, uint64 fingerprint of
+its table (`coding.fingerprint`) | [flags & 1: the tables, n_planes*C*Q uint16 entries f-1] | the rANS payload of
+include/vbq_b200.h (per plane: uint32 group end offsets, then the groups' 16-bit words).  `height` is H' of an
+item of H' x W' = item_rows latent rows (0 if unknown).
 """
 from __future__ import annotations
 
@@ -15,7 +23,7 @@ import struct
 import numpy as np
 import torch
 
-from . import ops
+from . import coding, ops
 
 MAGIC = b"VBQ1"
 _HDR = struct.Struct("<4sIIIIQ")
@@ -69,3 +77,207 @@ def ideal_code_length_bits(counts) -> float:
     t1 = torch.where(tot > 0, tot * torch.log2(tot.clamp(min=1)), torch.zeros_like(tot)).sum()
     t2 = torch.where(c > 0, c * torch.log2(c.clamp(min=1)), torch.zeros_like(c)).sum()
     return float(t1 - t2)
+
+
+# ------------------------------------------------------------------------------------------------------
+# VBQ2: rANS-coded planes
+# ------------------------------------------------------------------------------------------------------
+MAGIC2 = b"VBQ2"
+_HDR2 = struct.Struct("<4sIIIIIQQII")
+_PLANE2 = struct.Struct("<dQ")
+FLAG_TABLES = 1
+
+
+def _as_tables(tables, n_planes):
+    t = np.asarray(tables)
+    if t.ndim == 2:
+        t = np.broadcast_to(t, (n_planes,) + t.shape)
+    if t.ndim != 3 or t.shape[0] != n_planes:
+        raise ValueError("vbq_b200.serialize: need one (C, Q) table per plane, got shape %s" % (t.shape,))
+    return t
+
+
+def _encode_payload(qidx, tables, max_bits, items, seg_rows):
+    """-> (header fields, host payload as uint16 words, tables int64)."""
+    q = qidx if qidx.dim() == 3 else qidx.unsqueeze(0)
+    L, rows, C = q.shape
+    items = int(items)
+    if items < 1 or rows % items:
+        raise ValueError("vbq_b200.serialize: %d rows do not split into %d items" % (rows, items))
+    item_rows = rows // items
+    seg = max(1, item_rows if seg_rows is None else int(seg_rows))
+    t = _as_tables(tables, L)
+    P = coding.prob_bits_of(t)
+    t = coding.check_tables(t, P)
+    if t.shape[1:] != (C, ops.num_levels(max_bits)):
+        raise ValueError("vbq_b200.serialize: tables are %s, need (C, Q) = (%d, %d)" % (t.shape[1:], C,
+                                                                                     ops.num_levels(max_bits)))
+    cum = torch.from_numpy(coding.cum_table(t).view(np.int16)).to(q.device)
+    payload, size, status = ops.rans_encode(q.contiguous().reshape(L, items, item_rows, C), cum, max_bits, P, seg)
+    if int(status.item()) != 0:
+        raise ValueError("vbq_b200.serialize: a symbol lies outside [0, Q) for max_bits=%d" % max_bits)
+    n = int(size.item()) // 2
+    words = payload[:n].cpu().numpy().view(np.uint16)
+    return dict(N=max_bits, C=C, P=P, n_planes=L, items=items, item_rows=item_rows, seg_rows=seg), words, t
+
+
+def _header(f, lambdas, fingerprints, height, tables=None):
+    out = [_HDR2.pack(MAGIC2, f["N"], f["C"], f["P"], f["n_planes"], f["items"], f["item_rows"], f["seg_rows"],
+                      int(height), FLAG_TABLES if tables is not None else 0)]
+    out += [_PLANE2.pack(float(l), fp) for l, fp in zip(lambdas, fingerprints)]
+    if tables is not None:
+        out.append(np.ascontiguousarray(tables - 1, dtype="<u2").tobytes())
+    return out
+
+
+def _lambdas(lambdas, L):
+    lam = [0.0] * L if lambdas is None else [float(l) for l in lambdas]
+    if len(lam) != L:
+        raise ValueError("vbq_b200.serialize: %d lambdas for %d planes" % (len(lam), L))
+    return lam
+
+
+def encode(qidx, tables, max_bits: int, items: int = 1, seg_rows=None, embed_tables: bool = False, lambdas=None,
+           height: int = 0) -> bytes:
+    """Entropy-code sorted quantile indices into one VBQ2 blob (one kernel launch for all planes).
+
+    qidx: (rows, C) or (L, rows, C) int32 CUDA tensor, rows = items * item_rows (each item, e.g. one image, in row
+    order).  tables: (C, Q) or (L, C, Q) integer frequency tables (`coding.frequency_tables`).  seg_rows: rows per
+    coded segment (default: the whole item); every segment of every 32-channel group costs a 32-bit state per channel.
+    embed_tables: store the tables in the blob (for streams coded from their own counts).  lambdas: the plane labels
+    recorded in the header (default 0.0).  height: H' of an item of H' x W' latent rows, recorded for the receiver."""
+    f, words, t = _encode_payload(qidx, tables, max_bits, items, seg_rows)
+    fps = [coding.fingerprint(t[i]) for i in range(f["n_planes"])]
+    out = _header(f, _lambdas(lambdas, f["n_planes"]), fps, height, t if embed_tables else None)
+    out.append(words.astype("<u2").tobytes())
+    return b"".join(out)
+
+
+def encode_items(qidx, tables, max_bits: int, items: int, seg_rows=None, lambdas=None, height: int = 0):
+    """Like `encode` (one launch for every plane and item), but returns one separately decodable VBQ2 blob per
+    (plane, item): a list over planes of lists over items of bytes."""
+    f, words, t = _encode_payload(qidx, tables, max_bits, items, seg_rows)
+    lam = _lambdas(lambdas, f["n_planes"])
+    G = f["items"] * -(-f["item_rows"] // f["seg_rows"]) * -(-f["C"] // 32)
+    per_item = G // f["items"] if f["items"] else 0
+    one = dict(f, n_planes=1, items=1)
+    out, pos = [], 0
+    for p in range(f["n_planes"]):
+        ends = words[pos:pos + 2 * G].astype(np.uint64)
+        ends = ends[0::2] | (ends[1::2] << np.uint64(16))
+        data = words[pos + 2 * G:pos + 2 * G + (int(ends[-1]) if G else 0)]
+        pos += 2 * G + (int(ends[-1]) if G else 0)
+        hdr = b"".join(_header(one, [lam[p]], [coding.fingerprint(t[p])], height))
+        blobs = []
+        for i in range(f["items"]):
+            a = int(ends[i * per_item - 1]) if i and per_item else 0
+            b = int(ends[(i + 1) * per_item - 1]) if per_item else 0
+            e = ends[i * per_item:(i + 1) * per_item] - np.uint64(a)
+            tab = np.stack([e & np.uint64(0xFFFF), e >> np.uint64(16)], axis=1).reshape(-1).astype("<u2")
+            blobs.append(hdr + tab.tobytes() + data[a:b].astype("<u2").tobytes())
+        out.append(blobs)
+    return out
+
+
+def read_header(data: bytes) -> dict:
+    """Parse and check a VBQ2 header (host only): N, C, prob_bits, n_planes, items, item_rows, seg_rows, height,
+    flags, lambdas, fingerprints, embedded tables or None, and the byte offset of the payload.  Raises ValueError."""
+    data = memoryview(data)
+    if len(data) < _HDR2.size:
+        raise ValueError("vbq_b200.serialize: %d bytes are too short for a VBQ2 header" % len(data))
+    magic, N, C, P, L, items, item_rows, seg_rows, height, flags = _HDR2.unpack_from(data, 0)
+    if magic != MAGIC2:
+        raise ValueError("vbq_b200.serialize: bad magic %r (expected %r)" % (bytes(magic), MAGIC2))
+    if N > 10 or C < 1 or L < 1 or seg_rows < 1 or not 12 <= P <= 16 or flags & ~FLAG_TABLES:
+        raise ValueError("vbq_b200.serialize: bad VBQ2 header (N=%d C=%d prob_bits=%d planes=%d seg_rows=%d flags=%d)"
+                         % (N, C, P, L, seg_rows, flags))
+    if height and item_rows % height:
+        raise ValueError("vbq_b200.serialize: height %d does not divide %d rows" % (height, item_rows))
+    Q = ops.num_levels(N)
+    pos = _HDR2.size + L * _PLANE2.size
+    if len(data) < pos:
+        raise ValueError("vbq_b200.serialize: truncated plane table")
+    planes = [_PLANE2.unpack_from(data, _HDR2.size + i * _PLANE2.size) for i in range(L)]
+    tables = None
+    if flags & FLAG_TABLES:
+        n = L * C * Q
+        if len(data) < pos + 2 * n:
+            raise ValueError("vbq_b200.serialize: truncated frequency tables")
+        tables = np.frombuffer(data, dtype="<u2", count=n, offset=pos).astype(np.int64).reshape(L, C, Q) + 1
+        pos += 2 * n
+    return dict(max_bits=N, C=C, prob_bits=P, n_planes=L, items=items, item_rows=item_rows, seg_rows=seg_rows,
+                height=height, flags=flags, lambdas=[p[0] for p in planes], fingerprints=[p[1] for p in planes],
+                tables=tables, payload_offset=pos)
+
+
+def _group_bounds(words, h):
+    """Check the offset tables of a payload (monotone, every group holding at least its states, inside the payload,
+    nothing left over) -> (n_planes * groups, 2) int64 word ranges."""
+    C, items = h["C"], h["items"]
+    n_segs = -(-h["item_rows"] // h["seg_rows"])
+    CG = -(-C // 32)
+    G = items * n_segs * CG
+    nact = np.tile(np.minimum(32, C - 32 * np.arange(CG)), items * n_segs).astype(np.int64)
+    bounds, pos = [], 0
+    for _ in range(h["n_planes"]):
+        if pos + 2 * G > words.size:
+            raise ValueError("vbq_b200.serialize: payload truncated in an offset table")
+        e = words[pos:pos + 2 * G].astype(np.int64)
+        ends = e[0::2] | (e[1::2] << 16)
+        starts = np.concatenate([[0], ends[:-1]])[:G].astype(np.int64)
+        base = pos + 2 * G
+        if G and ((ends - starts < 2 * nact).any() or base + ends[-1] > words.size):
+            raise ValueError("vbq_b200.serialize: offset table out of range")
+        bounds.append(np.stack([base + starts, base + ends], axis=1))
+        pos = base + (int(ends[-1]) if G else 0)
+    if pos != words.size:
+        raise ValueError("vbq_b200.serialize: %d bytes after the last plane" % (2 * (words.size - pos)))
+    return np.concatenate(bounds) if bounds else np.zeros((0, 2), np.int64)
+
+
+def decode(data: bytes, tables=None, code_points=None, device="cuda", want_qidx: bool = True) -> dict:
+    """Inverse of `encode`.  tables: one (C, Q) integer table per plane (a sequence, an (L, C, Q) array, or a dict
+    keyed by the header's lambdas); default: the tables embedded in the blob.  Every table must have the fingerprint
+    the header records.  code_points: (C, Q) ascending code points (`code_points_by_channel`) to produce z_hat.
+
+    Returns dict(qidx, zhat: (n_planes, items, item_rows, C) device tensors or None, and the header fields).  A
+    malformed header or offset table, or a table with the wrong fingerprint, raises ValueError before any launch; a
+    payload that fails the decoder's integrity check raises ValueError after it."""
+    h = read_header(data)
+    L, C, P, N = h["n_planes"], h["C"], h["prob_bits"], h["max_bits"]
+    if tables is None:
+        if h["tables"] is None:
+            raise ValueError("vbq_b200.serialize: the blob embeds no frequency tables; pass `tables`")
+        tables = h["tables"]
+    elif isinstance(tables, dict):
+        try:
+            tables = [tables[lam] for lam in h["lambdas"]]
+        except KeyError as e:
+            raise ValueError("vbq_b200.serialize: no table for lambda %r" % (e.args[0],))
+    t = _as_tables([np.asarray(x) for x in tables] if isinstance(tables, (list, tuple)) else tables, L)
+    if t.shape[1:] != (C, ops.num_levels(N)):
+        raise ValueError("vbq_b200.serialize: tables are %s, the blob needs (%d, %d)" % (t.shape[1:], C, ops.num_levels(N)))
+    for i in range(L):
+        if coding.fingerprint(t[i]) != h["fingerprints"][i]:
+            raise ValueError("vbq_b200.serialize: the frequency table of plane %d (lambda %r) has another fingerprint "
+                             "than the one the stream was coded with" % (i, h["lambdas"][i]))
+    t = coding.check_tables(t, P)
+    rest = len(data) - h["payload_offset"]
+    if rest % 2:
+        raise ValueError("vbq_b200.serialize: payload of odd length")
+    words = np.frombuffer(data, dtype="<u2", count=rest // 2, offset=h["payload_offset"])
+    bounds = _group_bounds(words, h)
+    dev = torch.device(device)
+    w = torch.from_numpy(words.view(np.int16).copy()).to(dev)
+    b = torch.from_numpy(np.ascontiguousarray(bounds, dtype=np.int64)).to(dev)
+    cum = torch.from_numpy(coding.cum_table(t).view(np.int16)).to(dev)
+    cp = None if code_points is None else code_points.to(device=dev, dtype=torch.float32).contiguous()
+    q, z, status = ops.rans_decode(w, b, cum, h["items"], h["item_rows"], h["seg_rows"], N, P, cp, want_qidx)
+    st = int(status.item())
+    if st:
+        raise ValueError("vbq_b200.serialize: corrupt VBQ2 payload (decoder status %d: %s)" % (
+            st, ", ".join(m for bit, m in ((1, "a group ran out of words"), (2, "integrity check failed"),
+                                            (4, "bad group range or initial state")) if st & bit)))
+    out = {k: v for k, v in h.items() if k not in ("tables", "payload_offset")}
+    out.update(qidx=q, zhat=z)
+    return out
