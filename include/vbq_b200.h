@@ -274,6 +274,42 @@ int vbq_rans_decode(const unsigned short *d_payload, long long payload_words, co
                     const unsigned short *d_cum, const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status,
                     void *stream);
 
+/* ---- entropy coding with one shared table per plane: word embeddings (DESIGN.md §8d) ------------------------------
+ *
+ * All coordinates of an embedding matrix share one prior and one empirical model, so the channel axis of the layout
+ * above has no meaning.  This layout codes a plane as one flat sequence with ONE table:
+ *   PLANE   n int32 symbols q in [0, Q), Q = 2^(N+1)-1, N <= 10.  Symbol k sits at row k / 32, lane k % 32; a GROUP is
+ *           a segment of seg_rows rows (seg_rows chosen per plane).  The lanes of a group that hold at least one symbol
+ *           carry a state; on the plane's last row only the lanes with k < n take part.
+ *   TABLES  d_cum (n_planes, Q+1) uint32 with cum[0] = 0, cum[s+1] - cum[s] = f[s] and cum[Q] = 2^prob_bits
+ *           (12 <= prob_bits <= 16, Q <= 2^prob_bits).  Frequencies may be 0, and one symbol may hold all of 2^prob_bits
+ *           (its symbols then cost nothing and the group is only its states).
+ *   DECODER the decoded symbol is the largest s with cum[s] <= slot, which skips zero-frequency symbols wherever they
+ *           sit.  State, renormalisation, word order, the per-plane group end offset table, the payload layout and the
+ *           integrity rule (final state 2^16, every word read, every read inside the group's own range) are those of
+ *           vbq_rans_decode, with groups in segment order.
+ *
+ * seg_rows is a HOST array of n_planes entries (1 <= n_planes <= VBQ_RANS_SHARED_MAX_PLANES), each >= 1; a value
+ * above the plane's row count means one segment and is treated as that row count (the stream is the same).
+ * vbq_rans_shared_workspace_bytes / vbq_rans_shared_payload_bound: the encoder's workspace and the worst-case payload in
+ * bytes; -1 for a bad shape.  vbq_rans_shared_encode codes d_qidx (n_planes, n) in one launch into d_payload (at least
+ * vbq_rans_shared_payload_bound bytes) and leaves the payload size in bytes in *d_payload_size, without host
+ * synchronisation; *d_status gets bit 1 for a symbol outside [0, Q) and bit 2 for a symbol of frequency 0.
+ * vbq_rans_shared_decode takes the group word ranges d_group_bounds (all groups of the call, 2) int64 [start, end) from
+ * the offset tables and writes any of d_qidx (int32) and d_zhat (float32 d_code_points[q], a (Q,) ascending table) of
+ * shape (n_planes, n); *d_status as for vbq_rans_decode. */
+#define VBQ_RANS_SHARED_MAX_PLANES 64
+long long vbq_rans_shared_workspace_bytes(int n_planes, long long n, const long long *seg_rows);
+long long vbq_rans_shared_payload_bound(int n_planes, long long n, const long long *seg_rows);
+int vbq_rans_shared_encode(const int *d_qidx, int n_planes, long long n, const long long *seg_rows, int N, int prob_bits,
+                           const unsigned *d_cum, unsigned short *d_payload, long long payload_bytes,
+                           long long *d_payload_size, int *d_status, void *d_workspace, long long workspace_bytes,
+                           void *stream);
+int vbq_rans_shared_decode(const unsigned short *d_payload, long long payload_words, const long long *d_group_bounds,
+                           int n_planes, long long n, const long long *seg_rows, int N, int prob_bits,
+                           const unsigned *d_cum, const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status,
+                           void *stream);
+
 /* ---- stand-alone operator forms------------------------------------------------------------------------------- */
 
 /* ChannelwisePriorCDFQuantizer.get_all_N_bit_intervals (quantizer.py:65-80): d_mu (rows, C) -> d_left, d_right

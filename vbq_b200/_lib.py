@@ -26,6 +26,7 @@ GROUP = 16
 TOTALS = 4
 PRIOR_PARAMS = 43
 MAX_DEPTH = 20
+RANS_SHARED_MAX_PLANES = 64
 
 
 class VbqError(RuntimeError):
@@ -80,6 +81,10 @@ SIGNATURES = {
     "vbq_rans_payload_bound": (_ll, [_i, _i, _ll, _i, _ll]),
     "vbq_rans_encode": (_i, [_p, _i, _i, _ll, _i, _ll, _i, _i, _p, _p, _ll, _p, _p, _p, _ll, _p]),
     "vbq_rans_decode": (_i, [_p, _ll, _p, _i, _i, _ll, _i, _ll, _i, _i, _p, _p, _p, _p, _p, _p]),
+    "vbq_rans_shared_workspace_bytes": (_ll, [_i, _ll, _p]),
+    "vbq_rans_shared_payload_bound": (_ll, [_i, _ll, _p]),
+    "vbq_rans_shared_encode": (_i, [_p, _i, _ll, _p, _i, _i, _p, _p, _ll, _p, _p, _p, _ll, _p]),
+    "vbq_rans_shared_decode": (_i, [_p, _ll, _p, _i, _ll, _p, _i, _i, _p, _p, _p, _p, _p, _p]),
 }
 
 _lib = None

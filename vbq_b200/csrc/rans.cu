@@ -173,6 +173,27 @@ __device__ long long block_inclusive_sum(long long v, long long *sh_warp, long l
     return v;
 }
 
+// Block-wide exclusive scan of one plane's G group sizes: writes the plane's offset table at out[plane_start..] and
+// each group's destination word; returns the word where the next plane starts.
+__device__ long long scan_plane(const long long *__restrict__ sizes, long long *__restrict__ dst, long long G,
+                                long long plane_start, unsigned short *__restrict__ out, long long *sh_warp) {
+    long long carry = 0;
+    for (long long c0 = 0; c0 < G; c0 += blockDim.x) {
+        const long long i = c0 + threadIdx.x;
+        const long long v = i < G ? sizes[i] : 0;
+        long long chunk;
+        const long long incl = block_inclusive_sum(v, sh_warp, &chunk);
+        if (i < G) {
+            const unsigned long long e = (unsigned long long)(carry + incl);
+            out[plane_start + 2 * i] = (unsigned short)(e & 0xffffu);
+            out[plane_start + 2 * i + 1] = (unsigned short)(e >> 16);
+            dst[i] = plane_start + 2 * G + carry + incl - v;
+        }
+        carry += chunk;
+    }
+    return plane_start + 2 * G + carry;
+}
+
 // One CTA: exclusive scan of the group sizes of every plane -> each group's destination, the planes' offset tables
 // and the payload size in bytes.
 __global__ void __launch_bounds__(1024) vbq_rans_scan_kernel(const long long *__restrict__ sizes,
@@ -181,23 +202,8 @@ __global__ void __launch_bounds__(1024) vbq_rans_scan_kernel(const long long *__
                                                             long long *__restrict__ out_bytes) {
     __shared__ long long sh_warp[32];
     long long plane_start = 0;   // in words
-    for (int p = 0; p < n_planes; ++p) {
-        long long carry = 0;
-        for (long long c0 = 0; c0 < G; c0 += blockDim.x) {
-            const long long i = c0 + threadIdx.x;
-            const long long v = i < G ? sizes[(long long)p * G + i] : 0;
-            long long chunk;
-            const long long incl = block_inclusive_sum(v, sh_warp, &chunk);
-            if (i < G) {
-                const unsigned long long e = (unsigned long long)(carry + incl);
-                out[plane_start + 2 * i] = (unsigned short)(e & 0xffffu);
-                out[plane_start + 2 * i + 1] = (unsigned short)(e >> 16);
-                dst[(long long)p * G + i] = plane_start + 2 * G + carry + incl - v;
-            }
-            carry += chunk;
-        }
-        plane_start += 2 * G + carry;
-    }
+    for (int p = 0; p < n_planes; ++p)
+        plane_start = scan_plane(sizes + (long long)p * G, dst + (long long)p * G, G, plane_start, out, sh_warp);
     if (threadIdx.x == 0) *out_bytes = 2 * plane_start;
 }
 
@@ -336,6 +342,276 @@ __global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_decode_kernel(const 
     if (err && lane == 0) atomicOr(status, err);
 }
 
+// ---- the shared-table layout (vbq_rans_shared_*): one table per plane, symbols as one flat sequence ----------------
+//
+// Symbol k of a plane sits at row k / 32, lane k % 32; a group is a segment of seg_rows rows (seg_rows per plane), coded
+// by one warp.  Only the plane's last row can be partial.  The table is staged once per CTA (8 KiB at N = 10), so many
+// small CTAs share an SM and hide the dependent state chain of each warp.
+
+constexpr int kSharedWarps = 4;
+
+struct SharedShape {
+    int n_planes, P, Q;
+    long long n, rows;                             // symbols per plane, rows = ceil(n / 32)
+    long long seg[VBQ_RANS_SHARED_MAX_PLANES];     // seg_rows of each plane
+    long long gbase[VBQ_RANS_SHARED_MAX_PLANES + 1];   // the call's first group of each plane; [n_planes] = all groups
+    long long sbase[VBQ_RANS_SHARED_MAX_PLANES + 1];   // first encoder scratch word of each plane
+    long long max_groups;                          // of any plane
+};
+
+int shared_shape(const char *fn, int n_planes, long long n, const long long *seg_rows, int N, int prob_bits,
+                 SharedShape *s) {
+    if (n_planes < 1 || n_planes > VBQ_RANS_SHARED_MAX_PLANES || n < 0)
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "%s: n_planes=%d (1..%d) n=%lld", fn, n_planes, VBQ_RANS_SHARED_MAX_PLANES, n);
+    if (!seg_rows) return vbq_fail(VBQ_ERR_NULL_POINTER, "%s: seg_rows is NULL", fn);
+    if (N < 0 || N > 10) return vbq_fail(VBQ_ERR_BAD_DEPTH, "%s: N=%d (the coder holds N <= 10)", fn, N);
+    const int Q = (1 << (N + 1)) - 1;
+    if (prob_bits < 12 || prob_bits > 16 || Q > (1 << prob_bits))
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "%s: prob_bits=%d (12..16 with Q=%d <= 2^prob_bits)", fn, prob_bits, Q);
+    s->n_planes = n_planes; s->P = prob_bits; s->Q = Q; s->n = n; s->rows = n / 32 + (n % 32 != 0);
+    s->gbase[0] = 0; s->sbase[0] = 0; s->max_groups = 0;
+    for (int p = 0; p < n_planes; ++p) {
+        if (seg_rows[p] < 1) return vbq_fail(VBQ_ERR_BAD_SHAPE, "%s: seg_rows[%d]=%lld", fn, p, seg_rows[p]);
+        // a segment longer than the plane is the whole plane: clamp before the scratch is sized from it
+        const long long seg = min(seg_rows[p], max(s->rows, 1ll));
+        const long long G = (s->rows + seg - 1) / seg;
+        // worst-case words of the plane: a word per symbol, two per lane and group, its offset table
+        if ((double)n + 66.0 * (double)G >= 4294967296.0 || (double)s->gbase[p] + G >= 2147483647.0)
+            return vbq_fail(VBQ_ERR_BAD_SHAPE, "%s: a plane of %lld symbols in segments of %lld rows exceeds the 32-bit "
+                            "offset table", fn, n, seg);
+        s->seg[p] = seg;
+        s->gbase[p + 1] = s->gbase[p] + G;
+        s->sbase[p + 1] = s->sbase[p] + G * 32 * (seg + 2);
+        s->max_groups = max(s->max_groups, G);
+    }
+    return VBQ_OK;
+}
+
+// Lanes of row r of a plane that hold a symbol.
+__device__ __forceinline__ int shared_row_lanes(const SharedShape &s, long long r) {
+    return r == s.rows - 1 ? (int)(s.n - 32 * (s.rows - 1)) : 32;
+}
+
+__device__ __forceinline__ void load_plane_cum(unsigned *sh_cum, const unsigned *__restrict__ cum, int plane, int Q) {
+    const unsigned *src = cum + (size_t)plane * (Q + 1);
+    for (int i = threadIdx.x; i <= Q; i += blockDim.x) sh_cum[i] = __ldg(src + i);
+}
+
+// One warp per group: rows last to first, lanes high to low, words written back to front into the group's scratch
+// region [base, base + 32 (seg + 2)).  Status: 1 for a symbol outside [0, Q), 2 for a symbol of frequency 0.
+__global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_encode_kernel(const int *__restrict__ qidx,
+                                                                                  const unsigned *__restrict__ cum,
+                                                                                  SharedShape s,
+                                                                                  unsigned short *__restrict__ scratch,
+                                                                                  long long *__restrict__ sizes,
+                                                                                  int *__restrict__ status) {
+    extern __shared__ unsigned sh_tab[];   // [Q + 1]
+    const int plane = blockIdx.y;
+    const long long G = s.gbase[plane + 1] - s.gbase[plane];
+    if ((long long)blockIdx.x * kSharedWarps >= G) return;   // CTA-uniform
+    load_plane_cum(sh_tab, cum, plane, s.Q);
+    __syncthreads();
+    const long long g = (long long)blockIdx.x * kSharedWarps + (threadIdx.x >> 5);
+    if (g >= G) return;
+    const int lane = threadIdx.x & 31;
+    const long long seg = s.seg[plane];
+    const long long r0 = g * seg;
+    const long long len = min(seg, s.rows - r0);
+    const int *src = qidx + (long long)plane * s.n + r0 * 32 + lane;
+    const unsigned top = 1u << s.P;
+    const int fshift = 32 - s.P;
+    const long long base = s.sbase[plane] + g * 32 * (seg + 2);
+    long long pos = base + 32 * (seg + 2);
+    const long long end = pos;
+    unsigned x = kRansL;
+    int bad = 0;
+    const unsigned lt = lanemask_lt();
+
+    int cur[kEncBlock], nxt[kEncBlock];
+#pragma unroll
+    for (int k = 0; k < kEncBlock; ++k) {
+        const long long t = len - 1 - k;
+        cur[k] = (t >= 0 && lane < shared_row_lanes(s, r0 + t)) ? __ldg(src + t * 32) : 0;
+    }
+    for (long long t0 = len - 1; t0 >= 0; t0 -= kEncBlock) {
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) {
+            const long long t = t0 - kEncBlock - k;
+            nxt[k] = (t >= 0 && lane < shared_row_lanes(s, r0 + t)) ? __ldg(src + t * 32) : 0;
+        }
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) {
+            if (t0 - k < 0) break;                         // warp-uniform
+            const bool active = lane < shared_row_lanes(s, r0 + t0 - k);
+            const int sym = cur[k];
+            unsigned lo = 0, f = top;                      // f = 2^P leaves the state unchanged
+            if (active) {
+                if (sym < 0 || sym >= s.Q) {
+                    bad |= 1;
+                } else {
+                    lo = sh_tab[sym];
+                    f = sh_tab[sym + 1] - lo;
+                    if (f == 0) { bad |= 2; lo = 0; f = top; }
+                }
+            }
+            const bool emit = active && (unsigned long long)x >= ((unsigned long long)f << fshift);
+            const unsigned mask = __ballot_sync(0xffffffffu, emit);
+            pos -= __popc(mask);
+            if (emit) {
+                scratch[pos + __popc(mask & lt)] = (unsigned short)(x & 0xffffu);
+                x >>= 16;
+            }
+            if (active) x = ((x / f) << s.P) + (x % f) + lo;
+        }
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) cur[k] = nxt[k];
+    }
+    const int nact = shared_row_lanes(s, r0);
+    pos -= 2 * nact;
+    if (lane < nact) {
+        scratch[pos + 2 * lane] = (unsigned short)(x & 0xffffu);
+        scratch[pos + 2 * lane + 1] = (unsigned short)(x >> 16);
+    }
+    if (lane == 0) sizes[s.gbase[plane] + g] = end - pos;
+    bad = __reduce_or_sync(0xffffffffu, bad);
+    if (bad && lane == 0) atomicOr(status, bad);
+}
+
+// One CTA: the offset tables of every plane, each group's destination and the payload size in bytes.  (The minimum of
+// one CTA per SM lets ptxas use more than 32 registers, which keeps the plane loop free of spills.)
+__global__ void __launch_bounds__(1024, 1) vbq_rans_shared_scan_kernel(const long long *__restrict__ sizes,
+                                                                   long long *__restrict__ dst, SharedShape s,
+                                                                   unsigned short *__restrict__ out,
+                                                                   long long *__restrict__ out_bytes) {
+    __shared__ long long sh_warp[32];
+    long long plane_start = 0;
+    for (int p = 0; p < s.n_planes; ++p)
+        plane_start = scan_plane(sizes + s.gbase[p], dst + s.gbase[p], s.gbase[p + 1] - s.gbase[p], plane_start, out,
+                                 sh_warp);
+    if (threadIdx.x == 0) *out_bytes = 2 * plane_start;
+}
+
+// One CTA per group of the call: move its words from the end of its scratch region to their place in the payload.
+__global__ void vbq_rans_shared_compact_kernel(const unsigned short *__restrict__ scratch,
+                                               const long long *__restrict__ sizes, const long long *__restrict__ dst,
+                                               SharedShape s, unsigned short *__restrict__ out) {
+    const long long gid = blockIdx.x;
+    int p = 0;
+    while (s.gbase[p + 1] <= gid) ++p;
+    const long long g = gid - s.gbase[p];
+    const long long end = s.sbase[p] + (g + 1) * 32 * (s.seg[p] + 2);
+    const long long n = sizes[gid];
+    const unsigned short *src = scratch + end - n;
+    unsigned short *d = out + dst[gid];
+    for (long long i = threadIdx.x; i < n; i += blockDim.x) d[i] = src[i];
+}
+
+// Same CTA layout as the encoder.  Shared memory: the plane's cum table [Q + 1] and the coarse index
+// idx[b] = the largest s < Q with cum[s] <= b << (P - 8), b = 0..256, which brackets the decoded symbol of a slot in
+// bucket b between idx[b] and idx[b + 1].  Word windows and the deferred z_hat stores as in vbq_rans_decode_kernel.
+__global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_kernel(
+        const unsigned short *__restrict__ words, long long n_words, const long long *__restrict__ bounds,
+        const unsigned *__restrict__ cum, SharedShape s, const float *__restrict__ code_points,
+        int *__restrict__ qidx, float *__restrict__ zhat, int *__restrict__ status) {
+    extern __shared__ unsigned sh_tab[];   // [Q + 1] then [kRansBuckets + 1] uint16
+    unsigned short *sh_idx = (unsigned short *)(sh_tab + s.Q + 1);
+    const int plane = blockIdx.y;
+    const long long G = s.gbase[plane + 1] - s.gbase[plane];
+    if ((long long)blockIdx.x * kSharedWarps >= G) return;   // CTA-uniform
+    load_plane_cum(sh_tab, cum, plane, s.Q);
+    __syncthreads();
+    const int bshift = s.P - 8;
+    const unsigned top = 1u << s.P;
+    for (int b = threadIdx.x; b <= kRansBuckets; b += blockDim.x) {
+        const unsigned v = (unsigned)b << bshift;
+        int lo = 0, hi = s.Q - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (sh_tab[mid] <= v) lo = mid; else hi = mid - 1;
+        }
+        sh_idx[b] = (unsigned short)lo;
+    }
+    __syncthreads();
+
+    const long long g = (long long)blockIdx.x * kSharedWarps + (threadIdx.x >> 5);
+    if (g >= G) return;
+    const int lane = threadIdx.x & 31;
+    const long long seg = s.seg[plane];
+    const long long r0 = g * seg;
+    const long long len = min(seg, s.rows - r0);
+    const int nact = shared_row_lanes(s, r0);
+    const long long gid = s.gbase[plane] + g;
+    long long start = bounds[2 * gid], end = bounds[2 * gid + 1];
+    int err = 0;
+    if (start < 0 || end > n_words || end - start < 2ll * nact) { err = 4; end = start = 0; }
+    const long long out0 = (long long)plane * s.n + r0 * 32 + lane;
+    const unsigned lt = lanemask_lt();
+
+    unsigned x = kRansL;
+    if (!err && lane < nact)
+        x = (unsigned)__ldg(words + start + 2 * lane) | ((unsigned)__ldg(words + start + 2 * lane + 1) << 16);
+    if (__any_sync(0xffffffffu, lane < nact && x < kRansL)) err |= 4;
+    long long pos = start + 2 * nact;
+    long long wbase = pos;
+    unsigned w0 = ld_word(words, wbase + lane, end), w1 = ld_word(words, wbase + 32 + lane, end);
+    unsigned w2 = ld_word(words, wbase + 64 + lane, end), w3 = ld_word(words, wbase + 96 + lane, end);
+
+    float zprev[kDecBlock];
+    long long tprev = -1;
+    for (long long t0 = 0; t0 < len && !err; t0 += kDecBlock) {
+        int sy[kDecBlock];
+#pragma unroll
+        for (int k = 0; k < kDecBlock; ++k) {
+            sy[k] = 0;
+            if (t0 + k >= len) break;                      // warp-uniform
+            const bool active = lane < shared_row_lanes(s, r0 + t0 + k);
+            const unsigned slot = x & (top - 1);
+            int lo = sh_idx[slot >> bshift], hi = sh_idx[(slot >> bshift) + 1];
+            while (lo < hi) {
+                const int mid = (lo + hi + 1) >> 1;
+                if (sh_tab[mid] <= slot) lo = mid; else hi = mid - 1;
+            }
+            const unsigned c0 = sh_tab[lo];
+            const unsigned f = sh_tab[lo + 1] - c0;
+            if (active) x = f * (x >> s.P) + slot - c0;
+            const bool need = active && x < kRansL;
+            const unsigned mask = __ballot_sync(0xffffffffu, need);
+            const int n = __popc(mask);
+            if (pos + n > end) { err |= 1; break; }
+            const int rel = (int)(pos - wbase) + __popc(mask & lt);   // < 64 for the lanes that read
+            const unsigned a = __shfl_sync(0xffffffffu, w0, rel & 31), b = __shfl_sync(0xffffffffu, w1, rel & 31);
+            if (need) x = (x << 16) | (rel < 32 ? a : b);
+            pos += n;
+            if (pos - wbase >= 32) {
+                w0 = w1; w1 = w2; w2 = w3;
+                wbase += 32;
+                w3 = ld_word(words, wbase + 96 + lane, end);
+            }
+            sy[k] = lo;
+        }
+        if (zhat && tprev >= 0) {
+#pragma unroll
+            for (int k = 0; k < kDecBlock; ++k) zhat[out0 + (tprev + k) * 32] = zprev[k];   // a full block, full rows
+        }
+        if (err) break;
+#pragma unroll
+        for (int k = 0; k < kDecBlock; ++k) {
+            if (t0 + k < len && lane < shared_row_lanes(s, r0 + t0 + k)) {
+                if (qidx) qidx[out0 + (t0 + k) * 32] = sy[k];
+                if (zhat) zprev[k] = __ldg(code_points + sy[k]);
+            }
+        }
+        tprev = t0;
+    }
+    if (zhat && tprev >= 0 && !err) {
+#pragma unroll
+        for (int k = 0; k < kDecBlock; ++k)
+            if (tprev + k < len && lane < shared_row_lanes(s, r0 + tprev + k)) zhat[out0 + (tprev + k) * 32] = zprev[k];
+    }
+    if (!err && (__any_sync(0xffffffffu, lane < nact && x != kRansL) || pos != end)) err |= 2;
+    if (err && lane == 0) atomicOr(status, err);
+}
+
 }  // namespace
 
 extern "C" long long vbq_rans_workspace_bytes(int n_planes, int items, long long item_rows, int C, long long seg_rows) {
@@ -414,6 +690,91 @@ extern "C" int vbq_rans_decode(const unsigned short *d_payload, long long payloa
     VBQ_ENSURE_MAX_SMEM(vbq_rans_decode_kernel, dev);
     vbq_rans_decode_kernel<<<grid, kRansWarps * 32, smem, st>>>(d_payload, payload_words, d_group_bounds, d_cum, s,
                                                                 d_code_points, d_qidx, d_zhat, d_status);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+extern "C" long long vbq_rans_shared_workspace_bytes(int n_planes, long long n, const long long *seg_rows) {
+    SharedShape s;
+    if (shared_shape("vbq_rans_shared_workspace_bytes", n_planes, n, seg_rows, 0, 16, &s) != VBQ_OK) return -1;
+    const long long G = s.gbase[n_planes];
+    return 2 * align256(8 * G) + align256(2 * s.sbase[n_planes]);
+}
+
+extern "C" long long vbq_rans_shared_payload_bound(int n_planes, long long n, const long long *seg_rows) {
+    SharedShape s;
+    if (shared_shape("vbq_rans_shared_payload_bound", n_planes, n, seg_rows, 0, 16, &s) != VBQ_OK) return -1;
+    long long words = 0;
+    for (int p = 0; p < n_planes; ++p) {
+        const long long G = s.gbase[p + 1] - s.gbase[p];
+        const long long lanes = G ? 32 * (G - 1) + min(32ll, n - 32 * (G - 1) * s.seg[p]) : 0;
+        words += 2 * G + n + 2 * lanes;
+    }
+    return 2 * words;
+}
+
+extern "C" int vbq_rans_shared_encode(const int *d_qidx, int n_planes, long long n, const long long *seg_rows, int N,
+                                      int prob_bits, const unsigned *d_cum, unsigned short *d_payload,
+                                      long long payload_bytes, long long *d_payload_size, int *d_status,
+                                      void *d_workspace, long long workspace_bytes, void *stream) {
+    SharedShape s;
+    RETURN_IF(shared_shape("vbq_rans_shared_encode", n_planes, n, seg_rows, N, prob_bits, &s));
+    const long long G = s.gbase[n_planes];
+    if (!d_cum || !d_payload || !d_payload_size || !d_status || (G > 0 && (!d_qidx || !d_workspace)))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_shared_encode: null pointer");
+    const long long bound = vbq_rans_shared_payload_bound(n_planes, n, seg_rows);
+    if (payload_bytes < bound)
+        return vbq_fail(VBQ_ERR_WORKSPACE, "vbq_rans_shared_encode: payload capacity %lld < "
+                        "vbq_rans_shared_payload_bound %lld", payload_bytes, bound);
+    const long long need = vbq_rans_shared_workspace_bytes(n_planes, n, seg_rows);
+    if (G > 0 && workspace_bytes < need)
+        return vbq_fail(VBQ_ERR_WORKSPACE, "vbq_rans_shared_encode: workspace %lld < %lld bytes", workspace_bytes, need);
+    if (((uintptr_t)d_payload & 1) || ((uintptr_t)d_cum & 3) || ((uintptr_t)d_workspace & 7) ||
+        ((uintptr_t)d_qidx & 3) || ((uintptr_t)d_payload_size & 7) || ((uintptr_t)d_status & 3))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_shared_encode: misaligned pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int), st));
+    if (G == 0) {
+        CUDA_TRY(cudaMemsetAsync(d_payload_size, 0, sizeof(long long), st));
+        return VBQ_OK;
+    }
+    char *ws = (char *)d_workspace;
+    long long *sizes = (long long *)ws;
+    long long *dst = (long long *)(ws + align256(8 * G));
+    unsigned short *scratch = (unsigned short *)(ws + 2 * align256(8 * G));
+    const dim3 grid((unsigned)((s.max_groups + kSharedWarps - 1) / kSharedWarps), n_planes);
+    const size_t smem = (size_t)(s.Q + 1) * sizeof(unsigned);
+    vbq_rans_shared_encode_kernel<<<grid, kSharedWarps * 32, smem, st>>>(d_qidx, d_cum, s, scratch, sizes, d_status);
+    CUDA_TRY(cudaGetLastError());
+    vbq_rans_shared_scan_kernel<<<1, 1024, 0, st>>>(sizes, dst, s, d_payload, d_payload_size);
+    CUDA_TRY(cudaGetLastError());
+    vbq_rans_shared_compact_kernel<<<(unsigned)G, 256, 0, st>>>(scratch, sizes, dst, s, d_payload);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+extern "C" int vbq_rans_shared_decode(const unsigned short *d_payload, long long payload_words,
+                                      const long long *d_group_bounds, int n_planes, long long n,
+                                      const long long *seg_rows, int N, int prob_bits, const unsigned *d_cum,
+                                      const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status,
+                                      void *stream) {
+    SharedShape s;
+    RETURN_IF(shared_shape("vbq_rans_shared_decode", n_planes, n, seg_rows, N, prob_bits, &s));
+    if (payload_words < 0)
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "vbq_rans_shared_decode: payload_words=%lld", payload_words);
+    const long long G = s.gbase[n_planes];
+    if (!d_cum || !d_status || (d_zhat && !d_code_points) || (G > 0 && (!d_payload || !d_group_bounds)))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_shared_decode: null pointer");
+    if (((uintptr_t)d_payload & 1) || ((uintptr_t)d_cum & 3) || ((uintptr_t)d_group_bounds & 7) ||
+        ((uintptr_t)d_qidx & 3) || ((uintptr_t)d_zhat & 3) || ((uintptr_t)d_code_points & 3) || ((uintptr_t)d_status & 3))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_shared_decode: misaligned pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int), st));
+    if (G == 0) return VBQ_OK;
+    const dim3 grid((unsigned)((s.max_groups + kSharedWarps - 1) / kSharedWarps), n_planes);
+    const size_t smem = (size_t)(s.Q + 1) * sizeof(unsigned) + (kRansBuckets + 1) * sizeof(unsigned short);
+    vbq_rans_shared_decode_kernel<<<grid, kSharedWarps * 32, smem, st>>>(d_payload, payload_words, d_group_bounds, d_cum,
+                                                                       s, d_code_points, d_qidx, d_zhat, d_status);
     CUDA_TRY(cudaGetLastError());
     return VBQ_OK;
 }

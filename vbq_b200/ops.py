@@ -5,6 +5,7 @@ hand-written sm_100a kernels.  Every op raises if the library is missing or the 
 there is deliberately no CPU implementation (north_star: "no CPU fallback")."""
 from __future__ import annotations
 
+import ctypes
 from typing import List, Optional
 
 import torch
@@ -644,4 +645,67 @@ def rans_decode(words: torch.Tensor, bounds: torch.Tensor, cum: torch.Tensor, it
                                      seg_rows, max_bits, prob_bits, _ptr(cum), _ptr(code_points), _ptr(q), _ptr(z),
                                      status.data_ptr(), _stream(dev))
     _lib.check(st, "vbq_rans_decode")
+    return q, z, status
+
+
+# ------------------------------------------------------------------------------------------------------
+# entropy coding with one shared table per plane, symbols as one flat sequence (word embeddings; include/vbq_b200.h)
+# ------------------------------------------------------------------------------------------------------
+def _seg_array(seg_rows, n_planes):
+    seg = [int(seg_rows)] * n_planes if isinstance(seg_rows, int) else [int(x) for x in seg_rows]
+    if len(seg) != n_planes:
+        raise ValueError("vbq_b200: %d seg_rows for %d planes" % (len(seg), n_planes))
+    return (ctypes.c_longlong * n_planes)(*seg)
+
+
+def rans_shared_payload_bound(n_planes: int, n: int, seg_rows) -> int:
+    return int(_lib.load().vbq_rans_shared_payload_bound(n_planes, n, _seg_array(seg_rows, n_planes)))
+
+
+def rans_shared_encode(qidx: torch.Tensor, cum: torch.Tensor, max_bits: int, prob_bits: int, seg_rows):
+    """qidx (n_planes, n) int32 and cum (n_planes, Q+1) int32 (the uint32 cum tables of coding.cum_table_shared);
+    seg_rows: an int or one per plane -> (payload int16 words of vbq_rans_shared_payload_bound bytes, payload size in
+    bytes as a 1-element int64 tensor, status int32 tensor: bit 1 a symbol outside [0, Q), bit 2 a symbol of
+    frequency 0): one launch for all planes, no synchronisation."""
+    _need_cuda("qidx", qidx, torch.int32, 2)
+    _need_cuda("cum", cum, torch.int32, 2)
+    n_planes, n = qidx.shape
+    seg = _seg_array(seg_rows, n_planes)
+    lib = _lib.load()
+    bound = lib.vbq_rans_shared_payload_bound(n_planes, n, seg)
+    ws_bytes = lib.vbq_rans_shared_workspace_bytes(n_planes, n, seg)
+    if bound < 0 or ws_bytes < 0:
+        raise ValueError("vbq_b200: bad rANS shape: %s" % lib.vbq_last_error().decode())
+    dev = qidx.device
+    payload = torch.empty(max(1, bound // 2), dtype=torch.int16, device=dev)
+    size = torch.zeros(1, dtype=torch.int64, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    ws = torch.empty(max(1, ws_bytes), dtype=torch.uint8, device=dev)
+    st = lib.vbq_rans_shared_encode(_ptr(qidx), n_planes, n, seg, max_bits, prob_bits,
+                                    _ptr(cum), payload.data_ptr(), bound, size.data_ptr(),
+                                    status.data_ptr(), ws.data_ptr(), ws_bytes, _stream(dev))
+    _lib.check(st, "vbq_rans_shared_encode")
+    return payload, size, status
+
+
+def rans_shared_decode(words: torch.Tensor, bounds: torch.Tensor, cum: torch.Tensor, n: int, seg_rows, max_bits: int,
+                       prob_bits: int, code_points: Optional[torch.Tensor] = None, want_qidx: bool = True):
+    """words: the payload as int16 words; bounds (groups of all planes, 2) int64 word ranges; cum (n_planes, Q+1)
+    int32.  Returns (qidx or None, zhat or None, status): (n_planes, n) int32 symbols and float32 code_points[q]
+    (code_points (Q,) ascending), and the int32 device status (0 = every group passed the integrity check)."""
+    _need_cuda("words", words, torch.int16, 1)
+    _need_cuda("bounds", bounds, torch.int64, 2)
+    _need_cuda("cum", cum, torch.int32, 2)
+    n_planes = cum.shape[0]
+    dev = words.device
+    q = torch.empty((n_planes, n), dtype=torch.int32, device=dev) if want_qidx else None
+    z = None
+    if code_points is not None:
+        _need_cuda("code_points", code_points, torch.float32, 1)
+        z = torch.empty((n_planes, n), dtype=torch.float32, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    st = _lib.load().vbq_rans_shared_decode(_ptr(words), words.numel(), _ptr(bounds), n_planes, n,
+                                            _seg_array(seg_rows, n_planes), max_bits, prob_bits, _ptr(cum),
+                                            _ptr(code_points), _ptr(q), _ptr(z), status.data_ptr(), _stream(dev))
+    _lib.check(st, "vbq_rans_shared_decode")
     return q, z, status

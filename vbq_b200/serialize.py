@@ -15,9 +15,17 @@ n_planes, items | uint64 item_rows, seg_rows | uint32 height, flags | per plane:
 its table (`coding.fingerprint`) | [flags & 1: the tables, n_planes*C*Q uint16 entries f-1] | the rANS payload of
 include/vbq_b200.h (per plane: uint32 group end offsets, then the groups' 16-bit words).  `height` is H' of an
 item of H' x W' = item_rows latent rows (0 if unknown).
+
+VBQE (`encode_embeddings` / `decode_embedding`, behind `GaussianCodebook.compress_to_bytes`): one plane of word-embedding
+coordinates coded with the shared-table rANS coder (`vbq_rans_shared_*`), one table for all coordinates.  Layout
+(little endian):  magic b"VBQE" | uint32 N, prob_bits, ndim | ndim uint64 extents of the tensor | uint64 seg_rows |
+float64 empirical_std, beta | uint64 fingerprint of the codebook's float64 code points (`coding.code_points_fingerprint`)
+| the sparse table: uint32 k, k ascending uint16 symbols, k uint32 frequencies (those of every other symbol are 0) |
+the rANS payload (uint32 group end offsets, then the groups' 16-bit words).
 """
 from __future__ import annotations
 
+import math
 import struct
 
 import numpy as np
@@ -211,15 +219,20 @@ def read_header(data: bytes) -> dict:
 
 
 def _group_bounds(words, h):
-    """Check the offset tables of a payload (monotone, every group holding at least its states, inside the payload,
-    nothing left over) -> (n_planes * groups, 2) int64 word ranges."""
+    """The group word ranges of a VBQ2 payload (see _offset_bounds)."""
     C, items = h["C"], h["items"]
     n_segs = -(-h["item_rows"] // h["seg_rows"])
     CG = -(-C // 32)
-    G = items * n_segs * CG
     nact = np.tile(np.minimum(32, C - 32 * np.arange(CG)), items * n_segs).astype(np.int64)
+    return _offset_bounds(words, [nact] * h["n_planes"])
+
+
+def _offset_bounds(words, nacts):
+    """Check the offset tables of a payload whose planes have groups of nacts[p] state lanes each (monotone, every group
+    holding at least its states, inside the payload, nothing left over) -> (all groups, 2) int64 word ranges."""
     bounds, pos = [], 0
-    for _ in range(h["n_planes"]):
+    for nact in nacts:
+        G = nact.size
         if pos + 2 * G > words.size:
             raise ValueError("vbq_b200.serialize: payload truncated in an offset table")
         e = words[pos:pos + 2 * G].astype(np.int64)
@@ -280,4 +293,145 @@ def decode(data: bytes, tables=None, code_points=None, device="cuda", want_qidx:
                                             (4, "bad group range or initial state")) if st & bit)))
     out = {k: v for k, v in h.items() if k not in ("tables", "payload_offset")}
     out.update(qidx=q, zhat=z)
+    return out
+
+
+# ------------------------------------------------------------------------------------------------------
+# VBQE: rANS-coded word embeddings, one shared table per blob
+# ------------------------------------------------------------------------------------------------------
+MAGIC_E = b"VBQE"
+_HDRE = struct.Struct("<4sIII")       # magic, N, prob_bits, ndim; then ndim uint64 extents
+_HDRE2 = struct.Struct("<QddQI")      # seg_rows, empirical_std, beta, code-point fingerprint, used symbols k
+_MAX_NDIM = 32
+
+
+def shared_seg_rows(n: int, seg_rows: int) -> int:
+    """seg_rows as the shared-table coder uses it: a segment longer than the plane is the whole plane."""
+    return max(1, min(int(seg_rows), -(-int(n) // 32)))
+
+
+def shared_nact(n: int, seg_rows: int) -> np.ndarray:
+    """State lanes of every group of a plane of n symbols in the shared-table layout: 32, except for a group that
+    starts on the plane's last, partial row."""
+    seg = shared_seg_rows(n, seg_rows)
+    G = -(-(-(-n // 32)) // seg)
+    return np.minimum(32, n - 32 * seg * np.arange(G, dtype=np.int64))
+
+
+def embedding_header(max_bits, prob_bits, shape, seg_rows, empirical_std, beta, fingerprint, table) -> bytes:
+    """The VBQE header and sparse table of one plane (table: (Q,) integer frequencies)."""
+    t = np.asarray(table, dtype=np.int64)
+    used = np.flatnonzero(t)
+    return b"".join([_HDRE.pack(MAGIC_E, int(max_bits), int(prob_bits), len(shape)),
+                     struct.pack("<%dQ" % len(shape), *[int(d) for d in shape]),
+                     _HDRE2.pack(int(seg_rows), float(empirical_std), float(beta), int(fingerprint), used.size),
+                     used.astype("<u2").tobytes(), t[used].astype("<u4").tobytes()])
+
+
+def encode_embeddings(qidx, tables, max_bits: int, shape, seg_rows, empirical_std: float, betas, fingerprint: int):
+    """Entropy-code L planes of symbols with the shared-table coder in one launch; one VBQE blob per plane.
+
+    qidx: (L, n) int32 CUDA tensor of sorted quantile indices, n = prod(shape).  tables: (L, Q) integer frequencies
+    (`coding.frequency_tables(counts, keep_zeros=True)`).  seg_rows: one per plane.  empirical_std, betas and the
+    code-point fingerprint are recorded for the receiver.  Raises ValueError for a symbol outside [0, Q) or one whose
+    frequency is 0."""
+    L, n = qidx.shape
+    if n != math.prod(shape):
+        raise ValueError("vbq_b200.serialize: %d symbols do not fill shape %s" % (n, tuple(shape)))
+    Q = ops.num_levels(max_bits)
+    t = np.asarray(tables)
+    if t.shape != (L, Q):
+        raise ValueError("vbq_b200.serialize: tables are %s, need (%d, %d)" % (t.shape, L, Q))
+    P = coding.prob_bits_of(t)
+    t = coding.check_shared_tables(t, P)
+    if any(int(x) < 1 for x in seg_rows):
+        raise ValueError("vbq_b200.serialize: seg_rows must be >= 1, got %s" % (list(seg_rows),))
+    seg = [shared_seg_rows(n, x) for x in seg_rows]
+    cum = torch.from_numpy(coding.cum_table_shared(t).view(np.int32)).to(qidx.device)
+    payload, size, status = ops.rans_shared_encode(qidx, cum, max_bits, P, seg)
+    st = int(status.item())
+    if st:
+        raise ValueError("vbq_b200.serialize: " + " and ".join(
+            m for bit, m in ((1, "a symbol lies outside [0, Q) for max_bits=%d" % max_bits),
+                             (2, "a symbol has frequency 0 in its table")) if st & bit))
+    words = payload[:int(size.item()) // 2].cpu().numpy().view(np.uint16)
+    out, pos = [], 0
+    for p in range(L):
+        G = shared_nact(n, seg[p]).size
+        e = words[pos:pos + 2 * G].astype(np.int64)
+        end = pos + 2 * G + (int(e[-2] | (e[-1] << 16)) if G else 0)
+        hdr = embedding_header(max_bits, P, shape, seg[p], empirical_std, betas[p], fingerprint, t[p])
+        out.append(hdr + words[pos:end].astype("<u2").tobytes())
+        pos = end
+    return out
+
+
+def read_embedding_header(data: bytes) -> dict:
+    """Parse and check a VBQE blob on the host: max_bits, prob_bits, shape, seg_rows, empirical_std, beta,
+    fingerprint, table ((Q,) int64 frequencies), and the payload's group word ranges `bounds` and `words`.  Raises
+    ValueError for a bad magic, a truncated blob, a table that is unsorted, out of range or does not sum to
+    2^prob_bits, a malformed offset table or bytes after the payload."""
+    data = memoryview(data)
+    if len(data) < _HDRE.size:
+        raise ValueError("vbq_b200.serialize: %d bytes are too short for a VBQE header" % len(data))
+    magic, N, P, ndim = _HDRE.unpack_from(data, 0)
+    if magic != MAGIC_E:
+        raise ValueError("vbq_b200.serialize: bad magic %r (expected %r)" % (bytes(magic), MAGIC_E))
+    if N > 10 or not 12 <= P <= 16 or ndim > _MAX_NDIM:
+        raise ValueError("vbq_b200.serialize: bad VBQE header (N=%d prob_bits=%d ndim=%d)" % (N, P, ndim))
+    pos = _HDRE.size
+    if len(data) < pos + 8 * ndim + _HDRE2.size:
+        raise ValueError("vbq_b200.serialize: truncated VBQE header")
+    shape = tuple(struct.unpack_from("<%dQ" % ndim, data, pos))
+    pos += 8 * ndim
+    seg_rows, std, beta, fp, k = _HDRE2.unpack_from(data, pos)
+    pos += _HDRE2.size
+    Q = ops.num_levels(N)
+    n = math.prod(shape)
+    if not 1 <= seg_rows <= max(1, -(-n // 32)) or not 1 <= k <= Q:
+        raise ValueError("vbq_b200.serialize: bad VBQE header (seg_rows=%d, %d symbols, %d used)" % (seg_rows, n, k))
+    if n + 66 * -(-n // (32 * seg_rows)) >= 2 ** 32:       # the coder's limit: a plane's worst case in 32-bit offsets
+        raise ValueError("vbq_b200.serialize: %d symbols in segments of %d rows exceed the coder's 32-bit offsets"
+                         % (n, seg_rows))
+    if len(data) < pos + 6 * k:
+        raise ValueError("vbq_b200.serialize: truncated frequency table")
+    sym = np.frombuffer(data, dtype="<u2", count=k, offset=pos).astype(np.int64)
+    freq = np.frombuffer(data, dtype="<u4", count=k, offset=pos + 2 * k).astype(np.int64)
+    pos += 6 * k
+    if (np.diff(sym) <= 0).any() or sym[-1] >= Q:
+        raise ValueError("vbq_b200.serialize: table symbols unsorted or outside [0, %d)" % Q)
+    if (freq < 1).any() or freq.sum() != 1 << P:
+        raise ValueError("vbq_b200.serialize: table frequencies do not sum to 2^%d" % P)
+    table = np.zeros(Q, np.int64)
+    table[sym] = freq
+    rest = len(data) - pos
+    if rest % 2:
+        raise ValueError("vbq_b200.serialize: payload of odd length")
+    words = np.frombuffer(data, dtype="<u2", count=rest // 2, offset=pos)
+    if 2 * -(-n // (32 * seg_rows)) > words.size:      # checked before the per-group arrays are built
+        raise ValueError("vbq_b200.serialize: payload truncated in an offset table")
+    bounds = _offset_bounds(words, [shared_nact(n, seg_rows)])
+    return dict(max_bits=N, prob_bits=P, shape=shape, seg_rows=seg_rows, empirical_std=std, beta=beta,
+                fingerprint=fp, table=table, words=words, bounds=bounds)
+
+
+def decode_embedding(data: bytes, code_points=None, device="cuda", want_qidx: bool = True) -> dict:
+    """Inverse of `encode_embeddings` for one blob: the header fields of `read_embedding_header` plus qidx and zhat,
+    flat (n,) device tensors or None (zhat = code_points[q] for a (Q,) ascending table).  A malformed blob raises
+    ValueError before any launch; a payload that fails the decoder's integrity check raises ValueError after it."""
+    h = read_embedding_header(data)
+    n = math.prod(h["shape"])
+    dev = torch.device(device)
+    w = torch.from_numpy(h["words"].view(np.int16).copy()).to(dev)
+    b = torch.from_numpy(np.ascontiguousarray(h["bounds"], dtype=np.int64)).to(dev)
+    cum = torch.from_numpy(coding.cum_table_shared(h["table"][None]).view(np.int32)).to(dev)
+    cp = None if code_points is None else code_points.to(device=dev, dtype=torch.float32).contiguous()
+    q, z, status = ops.rans_shared_decode(w, b, cum, n, h["seg_rows"], h["max_bits"], h["prob_bits"], cp, want_qidx)
+    st = int(status.item())
+    if st:
+        raise ValueError("vbq_b200.serialize: corrupt VBQE payload (decoder status %d: %s)" % (
+            st, ", ".join(m for bit, m in ((1, "a group ran out of words"), (2, "integrity check failed"),
+                                            (4, "bad group range or initial state")) if st & bit)))
+    out = {k: v for k, v in h.items() if k not in ("words", "bounds")}
+    out.update(qidx=None if q is None else q[0], zhat=None if z is None else z[0])
     return out

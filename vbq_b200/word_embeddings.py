@@ -10,9 +10,11 @@ from __future__ import annotations
 import numpy as np
 import torch
 
-from . import ops
+from . import coding, ops, serialize
 
 _VC = 16  # virtual channels = VBQ_GROUP
+_FLUSH_BUDGET = 0.005   # default segmentation: flushed states cost at most this share of the plane's entropy
+_MIN_SEG_ROWS = 256
 
 
 def empirical_std(means):
@@ -31,6 +33,29 @@ def empirical_entropy(values):
     return float(total * torch.log2(total) - (c * torch.log2(c)).sum())
 
 
+def _entropy_of_counts(counts):
+    """ipynb:452-455 from a count table (the last axis): total log2 total - sum counts log2 counts."""
+    c = np.asarray(counts, dtype=np.float64)
+    total = c.sum(axis=-1)
+    plogp = np.where(c > 0, c * np.log2(np.maximum(c, 1.0)), 0.0).sum(axis=-1)
+    return np.where(total > 0, total * np.log2(np.maximum(total, 1.0)), 0.0) - plogp
+
+
+def default_seg_rows(n: int, entropy_bits: float) -> int:
+    """Rows per segment of the shared-table coder for a plane of n symbols: the most segments whose flushed states
+    (32 lanes x 32 bits per segment) cost at most 0.5 % of the plane's ideal code length, but no segment shorter than
+    256 rows.  More segments mean more warps decoding in parallel."""
+    rows = -(-int(n) // 32)
+    segs = max(1, int(_FLUSH_BUDGET * float(entropy_bits) // 1024))
+    return max(1, min(rows, max(_MIN_SEG_ROWS, -(-rows // segs))))
+
+
+def _pen_f32(beta):
+    """Whether the notebook forms (2 beta) sigma^2 in float32: always, unless beta is a NumPy float64 scalar, which
+    NumPy >= 2 promotes to float64."""
+    return not (isinstance(beta, np.floating) and np.lib.NumpyVersion(np.__version__) >= "2.0.0")
+
+
 class GaussianCodebook:
     """`codepoints` / `lengths` of the notebook (heap order, float64 / int64) plus the device tables."""
 
@@ -46,6 +71,7 @@ class GaussianCodebook:
         pts = ops.gaussian_inverse_cdf(xi_d, None, std_d).reshape(-1)          # norm.ppf(xi, scale=std), float64
         self.codepoints = pts.cpu().numpy()
         self.lengths = np.concatenate([np.full(2 ** n, n, dtype=np.int64) for n in range(N + 1)])
+        self._ascending = torch.sort(pts).values.to(torch.float32)                       # (Q,): z_hat of sorted index q
         self._table = pts.to(torch.float32).reshape(1, -1).repeat(_VC, 1).contiguous()   # (16, Q)
         self._packed = ops.pack_code_points(self._table, N)
         torch.cuda.current_stream(self._table.device).synchronize()
@@ -87,6 +113,22 @@ class GaussianCodebook:
 
         return dict(zhat=unpad(z), qidx=unpad(q), level=unpad(lv), bits=unpad(b), totals=tot)
 
+    def _sorted_index(self, heap, level):
+        """Heap index h of depth d -> sorted index (2 i + 1) 2^(N-d) - 1 with i = h - (2^d - 1)."""
+        i_in = heap - ((1 << level) - 1)
+        return ((2 * i_in + 1) << (self.max_codepoint_length - level)) - 1
+
+    def _add_counts(self, q, counts):
+        """Add the symbols of q (int32 CUDA tensor) to counts (16, Q) int64: `vbq_symbol_histogram` over 16 virtual
+        channels, the ragged tail (fewer than 16 symbols) by bincount."""
+        N = self.max_codepoint_length
+        q = q.reshape(-1)
+        k = (q.numel() // _VC) * _VC
+        if k:
+            ops.symbol_histogram(q[:k].reshape(-1, _VC).contiguous(), N, counts)
+        if k < q.numel():
+            counts[0] += torch.bincount(q[k:].long(), minlength=counts.shape[1])
+
     def beta_sweep(self, means, stds, betas, exact=False, reduce_fn=None, max_chunk_symbols=1 << 29):
         """The rate side of the notebook's beta sweep (ipynb:464-473, :1102-1103: `test_beta` for every beta of
         `np.exp(np.linspace(np.log(0.01), np.log(100000), 50))`): compresses all coordinates with every beta and
@@ -115,22 +157,14 @@ class GaussianCodebook:
                     b = min(n, a + step)
                     _, heap, level = ops.compress_coordinates_f64(m[a:b], s[a:b], cp, per_level, beta, True,
                                                                   want_index=True, want_level=True)
-                    # heap index h of depth d -> sorted index (2 i + 1) 2^(N-d) - 1 with i = h - (2^d - 1)
-                    i_in = heap - ((1 << level) - 1)
-                    q = ((2 * i_in + 1) << (N - level)) - 1
-                    flat = torch.bincount(q.reshape(-1).long(), minlength=Q)
-                    counts[i, 0] += flat
+                    self._add_counts(self._sorted_index(heap, level), counts[i])
         else:
             step = max(_VC, (max_chunk_symbols // max(L, 1) // _VC) * _VC)
             for a in range(0, n, step):
                 b = min(n, a + step)
-                k = ((b - a) // _VC) * _VC
                 q = self.quantize(m[a:b], s[a:b], betas, outputs=ops.OUT_QIDX)['qidx']        # (L, b - a)
                 for i in range(L):
-                    if k:
-                        ops.symbol_histogram(q[i, :k].reshape(-1, _VC).contiguous(), N, counts[i])
-                    if k < b - a:     # the ragged tail (fewer than 16 symbols)
-                        counts[i, 0] += torch.bincount(q[i, k:].long(), minlength=Q)
+                    self._add_counts(q[i], counts[i])
         counts = counts.sum(dim=1)
         if reduce_fn is not None:
             counts = reduce_fn(counts)
@@ -154,12 +188,67 @@ class GaussianCodebook:
         s32 = s.to(device=self.device, dtype=torch.float32).contiguous()
         if exact:
             per_level = self._level_lengths(self.lengths if bitlengths is None else bitlengths)
-            pen_f32 = not (isinstance(beta, np.floating) and np.lib.NumpyVersion(np.__version__) >= "2.0.0")
             out, _, _ = ops.compress_coordinates_f64(
                 m32, s32, torch.from_numpy(self.codepoints).to(self.device),
-                torch.from_numpy(per_level.astype(np.float64)).to(self.device), float(beta), pen_f32)
+                torch.from_numpy(per_level.astype(np.float64)).to(self.device), float(beta), _pen_f32(beta))
         else:
             out = self.quantize(m32, s32, [beta], bitlengths)['zhat'][0]
         if is_np:
             return out.cpu().numpy().astype(np.asarray(means).dtype), None
         return out.to(means.dtype), None
+
+    def compress_to_bytes(self, means, stds, betas, exact=True, prob_bits=coding.DEFAULT_PROB_BITS, seg_rows=None):
+        """Entropy-code the coordinates that `compress_coordinates(means, stds, beta, exact=exact)` chooses, for every
+        beta: returns {beta: bytes}, each a separately decodable VBQE blob (`serialize.read_embedding_header`) that
+        `decompress_from_bytes` turns back into those optima as float32.
+
+        The symbols (sorted quantile indices) are counted on the device, every beta gets one table that gives unused
+        symbols frequency 0 (`coding.frequency_tables(counts, keep_zeros=True)`), and all betas are coded in one launch
+        of the shared-table rANS coder.  ``seg_rows`` (rows of 32 coordinates per independently decodable segment)
+        defaults per beta to `default_seg_rows`.  The coder holds N <= 10."""
+        N = self.max_codepoint_length
+        if N > 10:
+            raise ValueError("vbq_b200: compress_to_bytes codes N <= 10, this codebook has N=%d" % N)
+        m = means if isinstance(means, torch.Tensor) else torch.as_tensor(np.asarray(means))
+        s = stds if isinstance(stds, torch.Tensor) else torch.as_tensor(np.asarray(stds))
+        shape = tuple(m.shape)
+        m32 = m.to(device=self.device, dtype=torch.float32).contiguous().reshape(-1)
+        s32 = s.to(device=self.device, dtype=torch.float32).contiguous().reshape(-1)
+        n = m32.numel()
+        Q = ops.num_levels(N)
+        if exact:
+            cp = torch.from_numpy(self.codepoints).to(self.device)
+            per_level = torch.from_numpy(self._level_lengths(self.lengths).astype(np.float64)).to(self.device)
+        planes = torch.empty((len(betas), n), dtype=torch.int32, device=self.device)
+        counts = torch.zeros((len(betas), _VC, Q), dtype=torch.int64, device=self.device)
+        for i, beta in enumerate(betas):
+            if exact:
+                _, heap, level = ops.compress_coordinates_f64(m32, s32, cp, per_level, float(beta), _pen_f32(beta),
+                                                              want_index=True, want_level=True)
+                planes[i] = self._sorted_index(heap, level)
+            else:
+                planes[i] = self.quantize(m32, s32, [beta], outputs=ops.OUT_QIDX)['qidx'][0]
+            self._add_counts(planes[i], counts[i])
+        counts = counts.sum(dim=1).cpu().numpy()
+        tables = np.stack([coding.frequency_tables(c, prob_bits, keep_zeros=True)[0] for c in counts])
+        if seg_rows is None:
+            seg = [default_seg_rows(n, h) for h in _entropy_of_counts(counts)]
+        else:
+            seg = [int(seg_rows)] * len(betas)
+        blobs = serialize.encode_embeddings(planes, tables, N, shape, seg, self.empirical_std,
+                                            [float(b) for b in betas], coding.code_points_fingerprint(self.codepoints))
+        return dict(zip(betas, blobs))
+
+    def decompress_from_bytes(self, blob):
+        """The float32 optima of a `compress_to_bytes` blob as a device tensor of the original shape.  Raises
+        ValueError if the blob was made with another N, empirical_std or code points, or is malformed or corrupt.  A
+        receiver that has only the blob builds the codebook from it:
+        ``h = serialize.read_embedding_header(blob); GaussianCodebook(h["empirical_std"], h["max_bits"])``."""
+        h = serialize.read_embedding_header(blob)
+        if (h["max_bits"] != self.max_codepoint_length or h["empirical_std"] != self.empirical_std
+                or h["fingerprint"] != coding.code_points_fingerprint(self.codepoints)):
+            raise ValueError("vbq_b200: the blob was coded with another codebook (N=%d, empirical_std=%r) than this "
+                             "one (N=%d, empirical_std=%r) or with other code points"
+                             % (h["max_bits"], h["empirical_std"], self.max_codepoint_length, self.empirical_std))
+        out = serialize.decode_embedding(blob, self._ascending, self.device, want_qidx=False)
+        return out["zhat"].reshape(h["shape"])
