@@ -310,6 +310,54 @@ int vbq_rans_shared_decode(const unsigned short *d_payload, long long payload_wo
                            const unsigned *d_cum, const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status,
                            void *stream);
 
+/* ---- row access into one shared-table plane: decoder checkpoints (DESIGN.md §8e) ---------------------------------
+ *
+ * A decoder's state at any row is fully determined by the stream, so one full pass can record it every K rows and a
+ * later decode can start there.  Both functions take ONE plane (n symbols, seg_rows, N, prob_bits, d_cum (Q+1) uint32,
+ * d_group_bounds (groups, 2) int64 word ranges into d_payload) as vbq_rans_shared_decode does, and checkpoint_rows
+ * K >= 1; a K of at least the (clamped) segment length is treated as that length and records no checkpoint.
+ *
+ * CHECKPOINT INDEX (normative).  In segment g (rows r0 = g seg_rows .. r0 + len - 1), checkpoint j = 1 .. (len - 1) / K
+ * is the decoder just before row r0 + j K: the word position of the next unread word as a uint32 offset from the
+ * group's start word (its range start in d_group_bounds), and the 32 lane states as uint32 (a lane without a symbol in
+ * the segment keeps 2^16).  It is entry c = g ((seg_rows - 1) / K) + j - 1 of d_offsets (M,) and d_states (M, 32), so
+ * every full segment has (seg_rows - 1) / K entries and only the last segment may have fewer.  The segment start
+ * (j = 0) is not stored: its states are the group's first words.  M = vbq_rans_shared_checkpoint_count(n, seg_rows, K);
+ * the index takes 132 M bytes.
+ *
+ * vbq_rans_shared_checkpoints decodes the plane exactly as vbq_rans_shared_decode (same bounds, same status bits 1, 2
+ * and 4, the same final integrity rule), writes no symbols and writes the index.
+ *
+ * vbq_rans_shared_decode_rows gathers embedding rows.  The plane is (n / row_size, row_size) symbols (row_size = D =
+ * prod(shape[1:]) >= 1, dividing n); d_rows (n_req,) int64 are sorted, unique embedding rows.  One warp runs each of
+ * the n_items WORK ITEMS of d_items: it restores checkpoint `checkpoint` of segment `segment` (0 = the segment's
+ * start), decodes coder rows up to `last_row` (inside that checkpoint's interval [r0 + j K, min(r0 + (j+1) K, r0 +
+ * len))) and writes every decoded symbol t (row t / 32, lane t % 32) whose embedding row t / D equals d_rows[u] for a u
+ * in [lo, hi) to element (u, t - D d_rows[u]) of d_qidx (int32) and/or d_zhat (float32 d_code_points[q]), both
+ * (n_req, D).  Items that cover disjoint coder rows write disjoint elements.  The kernel checks every field of every
+ * item (segment and checkpoint in range, last_row inside the interval, 0 <= lo <= hi <= n_req, d_rows[lo..hi) strictly
+ * increasing and below n / D): a bad item sets status bit 8 and writes nothing.  A partial decode cannot apply the
+ * final-state rule, so only bits 1 (ran out of words) and 4 (bad group range or restored state below 2^16) remain.
+ * Status codes: VBQ_ERR_BAD_SHAPE also for K < 1, row_size < 1 or not dividing n, n_req < 0 or above n / row_size. */
+typedef struct {
+    long long segment;      /* group of the plane */
+    long long checkpoint;   /* j: 0 = the segment's start, else index entry segment ((seg_rows - 1) / K) + j - 1 */
+    long long last_row;     /* the last coder row to decode, inside the checkpoint's interval */
+    long long lo, hi;       /* the slice [lo, hi) of d_rows this item writes */
+} vbq_rans_lookup_item;     /* 40 bytes: an (n_items, 5) int64 array */
+
+long long vbq_rans_shared_checkpoint_count(long long n, long long seg_rows, long long checkpoint_rows);
+int vbq_rans_shared_checkpoints(const unsigned short *d_payload, long long payload_words,
+                                const long long *d_group_bounds, long long n, long long seg_rows, int N, int prob_bits,
+                                const unsigned *d_cum, long long checkpoint_rows, unsigned *d_offsets,
+                                unsigned *d_states, int *d_status, void *stream);
+int vbq_rans_shared_decode_rows(const unsigned short *d_payload, long long payload_words,
+                                const long long *d_group_bounds, long long n, long long seg_rows, int N, int prob_bits,
+                                const unsigned *d_cum, long long checkpoint_rows, const unsigned *d_offsets,
+                                const unsigned *d_states, const vbq_rans_lookup_item *d_items, long long n_items,
+                                const long long *d_rows, long long n_req, long long row_size,
+                                const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status, void *stream);
+
 /* ---- stand-alone operator forms------------------------------------------------------------------------------- */
 
 /* ChannelwisePriorCDFQuantizer.get_all_N_bit_intervals (quantizer.py:65-80): d_mu (rows, C) -> d_left, d_right

@@ -85,6 +85,10 @@ SIGNATURES = {
     "vbq_rans_shared_payload_bound": (_ll, [_i, _ll, _p]),
     "vbq_rans_shared_encode": (_i, [_p, _i, _ll, _p, _i, _i, _p, _p, _ll, _p, _p, _p, _ll, _p]),
     "vbq_rans_shared_decode": (_i, [_p, _ll, _p, _i, _ll, _p, _i, _i, _p, _p, _p, _p, _p, _p]),
+    "vbq_rans_shared_checkpoint_count": (_ll, [_ll, _ll, _ll]),
+    "vbq_rans_shared_checkpoints": (_i, [_p, _ll, _p, _ll, _ll, _i, _i, _p, _ll, _p, _p, _p, _p]),
+    "vbq_rans_shared_decode_rows": (_i, [_p, _ll, _p, _ll, _ll, _i, _i, _p, _ll, _p, _p, _p, _ll, _p, _ll, _ll,
+                                         _p, _p, _p, _p, _p]),
 }
 
 _lib = None

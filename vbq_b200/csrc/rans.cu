@@ -15,6 +15,8 @@
 //   * the payload of a plane is its group end offset table (uint32 per group, in 16-bit words from the start of the
 //     plane's group data, groups in (item, segment, channel group) order) followed by the groups, each its states and
 //     then its words.  The payload of a call is its planes' payloads back to back.
+#include <climits>
+
 #include "common.h"
 
 namespace {
@@ -506,22 +508,14 @@ __global__ void vbq_rans_shared_compact_kernel(const unsigned short *__restrict_
     for (long long i = threadIdx.x; i < n; i += blockDim.x) d[i] = src[i];
 }
 
-// Same CTA layout as the encoder.  Shared memory: the plane's cum table [Q + 1] and the coarse index
+// Shared memory of the shared-table decoders: the plane's cum table [Q + 1] and the coarse index
 // idx[b] = the largest s < Q with cum[s] <= b << (P - 8), b = 0..256, which brackets the decoded symbol of a slot in
-// bucket b between idx[b] and idx[b + 1].  Word windows and the deferred z_hat stores as in vbq_rans_decode_kernel.
-__global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_kernel(
-        const unsigned short *__restrict__ words, long long n_words, const long long *__restrict__ bounds,
-        const unsigned *__restrict__ cum, SharedShape s, const float *__restrict__ code_points,
-        int *__restrict__ qidx, float *__restrict__ zhat, int *__restrict__ status) {
-    extern __shared__ unsigned sh_tab[];   // [Q + 1] then [kRansBuckets + 1] uint16
-    unsigned short *sh_idx = (unsigned short *)(sh_tab + s.Q + 1);
-    const int plane = blockIdx.y;
-    const long long G = s.gbase[plane + 1] - s.gbase[plane];
-    if ((long long)blockIdx.x * kSharedWarps >= G) return;   // CTA-uniform
+// bucket b between idx[b] and idx[b + 1].  Every thread of the CTA takes part (two barriers).
+__device__ __forceinline__ void stage_shared_table(unsigned *sh_tab, unsigned short *sh_idx,
+                                                   const unsigned *__restrict__ cum, int plane, const SharedShape &s) {
     load_plane_cum(sh_tab, cum, plane, s.Q);
     __syncthreads();
     const int bshift = s.P - 8;
-    const unsigned top = 1u << s.P;
     for (int b = threadIdx.x; b <= kRansBuckets; b += blockDim.x) {
         const unsigned v = (unsigned)b << bshift;
         int lo = 0, hi = s.Q - 1;
@@ -532,6 +526,75 @@ __global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_kern
         sh_idx[b] = (unsigned short)lo;
     }
     __syncthreads();
+}
+
+// A warp's decoder of one group in the shared-table layout is the lanes' states x, the group's next word pos and its
+// end, and a window of the next 128 words in registers (w0..w3, one word per lane each; wbase <= pos < wbase + 32).
+// The helpers take them as references rather than as one struct: with a struct ptxas adds register moves to every row
+// of the unrolled decode loop.
+
+// (Re)load the window at pos: after the initial states, or at a checkpoint.
+__device__ __forceinline__ void shared_load_window(const unsigned short *__restrict__ words, long long pos,
+                                                   long long end, int lane, long long &wbase, unsigned &w0,
+                                                   unsigned &w1, unsigned &w2, unsigned &w3) {
+    wbase = pos;
+    w0 = ld_word(words, wbase + lane, end);
+    w1 = ld_word(words, wbase + 32 + lane, end);
+    w2 = ld_word(words, wbase + 64 + lane, end);
+    w3 = ld_word(words, wbase + 96 + lane, end);
+}
+
+// Row r of the plane in the shared-table decoder (the DECODER rule of include/vbq_b200.h): coarse index, binary
+// search, state update and renormalisation of the lanes that hold a symbol on this row, then the window moves on.
+// Returns false on every lane if the group ran out of words (the state is then undefined), else the lane's symbol is
+// in `sym`.
+__device__ __forceinline__ bool shared_decode_row(unsigned &x, long long &pos, long long &wbase, long long end,
+                                                  unsigned &w0, unsigned &w1, unsigned &w2, unsigned &w3,
+                                                  const SharedShape &s, long long r, const unsigned *sh_tab,
+                                                  const unsigned short *sh_idx,
+                                                  const unsigned short *__restrict__ words, int lane, unsigned lt,
+                                                  int &sym) {
+    const int bshift = s.P - 8;
+    const unsigned top = 1u << s.P;
+    const bool active = lane < shared_row_lanes(s, r);
+    const unsigned slot = x & (top - 1);
+    int lo = sh_idx[slot >> bshift], hi = sh_idx[(slot >> bshift) + 1];
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (sh_tab[mid] <= slot) lo = mid; else hi = mid - 1;
+    }
+    const unsigned c0 = sh_tab[lo];
+    const unsigned f = sh_tab[lo + 1] - c0;
+    x = active ? f * (x >> s.P) + slot - c0 : x;   // a select: ptxas would branch around the table loads for an if
+    const bool need = active && x < kRansL;
+    const unsigned mask = __ballot_sync(0xffffffffu, need);
+    const int n = __popc(mask);
+    if (pos + n > end) return false;
+    const int rel = (int)(pos - wbase) + __popc(mask & lt);   // < 64 for the lanes that read
+    const unsigned a = __shfl_sync(0xffffffffu, w0, rel & 31), b = __shfl_sync(0xffffffffu, w1, rel & 31);
+    if (need) x = (x << 16) | (rel < 32 ? a : b);
+    pos += n;
+    if (pos - wbase >= 32) {
+        w0 = w1; w1 = w2; w2 = w3;
+        wbase += 32;
+        w3 = ld_word(words, wbase + 96 + lane, end);
+    }
+    sym = lo;
+    return true;
+}
+
+// Same CTA layout as the encoder; shared memory as stage_shared_table.  Deferred z_hat stores as in
+// vbq_rans_decode_kernel.
+__global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_kernel(
+        const unsigned short *__restrict__ words, long long n_words, const long long *__restrict__ bounds,
+        const unsigned *__restrict__ cum, SharedShape s, const float *__restrict__ code_points,
+        int *__restrict__ qidx, float *__restrict__ zhat, int *__restrict__ status) {
+    extern __shared__ unsigned sh_tab[];   // [Q + 1] then [kRansBuckets + 1] uint16
+    unsigned short *sh_idx = (unsigned short *)(sh_tab + s.Q + 1);
+    const int plane = blockIdx.y;
+    const long long G = s.gbase[plane + 1] - s.gbase[plane];
+    if ((long long)blockIdx.x * kSharedWarps >= G) return;   // CTA-uniform
+    stage_shared_table(sh_tab, sh_idx, cum, plane, s);
 
     const long long g = (long long)blockIdx.x * kSharedWarps + (threadIdx.x >> 5);
     if (g >= G) return;
@@ -551,10 +614,9 @@ __global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_kern
     if (!err && lane < nact)
         x = (unsigned)__ldg(words + start + 2 * lane) | ((unsigned)__ldg(words + start + 2 * lane + 1) << 16);
     if (__any_sync(0xffffffffu, lane < nact && x < kRansL)) err |= 4;
-    long long pos = start + 2 * nact;
-    long long wbase = pos;
-    unsigned w0 = ld_word(words, wbase + lane, end), w1 = ld_word(words, wbase + 32 + lane, end);
-    unsigned w2 = ld_word(words, wbase + 64 + lane, end), w3 = ld_word(words, wbase + 96 + lane, end);
+    long long pos = start + 2 * nact, wbase;
+    unsigned w0, w1, w2, w3;
+    shared_load_window(words, pos, end, lane, wbase, w0, w1, w2, w3);
 
     float zprev[kDecBlock];
     long long tprev = -1;
@@ -564,30 +626,8 @@ __global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_kern
         for (int k = 0; k < kDecBlock; ++k) {
             sy[k] = 0;
             if (t0 + k >= len) break;                      // warp-uniform
-            const bool active = lane < shared_row_lanes(s, r0 + t0 + k);
-            const unsigned slot = x & (top - 1);
-            int lo = sh_idx[slot >> bshift], hi = sh_idx[(slot >> bshift) + 1];
-            while (lo < hi) {
-                const int mid = (lo + hi + 1) >> 1;
-                if (sh_tab[mid] <= slot) lo = mid; else hi = mid - 1;
-            }
-            const unsigned c0 = sh_tab[lo];
-            const unsigned f = sh_tab[lo + 1] - c0;
-            if (active) x = f * (x >> s.P) + slot - c0;
-            const bool need = active && x < kRansL;
-            const unsigned mask = __ballot_sync(0xffffffffu, need);
-            const int n = __popc(mask);
-            if (pos + n > end) { err |= 1; break; }
-            const int rel = (int)(pos - wbase) + __popc(mask & lt);   // < 64 for the lanes that read
-            const unsigned a = __shfl_sync(0xffffffffu, w0, rel & 31), b = __shfl_sync(0xffffffffu, w1, rel & 31);
-            if (need) x = (x << 16) | (rel < 32 ? a : b);
-            pos += n;
-            if (pos - wbase >= 32) {
-                w0 = w1; w1 = w2; w2 = w3;
-                wbase += 32;
-                w3 = ld_word(words, wbase + 96 + lane, end);
-            }
-            sy[k] = lo;
+            if (!shared_decode_row(x, pos, wbase, end, w0, w1, w2, w3, s, r0 + t0 + k, sh_tab, sh_idx, words, lane, lt,
+                                   sy[k])) { err |= 1; break; }
         }
         if (zhat && tprev >= 0) {
 #pragma unroll
@@ -609,6 +649,164 @@ __global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_kern
             if (tprev + k < len && lane < shared_row_lanes(s, r0 + tprev + k)) zhat[out0 + (tprev + k) * 32] = zprev[k];
     }
     if (!err && (__any_sync(0xffffffffu, lane < nact && x != kRansL) || pos != end)) err |= 2;
+    if (err && lane == 0) atomicOr(status, err);
+}
+
+// ---- decoder checkpoints and row lookups (vbq_rans_shared_checkpoints / _decode_rows) -------------------------------
+//
+// A checkpoint is the warp's word offset from its group's start and the 32 lane states just before row j K of a segment
+// (j >= 1); segment g's checkpoints are entries g (seg - 1) / K + j - 1 of the index (K clamped to seg on the host).
+
+// Decode one plane exactly as vbq_rans_shared_decode_kernel (same bounds, status bits and final integrity rule), write
+// no symbols, and record every checkpoint.
+__global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_checkpoints_kernel(
+        const unsigned short *__restrict__ words, long long n_words, const long long *__restrict__ bounds,
+        const unsigned *__restrict__ cum, SharedShape s, long long K, unsigned *__restrict__ cp_offsets,
+        unsigned *__restrict__ cp_states, int *__restrict__ status) {
+    extern __shared__ unsigned sh_tab[];   // [Q + 1] then [kRansBuckets + 1] uint16
+    unsigned short *sh_idx = (unsigned short *)(sh_tab + s.Q + 1);
+    const long long G = s.gbase[1];
+    if ((long long)blockIdx.x * kSharedWarps >= G) return;   // CTA-uniform
+    stage_shared_table(sh_tab, sh_idx, cum, 0, s);
+
+    const long long g = (long long)blockIdx.x * kSharedWarps + (threadIdx.x >> 5);
+    if (g >= G) return;
+    const int lane = threadIdx.x & 31;
+    const long long seg = s.seg[0];
+    const long long r0 = g * seg;
+    const long long len = min(seg, s.rows - r0);
+    const int nact = shared_row_lanes(s, r0);
+    long long start = bounds[2 * g], end = bounds[2 * g + 1];
+    int err = 0;
+    if (start < 0 || end > n_words || end - start < 2ll * nact) { err = 4; end = start = 0; }
+    const unsigned lt = lanemask_lt();
+
+    unsigned x = kRansL;
+    if (!err && lane < nact)
+        x = (unsigned)__ldg(words + start + 2 * lane) | ((unsigned)__ldg(words + start + 2 * lane + 1) << 16);
+    if (__any_sync(0xffffffffu, lane < nact && x < kRansL)) err |= 4;
+    long long pos = start + 2 * nact, wbase;
+    unsigned w0, w1, w2, w3;
+    shared_load_window(words, pos, end, lane, wbase, w0, w1, w2, w3);
+
+    long long c = g * ((seg - 1) / K);   // the next checkpoint's entry
+    long long next = K;                  // and its row in the segment
+    for (long long t = 0; t < len && !err; ++t) {
+        if (t == next) {
+            if (lane == 0) cp_offsets[c] = (unsigned)(pos - start);
+            cp_states[32 * c + lane] = x;
+            ++c;
+            next += K;
+        }
+        int sym;
+        if (!shared_decode_row(x, pos, wbase, end, w0, w1, w2, w3, s, r0 + t, sh_tab, sh_idx, words, lane, lt, sym)) {
+            err |= 1;
+            break;
+        }
+    }
+    if (!err && (__any_sync(0xffffffffu, lane < nact && x != kRansL) || pos != end)) err |= 2;
+    if (err && lane == 0) atomicOr(status, err);
+}
+
+// One warp per work item: check every field, restore the checkpoint (or read the segment's initial states), decode
+// rows up to last_row and write each symbol t = 32 r + lane whose embedding row t / D is in the item's slice of rows to
+// out[u][t - D rows[u]].  Status: 8 for a bad item (nothing written), 4 for a bad group range or restored state, 1 for
+// a group that ran out of words.  A z_hat store is deferred by one row, so its code-point load never stalls the state
+// chain.
+__global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_rows_kernel(
+        const unsigned short *__restrict__ words, long long n_words, const long long *__restrict__ bounds,
+        const unsigned *__restrict__ cum, SharedShape s, long long K, const unsigned *__restrict__ cp_offsets,
+        const unsigned *__restrict__ cp_states, const vbq_rans_lookup_item *__restrict__ items, long long n_items,
+        const long long *__restrict__ rows, long long n_req, long long D, const float *__restrict__ code_points,
+        int *__restrict__ qidx, float *__restrict__ zhat, int *__restrict__ status) {
+    extern __shared__ unsigned sh_tab[];   // [Q + 1] then [kRansBuckets + 1] uint16
+    unsigned short *sh_idx = (unsigned short *)(sh_tab + s.Q + 1);
+    if ((long long)blockIdx.x * kSharedWarps >= n_items) return;   // CTA-uniform
+    stage_shared_table(sh_tab, sh_idx, cum, 0, s);
+
+    const long long it = (long long)blockIdx.x * kSharedWarps + (threadIdx.x >> 5);
+    if (it >= n_items) return;
+    const int lane = threadIdx.x & 31;
+    const long long G = s.gbase[1], seg = s.seg[0], V = s.n / D;
+    const vbq_rans_lookup_item w = items[it];
+    bool bad = w.segment < 0 || w.segment >= G;
+    long long r0 = 0, len = 0, first = 0;
+    if (!bad) {
+        r0 = w.segment * seg;
+        len = min(seg, s.rows - r0);
+        bad = w.checkpoint < 0 || w.checkpoint > (len - 1) / K;
+    }
+    if (!bad) {
+        first = r0 + w.checkpoint * K;
+        bad = w.last_row < first || w.last_row >= min(first + K, r0 + len);
+    }
+    if (!bad) bad = w.lo < 0 || w.hi < w.lo || w.hi > n_req;
+    for (long long i = w.lo + lane; !bad && i < w.hi; i += 32) {
+        const long long r = rows[i];
+        bad = r < 0 || r >= V || (i > w.lo && rows[i - 1] >= r);
+    }
+    if (__any_sync(0xffffffffu, bad)) {
+        if (lane == 0) atomicOr(status, 8);
+        return;
+    }
+
+    const int nact = shared_row_lanes(s, r0);
+    long long start = bounds[2 * w.segment], end = bounds[2 * w.segment + 1];
+    int err = 0;
+    if (start < 0 || end > n_words || end - start < 2ll * nact) { err = 4; end = start = 0; }
+    const unsigned lt = lanemask_lt();
+    unsigned x = kRansL;
+    long long pos, wbase;
+    if (w.checkpoint == 0) {
+        if (!err && lane < nact)
+            x = (unsigned)__ldg(words + start + 2 * lane) | ((unsigned)__ldg(words + start + 2 * lane + 1) << 16);
+        pos = start + 2 * nact;
+    } else {
+        const long long c = w.segment * ((seg - 1) / K) + w.checkpoint - 1;
+        x = __ldg(cp_states + 32 * c + lane);
+        pos = start + __ldg(cp_offsets + c);
+    }
+    if (__any_sync(0xffffffffu, lane < nact && x < kRansL)) err |= 4;
+    unsigned w0, w1, w2, w3;
+    shared_load_window(words, pos, end, lane, wbase, w0, w1, w2, w3);
+
+    // this lane's symbol on the current row: embedding row e, offset o in it; u = the first slice entry with rows[u] >= e
+    const unsigned long long t0 = 32ull * first + lane;
+    long long e = (long long)(t0 / (unsigned long long)D), o = (long long)t0 - e * D;
+    const long long de = 32 / D, dof = 32 % D;
+    long long u = w.lo;
+    long long ru = u < w.hi ? rows[u] : LLONG_MAX;
+    long long pend = -1;                 // output element of the deferred store
+    int qpend = 0;
+    float zpend = 0.f;
+    for (long long r = first; r <= w.last_row && !err; ++r) {
+        const bool active = lane < shared_row_lanes(s, r);
+        int sym;
+        if (!shared_decode_row(x, pos, wbase, end, w0, w1, w2, w3, s, r, sh_tab, sh_idx, words, lane, lt, sym)) {
+            err |= 1;
+            break;
+        }
+        if (pend >= 0) {
+            if (qidx) qidx[pend] = qpend;
+            if (zhat) zhat[pend] = zpend;
+        }
+        pend = -1;
+        if (active) {
+            while (ru < e) ru = ++u < w.hi ? rows[u] : LLONG_MAX;
+            if (ru == e) {
+                pend = u * D + o;
+                qpend = sym;
+                if (zhat) zpend = __ldg(code_points + sym);
+            }
+        }
+        e += de;
+        o += dof;
+        if (o >= D) { o -= D; ++e; }
+    }
+    if (!err && pend >= 0) {
+        if (qidx) qidx[pend] = qpend;
+        if (zhat) zhat[pend] = zpend;
+    }
     if (err && lane == 0) atomicOr(status, err);
 }
 
@@ -775,6 +973,96 @@ extern "C" int vbq_rans_shared_decode(const unsigned short *d_payload, long long
     const size_t smem = (size_t)(s.Q + 1) * sizeof(unsigned) + (kRansBuckets + 1) * sizeof(unsigned short);
     vbq_rans_shared_decode_kernel<<<grid, kSharedWarps * 32, smem, st>>>(d_payload, payload_words, d_group_bounds, d_cum,
                                                                        s, d_code_points, d_qidx, d_zhat, d_status);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+namespace {
+
+// shared_shape of one plane, plus K >= 1 clamped to the segment length (a longer interval holds no checkpoint).
+int lookup_shape(const char *fn, long long n, long long seg_rows, int N, int prob_bits, long long K, SharedShape *s,
+                 long long *k) {
+    if (K < 1) return vbq_fail(VBQ_ERR_BAD_SHAPE, "%s: checkpoint_rows=%lld (>= 1)", fn, K);
+    RETURN_IF(shared_shape(fn, 1, n, &seg_rows, N, prob_bits, s));
+    *k = min(K, s->seg[0]);
+    return VBQ_OK;
+}
+
+long long lookup_checkpoints(const SharedShape &s, long long k) {
+    const long long G = s.gbase[1];
+    if (G == 0) return 0;
+    return (G - 1) * ((s.seg[0] - 1) / k) + (s.rows - (G - 1) * s.seg[0] - 1) / k;
+}
+
+}  // namespace
+
+extern "C" long long vbq_rans_shared_checkpoint_count(long long n, long long seg_rows, long long checkpoint_rows) {
+    SharedShape s;
+    long long k;
+    if (lookup_shape("vbq_rans_shared_checkpoint_count", n, seg_rows, 0, 16, checkpoint_rows, &s, &k) != VBQ_OK)
+        return -1;
+    return lookup_checkpoints(s, k);
+}
+
+extern "C" int vbq_rans_shared_checkpoints(const unsigned short *d_payload, long long payload_words,
+                                           const long long *d_group_bounds, long long n, long long seg_rows, int N,
+                                           int prob_bits, const unsigned *d_cum, long long checkpoint_rows,
+                                           unsigned *d_offsets, unsigned *d_states, int *d_status, void *stream) {
+    SharedShape s;
+    long long k;
+    RETURN_IF(lookup_shape("vbq_rans_shared_checkpoints", n, seg_rows, N, prob_bits, checkpoint_rows, &s, &k));
+    if (payload_words < 0)
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "vbq_rans_shared_checkpoints: payload_words=%lld", payload_words);
+    const long long G = s.gbase[1], M = lookup_checkpoints(s, k);
+    if (!d_cum || !d_status || (G > 0 && (!d_payload || !d_group_bounds)) || (M > 0 && (!d_offsets || !d_states)))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_shared_checkpoints: null pointer");
+    if (((uintptr_t)d_payload & 1) || ((uintptr_t)d_cum & 3) || ((uintptr_t)d_group_bounds & 7) ||
+        ((uintptr_t)d_offsets & 3) || ((uintptr_t)d_states & 3) || ((uintptr_t)d_status & 3))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_shared_checkpoints: misaligned pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int), st));
+    if (G == 0) return VBQ_OK;
+    const size_t smem = (size_t)(s.Q + 1) * sizeof(unsigned) + (kRansBuckets + 1) * sizeof(unsigned short);
+    vbq_rans_shared_checkpoints_kernel<<<(unsigned)((G + kSharedWarps - 1) / kSharedWarps), kSharedWarps * 32, smem,
+                                         st>>>(d_payload, payload_words, d_group_bounds, d_cum, s, k, d_offsets,
+                                               d_states, d_status);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+extern "C" int vbq_rans_shared_decode_rows(const unsigned short *d_payload, long long payload_words,
+                                           const long long *d_group_bounds, long long n, long long seg_rows, int N,
+                                           int prob_bits, const unsigned *d_cum, long long checkpoint_rows,
+                                           const unsigned *d_offsets, const unsigned *d_states,
+                                           const vbq_rans_lookup_item *d_items, long long n_items,
+                                           const long long *d_rows, long long n_req, long long row_size,
+                                           const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status,
+                                           void *stream) {
+    SharedShape s;
+    long long k;
+    RETURN_IF(lookup_shape("vbq_rans_shared_decode_rows", n, seg_rows, N, prob_bits, checkpoint_rows, &s, &k));
+    if (payload_words < 0 || row_size < 1 || n % row_size != 0 || n_items < 0 ||
+        n_items > 2147483647ll * kSharedWarps || n_req < 0 || n_req > n / row_size)
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "vbq_rans_shared_decode_rows: payload_words=%lld row_size=%lld n=%lld "
+                        "n_items=%lld n_req=%lld", payload_words, row_size, n, n_items, n_req);
+    const long long G = s.gbase[1], M = lookup_checkpoints(s, k);
+    if (!d_cum || !d_status || (d_zhat && !d_code_points) ||
+        (n_items > 0 && (!d_payload || !d_group_bounds || !d_items || (G > 0 && M > 0 && (!d_offsets || !d_states)))) ||
+        (n_req > 0 && !d_rows))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_shared_decode_rows: null pointer");
+    if (((uintptr_t)d_payload & 1) || ((uintptr_t)d_cum & 3) || ((uintptr_t)d_group_bounds & 7) ||
+        ((uintptr_t)d_offsets & 3) || ((uintptr_t)d_states & 3) || ((uintptr_t)d_items & 7) ||
+        ((uintptr_t)d_rows & 7) || ((uintptr_t)d_code_points & 3) || ((uintptr_t)d_qidx & 3) ||
+        ((uintptr_t)d_zhat & 3) || ((uintptr_t)d_status & 3))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_shared_decode_rows: misaligned pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int), st));
+    if (n_items == 0) return VBQ_OK;
+    const size_t smem = (size_t)(s.Q + 1) * sizeof(unsigned) + (kRansBuckets + 1) * sizeof(unsigned short);
+    vbq_rans_shared_decode_rows_kernel<<<(unsigned)((n_items + kSharedWarps - 1) / kSharedWarps), kSharedWarps * 32,
+                                         smem, st>>>(d_payload, payload_words, d_group_bounds, d_cum, s, k, d_offsets,
+                                                     d_states, d_items, n_items, d_rows, n_req, row_size,
+                                                     d_code_points, d_qidx, d_zhat, d_status);
     CUDA_TRY(cudaGetLastError());
     return VBQ_OK;
 }

@@ -709,3 +709,67 @@ def rans_shared_decode(words: torch.Tensor, bounds: torch.Tensor, cum: torch.Ten
                                             _ptr(code_points), _ptr(q), _ptr(z), status.data_ptr(), _stream(dev))
     _lib.check(st, "vbq_rans_shared_decode")
     return q, z, status
+
+
+# ------------------------------------------------------------------------------------------------------
+# row access into one shared-table plane: decoder checkpoints and the row gather (include/vbq_b200.h)
+# ------------------------------------------------------------------------------------------------------
+LOOKUP_ITEM_FIELDS = 5      # vbq_rans_lookup_item: segment, checkpoint, last_row, lo, hi (int64 each)
+
+
+def rans_shared_checkpoint_count(n: int, seg_rows: int, checkpoint_rows: int) -> int:
+    """Checkpoints of a plane of n symbols in segments of seg_rows rows, one every checkpoint_rows rows; -1 for a bad
+    shape."""
+    return int(_lib.load().vbq_rans_shared_checkpoint_count(n, seg_rows, checkpoint_rows))
+
+
+def rans_shared_checkpoints(words: torch.Tensor, bounds: torch.Tensor, cum: torch.Tensor, n: int, seg_rows: int,
+                            max_bits: int, prob_bits: int, checkpoint_rows: int):
+    """One full decode pass over one plane (words, bounds as for rans_shared_decode; cum (1, Q+1) or (Q+1,) int32) that
+    records the checkpoint index.  Returns (offsets (M,) int32, states (M, 32) int32, status): the uint32 fields of
+    the index as int32, and the int32 device status of vbq_rans_shared_decode.  No synchronisation."""
+    _need_cuda("words", words, torch.int16, 1)
+    _need_cuda("bounds", bounds, torch.int64, 2)
+    _need_cuda("cum", cum, torch.int32)
+    M = rans_shared_checkpoint_count(n, seg_rows, checkpoint_rows)
+    if M < 0:
+        raise ValueError("vbq_b200: bad checkpoint shape: %s" % _lib.load().vbq_last_error().decode())
+    dev = words.device
+    offsets = torch.empty(M, dtype=torch.int32, device=dev)
+    states = torch.empty((M, 32), dtype=torch.int32, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    st = _lib.load().vbq_rans_shared_checkpoints(_ptr(words), words.numel(), _ptr(bounds), n, seg_rows, max_bits,
+                                                 prob_bits, _ptr(cum), checkpoint_rows, _ptr(offsets), _ptr(states),
+                                                 status.data_ptr(), _stream(dev))
+    _lib.check(st, "vbq_rans_shared_checkpoints")
+    return offsets, states, status
+
+
+def rans_shared_decode_rows(words: torch.Tensor, bounds: torch.Tensor, cum: torch.Tensor, n: int, seg_rows: int,
+                            max_bits: int, prob_bits: int, checkpoint_rows: int, offsets: torch.Tensor,
+                            states: torch.Tensor, items: torch.Tensor, rows: torch.Tensor, row_size: int,
+                            code_points: Optional[torch.Tensor] = None, want_qidx: bool = False):
+    """The row gather: items (n_items, 5) int64 work list (vbq_rans_lookup_item), rows (n_req,) int64 sorted unique
+    embedding rows, row_size = D.  Returns (qidx or None, zhat or None, status): (n_req, D) int32 symbols and float32
+    code_points[q], and the int32 device status (8 = a bad work item).  No synchronisation."""
+    for name, t, dt, nd in (("words", words, torch.int16, 1), ("bounds", bounds, torch.int64, 2),
+                            ("cum", cum, torch.int32, None), ("offsets", offsets, torch.int32, 1),
+                            ("states", states, torch.int32, 2), ("items", items, torch.int64, 2),
+                            ("rows", rows, torch.int64, 1)):
+        _need_cuda(name, t, dt, nd)
+    if items.shape[1] != LOOKUP_ITEM_FIELDS:
+        raise ValueError("vbq_b200: `items` must be (n_items, %d), got %s" % (LOOKUP_ITEM_FIELDS, tuple(items.shape)))
+    dev = words.device
+    n_req = rows.numel()
+    q = torch.empty((n_req, row_size), dtype=torch.int32, device=dev) if want_qidx else None
+    z = None
+    if code_points is not None:
+        _need_cuda("code_points", code_points, torch.float32, 1)
+        z = torch.empty((n_req, row_size), dtype=torch.float32, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    st = _lib.load().vbq_rans_shared_decode_rows(_ptr(words), words.numel(), _ptr(bounds), n, seg_rows, max_bits,
+                                                 prob_bits, _ptr(cum), checkpoint_rows, _ptr(offsets), _ptr(states),
+                                                 _ptr(items), items.shape[0], _ptr(rows), n_req, row_size,
+                                                 _ptr(code_points), _ptr(q), _ptr(z), status.data_ptr(), _stream(dev))
+    _lib.check(st, "vbq_rans_shared_decode_rows")
+    return q, z, status

@@ -7,6 +7,8 @@ replicated over 16 virtual channels so the same sm_100a kernel as the image path
 (bank-conflict-free interleaving, include/vbq_b200.h)."""
 from __future__ import annotations
 
+import math
+
 import numpy as np
 import torch
 
@@ -252,3 +254,177 @@ class GaussianCodebook:
                              % (h["max_bits"], h["empirical_std"], self.max_codepoint_length, self.empirical_std))
         out = serialize.decode_embedding(blob, self._ascending, self.device, want_qidx=False)
         return out["zhat"].reshape(h["shape"])
+
+
+_CHECKPOINT_BYTES = 4 + 32 * 4          # one index entry: the word offset and 32 lane states
+_INDEX_SHARE = 8                        # default K: the index takes at most 1/8 of the payload bytes
+_MIN_CHECKPOINT_ROWS = 32
+
+
+def default_checkpoint_rows(n: int, seg_rows: int, payload_bytes: int) -> int:
+    """Checkpoint interval of `CompressedEmbedding` for a plane of n symbols in segments of seg_rows rows: the smallest
+    number of coder rows (rows of 32 symbols), at least 32, for which the checkpoint index (132 bytes per checkpoint)
+    takes at most 1/8 of the payload bytes.  The checkpoint count only falls as the interval grows, and an interval of
+    a whole segment has none, so a bisection finds it."""
+    seg = serialize.shared_seg_rows(n, seg_rows)
+    lo, hi = _MIN_CHECKPOINT_ROWS, max(_MIN_CHECKPOINT_ROWS, seg)
+    while lo < hi:
+        mid = (lo + hi) // 2
+        if _INDEX_SHARE * _CHECKPOINT_BYTES * ops.rans_shared_checkpoint_count(n, seg, mid) <= payload_bytes:
+            hi = mid
+        else:
+            lo = mid + 1
+    return lo
+
+
+class CompressedEmbedding:
+    """Row access into a `GaussianCodebook.compress_to_bytes` blob without decoding all of it.
+
+    The payload, its frequency table and the ascending code points stay on the device, together with a checkpoint
+    index: every ``checkpoint_rows`` coder rows (rows of 32 coordinates) of each segment, the decoder's word position
+    and 32 lane states (132 bytes, include/vbq_b200.h).  A lookup starts each needed piece of the stream at the
+    checkpoint before it, so its cost is about ``checkpoint_rows`` decoded rows per touched interval instead of the
+    whole matrix.  The blob and its rate are unchanged; a smaller ``checkpoint_rows`` trades device memory for latency.
+
+    ``CompressedEmbedding(blob, device="cuda", checkpoint_rows=None)`` parses the blob (every `ValueError` of
+    `serialize.read_embedding_header` comes before anything is uploaded), rebuilds the codebook from its header, checks
+    the code-point fingerprint and runs one full decode pass that builds the index and applies the coder's integrity
+    check, so a corrupt payload raises `ValueError` here.  ``checkpoint_rows`` defaults to `default_checkpoint_rows`;
+    a value of at least the segment length means no checkpoints.  Not an `nn.Module`; no gradients."""
+
+    def __init__(self, blob, device="cuda", checkpoint_rows=None):
+        h = serialize.read_embedding_header(blob)
+        if len(h["shape"]) < 1:
+            raise ValueError("vbq_b200: a 0-d VBQE blob has no rows to look up")
+        if checkpoint_rows is not None and (isinstance(checkpoint_rows, bool) or int(checkpoint_rows) != checkpoint_rows
+                                            or checkpoint_rows < 1):
+            raise ValueError("vbq_b200: checkpoint_rows must be an integer >= 1, got %r" % (checkpoint_rows,))
+        self.device = torch.device(device)
+        self._shape = tuple(int(d) for d in h["shape"])
+        self._beta = h["beta"]
+        self._n = math.prod(self._shape)
+        self._D = math.prod(self._shape[1:])
+        self._seg = serialize.shared_seg_rows(self._n, h["seg_rows"])
+        self._N, self._P = h["max_bits"], h["prob_bits"]
+        payload_bytes = 2 * h["words"].size
+        K = default_checkpoint_rows(self._n, self._seg, payload_bytes) if checkpoint_rows is None else int(checkpoint_rows)
+        self._K = K
+        self._k = min(K, self._seg)                  # what the kernels use: an interval never spans two segments
+        cb = GaussianCodebook(h["empirical_std"], self._N, device=self.device)
+        if coding.code_points_fingerprint(cb.codepoints) != h["fingerprint"]:
+            raise ValueError("vbq_b200: the blob's code-point fingerprint does not match the codebook rebuilt from its "
+                             "header (N=%d, empirical_std=%r)" % (self._N, h["empirical_std"]))
+        self._code_points = cb._ascending
+        self._words = torch.from_numpy(h["words"].view(np.int16).copy()).to(self.device)
+        self._bounds = torch.from_numpy(np.ascontiguousarray(h["bounds"], dtype=np.int64)).to(self.device)
+        self._cum = torch.from_numpy(coding.cum_table_shared(h["table"][None]).view(np.int32)).to(self.device)
+        self._offsets, self._states, status = ops.rans_shared_checkpoints(
+            self._words, self._bounds, self._cum, self._n, self._seg, self._N, self._P, self._k)
+        st = int(status.item())
+        if st:
+            raise ValueError("vbq_b200: corrupt VBQE payload (decoder status %d: %s)" % (
+                st, ", ".join(m for bit, m in ((1, "a group ran out of words"), (2, "integrity check failed"),
+                                                (4, "bad group range or initial state")) if st & bit)))
+
+    @property
+    def shape(self):
+        return self._shape
+
+    @property
+    def beta(self):
+        return self._beta
+
+    @property
+    def checkpoint_rows(self):
+        return self._K
+
+    @property
+    def nbytes(self):
+        """Device bytes held: payload, checkpoint index, group ranges, cum table and code points."""
+        return sum(t.numel() * t.element_size() for t in (self._words, self._offsets, self._states, self._bounds,
+                                                          self._cum, self._code_points))
+
+    def _ids(self, ids):
+        """ids -> flat int64 tensor and its shape; TypeError / IndexError before anything runs on the device for
+        host ids (device ids are range-checked with the work list's size)."""
+        if isinstance(ids, torch.Tensor):
+            t = ids
+        else:
+            a = np.asarray(ids)
+            if a.size == 0 and not isinstance(ids, np.ndarray):
+                a = a.astype(np.int64)
+            if a.dtype.kind not in "iu":
+                raise TypeError("vbq_b200: ids must be integers, got %s" % a.dtype)
+            t = torch.from_numpy(a.astype(np.int64, copy=False))
+        if t.dtype not in (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8):
+            raise TypeError("vbq_b200: ids must be an integer tensor, got %s" % t.dtype)
+        flat = t.reshape(-1)
+        if not flat.is_cuda and flat.numel():
+            lo, hi = int(flat.min()), int(flat.max())
+            if lo < 0 or hi >= self._shape[0]:
+                raise IndexError("vbq_b200: id %d outside [0, %d)" % (lo if lo < 0 else hi, self._shape[0]))
+        return flat.to(device=self.device, dtype=torch.int64), tuple(t.shape)
+
+    def _work_list(self, u, flat=None):
+        """Sorted unique rows u -> (items (n_items, 5) int64, whether the requested ids `flat` already equal u), built
+        on the device; one host synchronisation reads the id range, the list's size and that flag together."""
+        D, S, K = self._D, self._seg, self._k
+        C1 = (S - 1) // K + 1                        # interval slots per segment: interval I = segment C1 + j
+        coder_rows = -(-self._n // 32)
+        rf, rl = (u * D) // 32, (u * D + D - 1) // 32
+        a = (rf // S) * C1 + (rf % S) // K
+        b = (rl // S) * C1 + (rl % S) // K
+        cnt = b - a + 1
+        n_u = u.numel()
+        total = cnt.sum()
+        same = (u == flat).all() if flat is not None and flat.numel() == n_u else torch.zeros((), dtype=torch.bool,
+                                                                                              device=u.device)
+        lo_id, hi_id, n_pairs, n_items, same = torch.stack(
+            [u[0], u[-1], total, total - (a[1:] == b[:-1]).sum(), same.to(torch.int64)]).tolist()
+        if lo_id < 0 or hi_id >= self._shape[0]:
+            raise IndexError("vbq_b200: id %d outside [0, %d)" % (lo_id if lo_id < 0 else hi_id, self._shape[0]))
+        # one (row, interval) pair per interval a row touches; rows are sorted, so intervals are too
+        row = torch.repeat_interleave(torch.arange(n_u, device=u.device), cnt, output_size=n_pairs)
+        first = torch.cumsum(cnt, 0) - cnt
+        I = a[row] + torch.arange(n_pairs, device=u.device) - first[row]
+        new = torch.ones(n_pairs, dtype=torch.bool, device=u.device)
+        new[1:] = I[1:] != I[:-1]
+        item = torch.cumsum(new, 0) - 1
+        seg, j = I // C1, I % C1
+        r_end = torch.clamp(torch.minimum(seg * S + j * K + K, seg * S + S), max=coder_rows)
+        last = torch.minimum(rl[row], r_end - 1)
+
+        def reduce(v, how):
+            return torch.zeros(n_items, dtype=torch.int64, device=u.device).scatter_reduce(0, item, v, how,
+                                                                                            include_self=False)
+        items = torch.stack([reduce(seg, "amax"), reduce(j, "amax"), reduce(last, "amax"), reduce(row, "amin"),
+                             reduce(row, "amax") + 1], dim=1).contiguous()
+        return items, bool(same)
+
+    def lookup(self, ids):
+        """float32 z_hat of the embedding rows `ids`: shape ids.shape + shape[1:], bit-identical to
+        ``GaussianCodebook.decompress_from_bytes(blob)[ids]``.  ids: an integer tensor (any device), array or list, in
+        any order and with duplicates.  Raises TypeError for non-integer ids and IndexError for an id outside
+        [0, shape[0]) before the gather runs.  The work list (unique sorted rows, the checkpoint interval of every
+        piece of each row, per-item slices) is built on the device with torch ops.  Sorted unique ids are gathered
+        straight into the result; other ids are gathered once per distinct row and then indexed.
+
+        A non-empty call makes three host synchronisations: one inside `torch.unique` (it sizes its output), one that
+        reads the id range and the work list's size together, and one that reads the gather's status."""
+        flat, shape = self._ids(ids)
+        out_shape = shape + self._shape[1:]
+        if flat.numel() == 0:
+            return torch.empty(out_shape, dtype=torch.float32, device=self.device)
+        u, inv = torch.unique(flat, sorted=True, return_inverse=True)
+        items, sorted_unique = self._work_list(u, flat)
+        _, z, status = ops.rans_shared_decode_rows(self._words, self._bounds, self._cum, self._n, self._seg, self._N,
+                                                   self._P, self._k, self._offsets, self._states, items, u, self._D,
+                                                   self._code_points)
+        st = int(status.item())
+        if st:
+            raise RuntimeError("vbq_b200: row gather failed (status %d)" % st)
+        if sorted_unique:                            # the gather wrote the answer in place
+            return z.reshape(out_shape)
+        return z[inv].reshape(out_shape)
+
+    __call__ = lookup
