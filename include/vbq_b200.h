@@ -358,6 +358,44 @@ int vbq_rans_shared_decode_rows(const unsigned short *d_payload, long long paylo
                                 const long long *d_rows, long long n_req, long long row_size,
                                 const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status, void *stream);
 
+/* ---- query scores against one shared-table plane (DESIGN.md §8f) ------------------------------------------------
+ *
+ * vbq_rans_shared_row_scores decodes the embedding rows [row_begin, row_end) of one plane (arguments as for
+ * vbq_rans_shared_decode_rows; the plane is (n / row_size, row_size)) from the checkpoint index and writes
+ * d_scores (n_queries, row_end - row_begin) float32: the dot product (metric VBQ_SCORE_DOT) or the cosine
+ * (VBQ_SCORE_COSINE) of every query row of d_queries (n_queries, row_size) float32 with every embedding row.  The
+ * matrix is never written.  1 <= n_queries <= vbq_rans_shared_score_max_queries(row_size) (the launch's query tile
+ * sits in shared memory; 0 means no query of that length fits), or 0 for no work.
+ *
+ * NUMERICS (normative).  For query b and row e with D = row_size, z_d = d_code_points[symbol (e, d)], q_d =
+ * queries[b, d], in IEEE float32 with round-to-nearest and no flush-to-zero (the kernel uses __fmaf_rn, __fadd_rn,
+ * __fsqrt_rn, __fmul_rn and __fdiv_rn, so no contraction or build flag changes a bit):
+ *     a0 = a1 = a2 = a3 = +0;  for d = 0 .. D-1: a[d % 4] = fmaf(z_d, q_d, a[d % 4]);  dot = (a0 + a1) + (a2 + a3)
+ *     cosine: zz and qq by the same rule from z.z and q.q;  den = sqrtf(zz) * sqrtf(qq);
+ *             cosine = den > 0 ? dot / den : 0
+ * A score depends only on (b, e): not on the row range, the number of queries in the launch, the checkpoint interval
+ * or the split of the work.
+ *
+ * WORK SPLIT.  With C1 = (seg_rows - 1) / K + 1 interval slots per segment, interval segment C1 + j holds coder rows
+ * [segment seg_rows + j K, min(segment seg_rows + (j + 1) K, (segment + 1) seg_rows, rows)).  Warp w owns intervals
+ * [w ipw, (w + 1) ipw) (ipw chosen by the function from the shape) and scores every row e of the range whose first coder
+ * row floor(e D / 32) lies in them: it restores the checkpoint of the interval of its first such row and decodes, across
+ * a segment boundary from the next group's initial states, up to the coder row of its last row's last symbol.  Every
+ * row is scored whole by one warp; there are no partial sums across warps.
+ *
+ * Status: bit 1 = a group ran out of words, bit 4 = a bad group range or a restored state below 2^16 (as for
+ * vbq_rans_shared_decode_rows); every word read stays inside its group's range.  VBQ_ERR_BAD_SHAPE also for a bad row
+ * range, row_size not dividing n, too many queries or an unknown metric. */
+#define VBQ_SCORE_DOT 0
+#define VBQ_SCORE_COSINE 1
+int vbq_rans_shared_score_max_queries(long long row_size);
+int vbq_rans_shared_row_scores(const unsigned short *d_payload, long long payload_words,
+                               const long long *d_group_bounds, long long n, long long seg_rows, int N, int prob_bits,
+                               const unsigned *d_cum, long long checkpoint_rows, const unsigned *d_offsets,
+                               const unsigned *d_states, long long row_size, long long row_begin, long long row_end,
+                               const float *d_queries, int n_queries, int metric, const float *d_code_points,
+                               float *d_scores, int *d_status, void *stream);
+
 /* ---- stand-alone operator forms------------------------------------------------------------------------------- */
 
 /* ChannelwisePriorCDFQuantizer.get_all_N_bit_intervals (quantizer.py:65-80): d_mu (rows, C) -> d_left, d_right

@@ -27,6 +27,8 @@ TOTALS = 4
 PRIOR_PARAMS = 43
 MAX_DEPTH = 20
 RANS_SHARED_MAX_PLANES = 64
+SCORE_DOT = 0
+SCORE_COSINE = 1
 
 
 class VbqError(RuntimeError):
@@ -89,6 +91,9 @@ SIGNATURES = {
     "vbq_rans_shared_checkpoints": (_i, [_p, _ll, _p, _ll, _ll, _i, _i, _p, _ll, _p, _p, _p, _p]),
     "vbq_rans_shared_decode_rows": (_i, [_p, _ll, _p, _ll, _ll, _i, _i, _p, _ll, _p, _p, _p, _ll, _p, _ll, _ll,
                                          _p, _p, _p, _p, _p]),
+    "vbq_rans_shared_score_max_queries": (_i, [_ll]),
+    "vbq_rans_shared_row_scores": (_i, [_p, _ll, _p, _ll, _ll, _i, _i, _p, _ll, _p, _p, _ll, _ll, _ll, _p, _i, _i, _p,
+                                        _p, _p, _p]),
 }
 
 _lib = None

@@ -810,6 +810,199 @@ __global__ void __launch_bounds__(kSharedWarps * 32) vbq_rans_shared_decode_rows
     if (err && lane == 0) atomicOr(status, err);
 }
 
+// ---- query scores against one shared-table plane (vbq_rans_shared_row_scores) --------------------------------------
+//
+// Warp w owns checkpoint intervals [w ipw, (w + 1) ipw), numbered segment C1 + j (C1 = (seg - 1) / K + 1 slots per
+// segment), and scores every embedding row of [row_begin, row_end) whose first coder row lies in them, decoding past its
+// last interval (and into later segments) until that row's last symbol.  Each decoded coder row is staged in the warp's
+// 32-float buffer; lane l serves queries l and l + 32 and walks the 32 symbols in d order, so the sums follow the
+// numerics contract of include/vbq_b200.h exactly.  The four accumulators of a (query, row) pair need no data movement:
+// at position i of a coder row, register i & 3 holds the class of the current d (d advances with i, and 32 is a multiple
+// of 4), and a row end resets all four.
+
+constexpr int kScoreWarps = 16;
+constexpr int kScoreMaxQueries = 64;                  // two per lane
+constexpr long long kScoreTargetWarps = 16384;        // ipw is the fewest intervals per warp that stays below this
+constexpr long long kScoreSmemBudget = 112 * 1024;    // per CTA (100-128 registers already allow one CTA per SM)
+
+__host__ __device__ long long score_stride(long long D) { return D | 1; }   // odd: the 32 lanes' rows start in 32 different banks
+
+struct ScoreSmem {
+    long long tab, idx, cp, z, q, total;              // byte offsets of the parts; q takes B queries
+};
+
+__host__ __device__ ScoreSmem score_smem(int Q, long long D, long long B) {
+    ScoreSmem m;
+    m.tab = 0;
+    m.idx = m.tab + 4ll * (Q + 1);
+    m.cp = m.idx + ((2ll * (kRansBuckets + 1) + 15) & ~15ll);
+    m.z = (m.cp + 4ll * Q + 15) & ~15ll;
+    m.q = m.z + 4ll * 32 * kScoreWarps;
+    m.total = m.q + 4 * B * score_stride(D);
+    return m;
+}
+
+// dot = (a0 + a1) + (a2 + a3) where accumulator class c sits in a[(sh + c) & 3]; selects, not an indexed array, so the
+// four stay in registers.
+__device__ __forceinline__ float score_sum4(const float (&a)[4], int sh) {
+    const float a0 = sh == 0 ? a[0] : sh == 1 ? a[1] : sh == 2 ? a[2] : a[3];
+    const float a1 = sh == 0 ? a[1] : sh == 1 ? a[2] : sh == 2 ? a[3] : a[0];
+    const float a2 = sh == 0 ? a[2] : sh == 1 ? a[3] : sh == 2 ? a[0] : a[1];
+    const float a3 = sh == 0 ? a[3] : sh == 1 ? a[0] : sh == 2 ? a[1] : a[2];
+    return __fadd_rn(__fadd_rn(a0, a1), __fadd_rn(a2, a3));
+}
+
+template <int QPL, bool COS>
+__global__ void __launch_bounds__(kScoreWarps * 32, 1) vbq_rans_shared_row_scores_kernel(
+        const unsigned short *__restrict__ words, long long n_words, const long long *__restrict__ bounds,
+        const unsigned *__restrict__ cum, SharedShape s, long long K, const unsigned *__restrict__ cp_offsets,
+        const unsigned *__restrict__ cp_states, const float *__restrict__ code_points,
+        const float *__restrict__ queries, int B, long long D, long long row_begin, long long row_end,
+        long long ipw, long long w_first, float *__restrict__ scores, int *__restrict__ status) {
+    extern __shared__ __align__(16) unsigned char sh_raw[];
+    const ScoreSmem m = score_smem(s.Q, D, B);
+    unsigned *sh_tab = (unsigned *)(sh_raw + m.tab);
+    unsigned short *sh_idx = (unsigned short *)(sh_raw + m.idx);
+    float *sh_cp = (float *)(sh_raw + m.cp);
+    float *sh_q = (float *)(sh_raw + m.q);
+    const long long qs = score_stride(D);
+    for (int i = threadIdx.x; i < s.Q; i += blockDim.x) sh_cp[i] = __ldg(code_points + i);
+    for (long long i = threadIdx.x; i < (long long)B * D; i += blockDim.x) {
+        const long long b = i / D;
+        sh_q[b * qs + (i - b * D)] = __ldg(queries + i);
+    }
+    stage_shared_table(sh_tab, sh_idx, cum, 0, s);      // its barriers also publish sh_cp and sh_q
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    float *sh_z = (float *)(sh_raw + m.z) + 32 * warp;
+    const long long S = s.seg[0], G = s.gbase[1], C1 = (S - 1) / K + 1, T = G * C1;
+    const long long I0 = (w_first + (long long)blockIdx.x * kScoreWarps + warp) * ipw;
+    if (I0 >= T) return;
+    const long long I1 = min(I0 + ipw, T);
+    const long long ra = min((I0 / C1) * S + (I0 % C1) * K, s.rows);
+    const long long rb = min((I1 / C1) * S + (I1 % C1) * K, s.rows);
+    const long long e_lo = max((32 * ra + D - 1) / D, row_begin), e_hi = min((32 * rb + D - 1) / D, row_end);
+    if (ra >= rb || e_lo >= e_hi) return;               // warp-uniform
+
+    // D < kScoreSmemBudget / 4 here (vbq_rans_shared_score_max_queries), so d and the tile offsets fit 32 bits
+    const int Di = (int)D;
+    int qb[QPL];                                         // the lane's query rows in sh_q (the last one for lanes past B)
+    float qn[QPL];                                       // sqrtf(q . q) for the cosine
+#pragma unroll
+    for (int k = 0; k < QPL; ++k) {
+        qb[k] = min(lane + 32 * k, B - 1) * (int)qs;
+        float a[4] = {0.f, 0.f, 0.f, 0.f};
+        if (COS) {
+            for (int d0 = 0; d0 < Di; d0 += 4) {
+#pragma unroll
+                for (int u = 0; u < 4; ++u)
+                    if (d0 + u < Di) a[u] = __fmaf_rn(sh_q[qb[k] + d0 + u], sh_q[qb[k] + d0 + u], a[u]);
+            }
+        }
+        qn[k] = __fsqrt_rn(score_sum4(a, 0));
+    }
+
+    // restore the checkpoint of the interval that holds the first owned row's first coder row
+    const long long r_first = e_lo * D / 32, r_stop = (e_hi * D - 1) / 32;
+    long long g = r_first / S;
+    const long long j = (r_first - g * S) / K;
+    const long long r_start = g * S + j * K;
+    const unsigned lt = lanemask_lt();
+    int err = 0;
+    unsigned x = kRansL;
+    long long start = bounds[2 * g], end = bounds[2 * g + 1], pos, wbase;
+    int nact = shared_row_lanes(s, g * S);
+    if (start < 0 || end > n_words || end - start < 2ll * nact) { err = 4; end = start = 0; }
+    if (j == 0) {
+        if (!err && lane < nact)
+            x = (unsigned)__ldg(words + start + 2 * lane) | ((unsigned)__ldg(words + start + 2 * lane + 1) << 16);
+        pos = start + 2 * nact;
+    } else {
+        const long long c = g * ((S - 1) / K) + j - 1;
+        x = __ldg(cp_states + 32 * c + lane);
+        pos = start + __ldg(cp_offsets + c);
+    }
+    if (__any_sync(0xffffffffu, lane < nact && x < kRansL)) err |= 4;
+    unsigned w0, w1, w2, w3;
+    shared_load_window(words, pos, end, lane, wbase, w0, w1, w2, w3);
+
+    const long long span = row_end - row_begin;
+    long long e = 32 * r_start / D;                      // embedding row of the coder row's first symbol
+    int qoff = (int)(32 * r_start - e * D);              // its d; symbol i of the row has d = qoff + i until a row end
+    int qp[QPL];                                         // sh_q[qp[k] + i] = the lane's q_d of symbol i of the coder row
+#pragma unroll
+    for (int k = 0; k < QPL; ++k) qp[k] = qb[k] + qoff;
+    float acc[QPL][4], zz[4];
+#pragma unroll
+    for (int k = 0; k < QPL; ++k) acc[k][0] = acc[k][1] = acc[k][2] = acc[k][3] = 0.f;
+    zz[0] = zz[1] = zz[2] = zz[3] = 0.f;
+    for (long long r = r_start; r <= r_stop && !err; ++r) {
+        if (r != r_start && r == g * S + S) {            // the next segment: start its group from its initial states
+            ++g;
+            nact = shared_row_lanes(s, r);
+            start = bounds[2 * g];
+            end = bounds[2 * g + 1];
+            if (start < 0 || end > n_words || end - start < 2ll * nact) { err = 4; break; }
+            x = kRansL;
+            if (lane < nact)
+                x = (unsigned)__ldg(words + start + 2 * lane) | ((unsigned)__ldg(words + start + 2 * lane + 1) << 16);
+            if (__any_sync(0xffffffffu, lane < nact && x < kRansL)) { err |= 4; break; }
+            pos = start + 2 * nact;
+            shared_load_window(words, pos, end, lane, wbase, w0, w1, w2, w3);
+        }
+        int sym;
+        if (!shared_decode_row(x, pos, wbase, end, w0, w1, w2, w3, s, r, sh_tab, sh_idx, words, lane, lt, sym)) {
+            err |= 1;
+            break;
+        }
+        __syncwarp();                                    // the previous row's reads of sh_z are done
+        sh_z[lane] = lane < shared_row_lanes(s, r) ? sh_cp[sym] : 0.f;
+        __syncwarp();
+        unsigned ends = 0;                               // positions whose symbol is the last of its embedding row
+        for (int p = Di - 1 - qoff; p < 32; p += Di) ends |= 1u << p;
+#pragma unroll
+        for (int i4 = 0; i4 < 32; i4 += 4) {
+            const float4 z4 = *(const float4 *)(sh_z + i4);
+            const float zv[4] = {z4.x, z4.y, z4.z, z4.w};
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const int i = i4 + u;
+                const float z = zv[u];
+#pragma unroll
+                for (int k = 0; k < QPL; ++k) acc[k][u] = __fmaf_rn(z, sh_q[qp[k] + i], acc[k][u]);
+                if (COS) zz[u] = __fmaf_rn(z, z, zz[u]);
+                if (ends & (1u << i)) {                  // warp-uniform
+                    const int sh = (i + 1 - Di) & 3;   // accumulator class c lives in register (sh + c) & 3
+                    if (e >= e_lo && e < e_hi) {
+                        const float zn = COS ? __fsqrt_rn(score_sum4(zz, sh)) : 0.f;
+#pragma unroll
+                        for (int k = 0; k < QPL; ++k) {
+                            float v = score_sum4(acc[k], sh);
+                            if (COS) {
+                                const float den = __fmul_rn(zn, qn[k]);
+                                v = den > 0.f ? __fdiv_rn(v, den) : 0.f;
+                            }
+                            if (lane + 32 * k < B) scores[(long long)(lane + 32 * k) * span + (e - row_begin)] = v;
+                        }
+                    }
+#pragma unroll
+                    for (int k = 0; k < QPL; ++k) {
+                        acc[k][0] = acc[k][1] = acc[k][2] = acc[k][3] = 0.f;
+                        qp[k] = qb[k] - (i + 1);
+                    }
+                    zz[0] = zz[1] = zz[2] = zz[3] = 0.f;
+                    ++e;
+                    qoff = -(i + 1);
+                }
+            }
+        }
+        qoff += 32;
+#pragma unroll
+        for (int k = 0; k < QPL; ++k) qp[k] += 32;
+    }
+    if (err && lane == 0) atomicOr(status, err);
+}
+
 }  // namespace
 
 extern "C" long long vbq_rans_workspace_bytes(int n_planes, int items, long long item_rows, int C, long long seg_rows) {
@@ -1063,6 +1256,72 @@ extern "C" int vbq_rans_shared_decode_rows(const unsigned short *d_payload, long
                                          smem, st>>>(d_payload, payload_words, d_group_bounds, d_cum, s, k, d_offsets,
                                                      d_states, d_items, n_items, d_rows, n_req, row_size,
                                                      d_code_points, d_qidx, d_zhat, d_status);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+extern "C" int vbq_rans_shared_score_max_queries(long long row_size) {
+    if (row_size < 1) return 0;
+    const long long fixed = score_smem(2047, row_size, 0).total;      // the largest table: N = 10
+    const long long per = 4 * score_stride(row_size);
+    return (int)max(0ll, min((long long)kScoreMaxQueries, (kScoreSmemBudget - fixed) / per));
+}
+
+extern "C" int vbq_rans_shared_row_scores(const unsigned short *d_payload, long long payload_words,
+                                          const long long *d_group_bounds, long long n, long long seg_rows, int N,
+                                          int prob_bits, const unsigned *d_cum, long long checkpoint_rows,
+                                          const unsigned *d_offsets, const unsigned *d_states, long long row_size,
+                                          long long row_begin, long long row_end, const float *d_queries,
+                                          int n_queries, int metric, const float *d_code_points, float *d_scores,
+                                          int *d_status, void *stream) {
+    SharedShape s;
+    long long k;
+    RETURN_IF(lookup_shape("vbq_rans_shared_row_scores", n, seg_rows, N, prob_bits, checkpoint_rows, &s, &k));
+    const long long V = row_size >= 1 ? n / row_size : 0;
+    if (payload_words < 0 || row_size < 1 || n % row_size != 0 || row_begin < 0 || row_end < row_begin ||
+        row_end > V || n_queries < 0 || n_queries > vbq_rans_shared_score_max_queries(row_size) ||
+        (metric != VBQ_SCORE_DOT && metric != VBQ_SCORE_COSINE))
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "vbq_rans_shared_row_scores: payload_words=%lld row_size=%lld n=%lld rows "
+                        "[%lld, %lld) n_queries=%d (max %d) metric=%d", payload_words, row_size, n, row_begin, row_end,
+                        n_queries, vbq_rans_shared_score_max_queries(row_size), metric);
+    const long long G = s.gbase[1], M = lookup_checkpoints(s, k);
+    const bool work = row_end > row_begin && n_queries > 0;
+    if (!d_cum || !d_status ||
+        (work && (!d_payload || !d_group_bounds || !d_queries || !d_code_points || !d_scores ||
+                  (G > 0 && M > 0 && (!d_offsets || !d_states)))))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_shared_row_scores: null pointer");
+    if (((uintptr_t)d_payload & 1) || ((uintptr_t)d_cum & 3) || ((uintptr_t)d_group_bounds & 7) ||
+        ((uintptr_t)d_offsets & 3) || ((uintptr_t)d_states & 3) || ((uintptr_t)d_queries & 3) ||
+        ((uintptr_t)d_code_points & 3) || ((uintptr_t)d_scores & 3) || ((uintptr_t)d_status & 3))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_shared_row_scores: misaligned pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int), st));
+    if (!work) return VBQ_OK;
+    int dev = 0, sms = 0;
+    RETURN_IF(vbq_current_device(&dev, &sms));
+    // the intervals that hold the first coder rows of row_begin and row_end - 1, and the fewest intervals per warp
+    // that keep the launch at most kScoreTargetWarps warps
+    const long long S = s.seg[0], C1 = (S - 1) / k + 1;
+    auto interval = [&](long long r) { return (r / S) * C1 + (r % S) / k; };
+    const long long Ia = interval(row_begin * row_size / 32), Ib = interval((row_end - 1) * row_size / 32);
+    const long long ipw = max(1ll, (Ib - Ia + kScoreTargetWarps) / kScoreTargetWarps);
+    const long long w_first = Ia / ipw, warps = Ib / ipw - w_first + 1;
+    const size_t smem = (size_t)score_smem(s.Q, row_size, n_queries).total;
+    const unsigned grid = (unsigned)((warps + kScoreWarps - 1) / kScoreWarps);
+#define VBQ_SCORE_LAUNCH(QPL, COS)                                                                                    \
+    do {                                                                                                              \
+        VBQ_ENSURE_MAX_SMEM((vbq_rans_shared_row_scores_kernel<QPL, COS>), dev);                                      \
+        vbq_rans_shared_row_scores_kernel<QPL, COS><<<grid, kScoreWarps * 32, smem, st>>>(                            \
+            d_payload, payload_words, d_group_bounds, d_cum, s, k, d_offsets, d_states, d_code_points, d_queries,     \
+            n_queries, row_size, row_begin, row_end, ipw, w_first, d_scores, d_status);                               \
+    } while (0)
+    const bool cosine = metric == VBQ_SCORE_COSINE;
+    if (n_queries <= 32) {
+        if (cosine) VBQ_SCORE_LAUNCH(1, true); else VBQ_SCORE_LAUNCH(1, false);
+    } else {
+        if (cosine) VBQ_SCORE_LAUNCH(2, true); else VBQ_SCORE_LAUNCH(2, false);
+    }
+#undef VBQ_SCORE_LAUNCH
     CUDA_TRY(cudaGetLastError());
     return VBQ_OK;
 }

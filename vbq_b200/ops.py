@@ -773,3 +773,46 @@ def rans_shared_decode_rows(words: torch.Tensor, bounds: torch.Tensor, cum: torc
                                                  _ptr(code_points), _ptr(q), _ptr(z), status.data_ptr(), _stream(dev))
     _lib.check(st, "vbq_rans_shared_decode_rows")
     return q, z, status
+
+
+SCORE_METRICS = {"dot": _lib.SCORE_DOT, "cosine": _lib.SCORE_COSINE}
+
+
+def rans_shared_score_max_queries(row_size: int) -> int:
+    """Queries of length row_size that one vbq_rans_shared_row_scores launch takes (0: none fits)."""
+    return int(_lib.load().vbq_rans_shared_score_max_queries(row_size))
+
+
+def rans_shared_row_scores(words: torch.Tensor, bounds: torch.Tensor, cum: torch.Tensor, n: int, seg_rows: int,
+                           max_bits: int, prob_bits: int, checkpoint_rows: int, offsets: torch.Tensor,
+                           states: torch.Tensor, row_size: int, row_begin: int, row_end: int, queries: torch.Tensor,
+                           code_points: torch.Tensor, metric: str = "dot", out: Optional[torch.Tensor] = None):
+    """Scores of queries (B, row_size) float32 against the embedding rows [row_begin, row_end) of one plane, decoded from
+    the checkpoint index (arguments as for rans_shared_decode_rows).  Returns (scores (B, row_end - row_begin) float32,
+    status int32: bit 1 a group ran out of words, bit 4 a bad group range or restored state).  `out`, if given, is a
+    contiguous float32 tensor of that shape.  B <= rans_shared_score_max_queries(row_size).  No synchronisation."""
+    for name, t, dt, nd in (("words", words, torch.int16, 1), ("bounds", bounds, torch.int64, 2),
+                            ("cum", cum, torch.int32, None), ("offsets", offsets, torch.int32, 1),
+                            ("states", states, torch.int32, 2), ("queries", queries, torch.float32, 2),
+                            ("code_points", code_points, torch.float32, 1)):
+        _need_cuda(name, t, dt, nd)
+    if metric not in SCORE_METRICS:
+        raise ValueError("vbq_b200: metric must be one of %s, got %r" % (sorted(SCORE_METRICS), metric))
+    if queries.shape[1] != row_size:
+        raise ValueError("vbq_b200: queries must be (B, %d), got %s" % (row_size, tuple(queries.shape)))
+    dev = words.device
+    B = queries.shape[0]
+    shape = (B, row_end - row_begin)
+    if out is None:
+        out = torch.empty(shape, dtype=torch.float32, device=dev)
+    else:
+        _need_cuda("out", out, torch.float32, 2)
+        if tuple(out.shape) != shape:
+            raise ValueError("vbq_b200: out must be %s, got %s" % (shape, tuple(out.shape)))
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    st = _lib.load().vbq_rans_shared_row_scores(_ptr(words), words.numel(), _ptr(bounds), n, seg_rows, max_bits,
+                                                prob_bits, _ptr(cum), checkpoint_rows, _ptr(offsets), _ptr(states),
+                                                row_size, row_begin, row_end, _ptr(queries), B, SCORE_METRICS[metric],
+                                                _ptr(code_points), _ptr(out), status.data_ptr(), _stream(dev))
+    _lib.check(st, "vbq_rans_shared_row_scores")
+    return out, status

@@ -428,3 +428,160 @@ class CompressedEmbedding:
         return z[inv].reshape(out_shape)
 
     __call__ = lookup
+
+    # -- scoring queries against every row -------------------------------------------------------------------------
+    TOPK_WORKSPACE_BYTES = 256 << 20    # topk's row-block workspace; the block shrinks as the batch grows
+    _TOPK_CELL_BYTES = 48               # device bytes per (query, block row) cell: scores, keys, values, temporaries
+
+    def _queries(self, queries, metric):
+        """queries -> (B, D) on their own device; TypeError / ValueError before anything reaches this device."""
+        if metric not in ops.SCORE_METRICS:
+            raise ValueError("vbq_b200: metric must be one of %s, got %r" % (sorted(ops.SCORE_METRICS), metric))
+        if isinstance(queries, torch.Tensor):
+            if not queries.dtype.is_floating_point:
+                raise TypeError("vbq_b200: queries must be floating point, got %s" % queries.dtype)
+            t = queries
+        else:
+            a = np.asarray(queries)
+            if a.dtype.kind != "f":
+                raise TypeError("vbq_b200: queries must be floating point, got %s" % a.dtype)
+            t = torch.from_numpy(np.ascontiguousarray(a))
+        tail = self._shape[1:]
+        if tuple(t.shape) == tail:
+            t = t.reshape((1,) + tail)
+        if t.dim() != len(tail) + 1 or tuple(t.shape[1:]) != tail:
+            raise ValueError("vbq_b200: queries must have shape (B, %s) or %s, got %s"
+                             % (", ".join(map(str, tail)), tail, tuple(t.shape)))
+        if ops.rans_shared_score_max_queries(self._D) < 1:
+            raise ValueError("vbq_b200: a query of %d coordinates does not fit the scoring kernel's shared memory"
+                             % self._D)
+        return t.reshape(t.shape[0], self._D)
+
+    def _upload(self, q):
+        return q.to(device=self.device, dtype=torch.float32).contiguous()
+
+    def _scores_into(self, q, start, stop, metric, out, status):
+        """Scores of q (B, D) against rows [start, stop) into out (B, stop - start), one launch per query tile; the
+        launches' status bits are ORed into `status` on the device."""
+        tile = ops.rans_shared_score_max_queries(self._D)
+        for b0 in range(0, q.shape[0], tile):
+            b1 = min(b0 + tile, q.shape[0])
+            _, st = ops.rans_shared_row_scores(self._words, self._bounds, self._cum, self._n, self._seg, self._N,
+                                               self._P, self._k, self._offsets, self._states, self._D, start, stop,
+                                               q[b0:b1], self._code_points, metric, out=out[b0:b1])
+            status.bitwise_or_(st)
+
+    def _check_status(self, status):
+        st = int(status.item())
+        if st:
+            raise RuntimeError("vbq_b200: scoring decode failed (status %d)" % st)
+
+    def scores(self, queries, start=0, stop=None, metric="dot"):
+        """float32 scores (B, stop - start) of every query against the embedding rows [start, stop), computed while
+        the rows are decoded from the blob; the dense matrix is never built.
+
+        queries: (B, *shape[1:]) or shape[1:] (one query, B = 1); a float tensor on any device, an array or a list of
+        floats; values are cast to float32.  metric: "dot" or "cosine".  Each score is the float32 value of the numerics
+        contract of include/vbq_b200.h (four accumulators stepped in coordinate order, fmaf with round-to-nearest; a
+        cosine with a zero norm is 0), so it is bit-reproducible and independent of the range, the batch and
+        checkpoint_rows.  Batches above ``ops.rans_shared_score_max_queries(D)`` queries run as several launches.
+
+        Raises TypeError for non-float queries, ValueError for a wrong trailing shape, an unknown metric or a
+        non-finite query, and IndexError unless 0 <= start <= stop <= shape[0].  A call makes two host
+        synchronisations: the finiteness check and the status read."""
+        V = self._shape[0]
+        stop = V if stop is None else stop
+        if (isinstance(start, bool) or isinstance(stop, bool) or int(start) != start or int(stop) != stop
+                or not 0 <= int(start) <= int(stop) <= V):
+            raise IndexError("vbq_b200: row range [%r, %r) outside [0, %d]" % (start, stop, V))
+        start, stop = int(start), int(stop)
+        q = self._upload(self._queries(queries, metric))
+        if not bool(torch.isfinite(q).all()):
+            raise ValueError("vbq_b200: queries must be finite")
+        out = torch.empty((q.shape[0], stop - start), dtype=torch.float32, device=self.device)
+        status = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self._scores_into(q, start, stop, metric, out, status)
+        self._check_status(status)
+        return out
+
+    def topk(self, queries, k, metric="dot", exclude=None):
+        """The k best rows of every query: (values (B, k) float32, ids (B, k) int64), ordered by score descending and
+        then by id ascending, so ties between equal rows resolve the same way on every run.  values are the `scores` of
+        the returned ids, bit for bit.
+
+        queries and metric as for `scores`.  exclude: an optional (B, E) integer array (any device) of rows that query b
+        must skip, -1 for padding (for an analogy query, the three words of the question).  1 <= k <= shape[0] minus the
+        most distinct rows any query excludes.
+
+        The plane is scanned in blocks of R rows.  A block's scores become int64 keys: the order-preserving map of the
+        float32 bits (-0.0 as +0.0, NaN lowest) in the high half and 0xFFFFFFFF - id in the low half, excluded rows get
+        the minimum, and `torch.topk` over the block's keys and the running top k is an exact, tie-free selection.  R is
+        chosen so that the block's scores, keys and temporaries take at most TOPK_WORKSPACE_BYTES (256 MiB) whatever
+        shape[0] is; besides that the call holds a few (B, k) arrays.  A call makes two host synchronisations: one reads
+        the finiteness and exclude checks together, one reads the decode status."""
+        q = self._queries(queries, metric)
+        V = self._shape[0]
+        B = q.shape[0]
+        if isinstance(k, bool) or int(k) != k:
+            raise ValueError("vbq_b200: k must be an integer, got %r" % (k,))
+        k = int(k)
+        dev = self.device
+        if not 1 <= k <= V:
+            raise ValueError("vbq_b200: k=%d outside [1, %d]" % (k, V))
+        if exclude is None:
+            ex = torch.full((B, 0), -1, dtype=torch.int64, device=dev)
+        else:
+            ex = exclude if isinstance(exclude, torch.Tensor) else torch.from_numpy(np.asarray(exclude))
+            if ex.dtype.is_floating_point or ex.dtype.is_complex or ex.dtype == torch.bool:
+                raise TypeError("vbq_b200: exclude must be integers, got %s" % ex.dtype)
+            if ex.dim() != 2 or ex.shape[0] != B:
+                raise ValueError("vbq_b200: exclude must be (%d, E), got %s" % (B, tuple(ex.shape)))
+            ex = ex.to(device=dev, dtype=torch.int64).contiguous()
+        q = self._upload(q)
+        checks = [torch.isfinite(q).all().to(torch.int64)]
+        if ex.shape[1]:
+            srt = ex.sort(dim=1).values
+            new = torch.ones_like(srt, dtype=torch.bool)
+            new[:, 1:] = srt[:, 1:] != srt[:, :-1]
+            checks += [srt[:, 0].min(), srt[:, -1].max(), ((srt >= 0) & new).sum(dim=1).max()]
+        got = torch.stack(checks).tolist()
+        if not got[0]:
+            raise ValueError("vbq_b200: queries must be finite")
+        n_ex = 0
+        if ex.shape[1]:
+            if got[1] < -1 or got[2] >= V:
+                raise IndexError("vbq_b200: exclude id %d outside [-1, %d)" % (got[1] if got[1] < -1 else got[2], V))
+            n_ex = got[3]
+        if not 1 <= k <= V - n_ex:
+            raise ValueError("vbq_b200: k=%d outside [1, %d]" % (k, V - n_ex))
+
+        R = max(1, min(V, self.TOPK_WORKSPACE_BYTES // (self._TOPK_CELL_BYTES * B)))
+        buf = torch.empty(B * R, dtype=torch.float32, device=dev)
+        keys = torch.full((B, k + R + 1), torch.iinfo(torch.int64).min, dtype=torch.int64, device=dev)   # last: scratch
+        vals = torch.zeros((B, k + R), dtype=torch.float32, device=dev)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        brow = torch.arange(B, device=dev)[:, None].expand_as(ex)
+        low = 0xFFFFFFFF - torch.arange(R, dtype=torch.int64, device=dev)
+        for start in range(0, V, R):
+            Rb = min(R, V - start)
+            s = buf[:B * Rb].view(B, Rb)
+            self._scores_into(q, start, start + Rb, metric, s, status)
+            vals[:, k:k + Rb] = s
+            bits = s.view(torch.int32)
+            hi = torch.where(bits < 0, bits ^ 0x7FFFFFFF, bits)              # order-preserving on the float's bits
+            hi.masked_fill_(s == 0, 0)                                       # -0.0 ties with +0.0
+            hi.masked_fill_(torch.isnan(s), -(1 << 31))                      # NaN (after an overflow) is lowest
+            kb = keys[:, k:k + Rb]
+            kb.copy_(hi)
+            kb.bitwise_left_shift_(32).bitwise_or_(low[:Rb] - start)
+            if ex.shape[1]:
+                inb = (ex >= start) & (ex < start + Rb)
+                keys.index_put_((brow, torch.where(inb, ex - start + k, k + R)),
+                                torch.tensor(torch.iinfo(torch.int64).min, device=dev))
+            tk, ti = torch.topk(keys[:, :k + Rb], k, dim=1)
+            tv = vals.gather(1, ti)
+            keys[:, :k] = tk
+            vals[:, :k] = tv
+        self._check_status(status)
+        ids = 0xFFFFFFFF - (keys[:, :k] & 0xFFFFFFFF)
+        return vals[:, :k].clone(), ids
