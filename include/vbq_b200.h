@@ -396,6 +396,31 @@ int vbq_rans_shared_row_scores(const unsigned short *d_payload, long long payloa
                                const float *d_queries, int n_queries, int metric, const float *d_code_points,
                                float *d_scores, int *d_status, void *stream);
 
+/* ---- exact target ranks against dense float32 rows (DESIGN.md §8g) ---------------------------------------------
+ *
+ * SCORES follow the numerics above (four accumulators a[d % 4] = fmaf(z_d, q_d, a[d % 4]) in d order, dot = (a0 + a1)
+ * + (a2 + a3), cosine = dot / (sqrtf(zz) * sqrtf(qq)) when that product is > 0, else 0; _rn intrinsics throughout),
+ * so a score here equals vbq_rans_shared_row_scores on the same float32 rows bit for bit.
+ * ORDER is that of CompressedEmbedding.topk: the key of a score is the order-preserving map of its float32 bits, with
+ * -0.0 equal to +0.0 and NaN lowest; row j BEATS target t of query i iff key(s_ij) > key(s_it), or the keys are equal
+ * and j < t (ids are global row ids).  The RANK of t is 1 + the number of rows that beat it (minus any the caller
+ * excludes); the target never beats itself.
+ *
+ * vbq_score_ranks ADDS to d_counts[i] (n_queries,) int64 the number of rows of the block d_rows (n_rows, row_size)
+ * float32, whose first row has global id row_offset, that beat target d_targets[i] (n_queries,) int64 of query i of
+ * d_queries (n_queries, row_size) float32, given d_thresholds[i] = s_it (float32, e.g. from vbq_pair_scores).  No
+ * score is written; the counts are integers, so they do not depend on the tiling, the block split or the launch order.
+ * Any n_rows >= 0, row_size >= 1 and 0 <= n_queries <= INT_MAX - 64.
+ * vbq_pair_scores writes d_scores[p] = the score of query d_pair_queries[p] with row d_pair_rows[p] of d_rows, for
+ * n_pairs pairs (both index arrays int64; a pair with an index out of range gets NaN).
+ * Status codes: VBQ_ERR_BAD_SHAPE for a bad size or an unknown metric (VBQ_SCORE_DOT / VBQ_SCORE_COSINE). */
+int vbq_score_ranks(const float *d_rows, long long n_rows, long long row_size, long long row_offset,
+                    const float *d_queries, long long n_queries, int metric, const float *d_thresholds,
+                    const long long *d_targets, long long *d_counts, void *stream);
+int vbq_pair_scores(const float *d_rows, long long n_rows, long long row_size, const float *d_queries,
+                    long long n_queries, const long long *d_pair_rows, const long long *d_pair_queries,
+                    long long n_pairs, int metric, float *d_scores, void *stream);
+
 /* ---- stand-alone operator forms------------------------------------------------------------------------------- */
 
 /* ChannelwisePriorCDFQuantizer.get_all_N_bit_intervals (quantizer.py:65-80): d_mu (rows, C) -> d_left, d_right

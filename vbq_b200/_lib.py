@@ -94,6 +94,8 @@ SIGNATURES = {
     "vbq_rans_shared_score_max_queries": (_i, [_ll]),
     "vbq_rans_shared_row_scores": (_i, [_p, _ll, _p, _ll, _ll, _i, _i, _p, _ll, _p, _p, _ll, _ll, _ll, _p, _i, _i, _p,
                                         _p, _p, _p]),
+    "vbq_score_ranks": (_i, [_p, _ll, _ll, _ll, _p, _ll, _i, _p, _p, _p, _p]),
+    "vbq_pair_scores": (_i, [_p, _ll, _ll, _p, _ll, _p, _p, _ll, _i, _p, _p]),
 }
 
 _lib = None

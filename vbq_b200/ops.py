@@ -816,3 +816,49 @@ def rans_shared_row_scores(words: torch.Tensor, bounds: torch.Tensor, cum: torch
                                                 _ptr(code_points), _ptr(out), status.data_ptr(), _stream(dev))
     _lib.check(st, "vbq_rans_shared_row_scores")
     return out, status
+
+
+# ------------------------------------------------------------------------------------------------------
+# exact target ranks against dense float32 rows (include/vbq_b200.h, vbq_score_ranks / vbq_pair_scores)
+# ------------------------------------------------------------------------------------------------------
+def score_ranks(rows: torch.Tensor, queries: torch.Tensor, metric: str, thresholds: torch.Tensor,
+                targets: torch.Tensor, counts: torch.Tensor, row_offset: int = 0):
+    """Adds to counts (B,) int64 the number of rows of rows (n_rows, D) float32 (global ids row_offset ..) that beat
+    each query's target under the score and order contract: queries (B, D) float32, thresholds (B,) float32 = the
+    target's score, targets (B,) int64 global ids.  Returns counts.  No synchronisation."""
+    for name, t, dt, nd in (("rows", rows, torch.float32, 2), ("queries", queries, torch.float32, 2),
+                            ("thresholds", thresholds, torch.float32, 1), ("targets", targets, torch.int64, 1),
+                            ("counts", counts, torch.int64, 1)):
+        _need_cuda(name, t, dt, nd)
+    if metric not in SCORE_METRICS:
+        raise ValueError("vbq_b200: metric must be one of %s, got %r" % (sorted(SCORE_METRICS), metric))
+    B, D = queries.shape
+    if rows.shape[1] != D or not thresholds.numel() == targets.numel() == counts.numel() == B:
+        raise ValueError("vbq_b200: score_ranks shapes: rows %s, queries %s, thresholds %s, targets %s, counts %s"
+                         % tuple(tuple(t.shape) for t in (rows, queries, thresholds, targets, counts)))
+    st = _lib.load().vbq_score_ranks(_ptr(rows), rows.shape[0], D, int(row_offset), _ptr(queries), B,
+                                     SCORE_METRICS[metric], _ptr(thresholds), _ptr(targets), _ptr(counts),
+                                     _stream(rows.device))
+    _lib.check(st, "vbq_score_ranks")
+    return counts
+
+
+def pair_scores(rows: torch.Tensor, queries: torch.Tensor, pair_rows: torch.Tensor, pair_queries: torch.Tensor,
+                metric: str = "dot"):
+    """float32 (P,) scores of query pair_queries[p] with row pair_rows[p] of rows (n_rows, D) float32, under the
+    contract; queries (B, D) float32, both index arrays (P,) int64 (an index out of range gives NaN).  No
+    synchronisation."""
+    for name, t, dt, nd in (("rows", rows, torch.float32, 2), ("queries", queries, torch.float32, 2),
+                            ("pair_rows", pair_rows, torch.int64, 1), ("pair_queries", pair_queries, torch.int64, 1)):
+        _need_cuda(name, t, dt, nd)
+    if metric not in SCORE_METRICS:
+        raise ValueError("vbq_b200: metric must be one of %s, got %r" % (sorted(SCORE_METRICS), metric))
+    if rows.shape[1] != queries.shape[1] or pair_rows.numel() != pair_queries.numel():
+        raise ValueError("vbq_b200: pair_scores shapes: rows %s, queries %s, pair_rows %s, pair_queries %s"
+                         % tuple(tuple(t.shape) for t in (rows, queries, pair_rows, pair_queries)))
+    out = torch.empty(pair_rows.numel(), dtype=torch.float32, device=rows.device)
+    st = _lib.load().vbq_pair_scores(_ptr(rows), rows.shape[0], rows.shape[1], _ptr(queries), queries.shape[0],
+                                     _ptr(pair_rows), _ptr(pair_queries), pair_rows.numel(), SCORE_METRICS[metric],
+                                     _ptr(out), _stream(rows.device))
+    _lib.check(st, "vbq_pair_scores")
+    return out

@@ -58,6 +58,189 @@ def _pen_f32(beta):
     return not (isinstance(beta, np.floating) and np.lib.NumpyVersion(np.__version__) >= "2.0.0")
 
 
+def _query_matrix(queries, metric, tail):
+    """queries (B, *tail) or tail -> (B, prod(tail)) on their own device; TypeError / ValueError before anything
+    reaches a device."""
+    if metric not in ops.SCORE_METRICS:
+        raise ValueError("vbq_b200: metric must be one of %s, got %r" % (sorted(ops.SCORE_METRICS), metric))
+    if isinstance(queries, torch.Tensor):
+        if not queries.dtype.is_floating_point:
+            raise TypeError("vbq_b200: queries must be floating point, got %s" % queries.dtype)
+        t = queries
+    else:
+        a = np.asarray(queries)
+        if a.dtype.kind != "f":
+            raise TypeError("vbq_b200: queries must be floating point, got %s" % a.dtype)
+        t = torch.from_numpy(np.ascontiguousarray(a))
+    if tuple(t.shape) == tail:
+        t = t.reshape((1,) + tail)
+    if t.dim() != len(tail) + 1 or tuple(t.shape[1:]) != tail:
+        raise ValueError("vbq_b200: queries must have shape (B, %s) or %s, got %s"
+                         % (", ".join(map(str, tail)), tail, tuple(t.shape)))
+    return t.reshape(t.shape[0], math.prod(tail))
+
+
+def _int_tensor(x, name):
+    """An integer tensor (any device) from a tensor, array or list; TypeError for anything else."""
+    if isinstance(x, torch.Tensor):
+        t = x
+    else:
+        a = np.asarray(x)
+        if a.size == 0 and not isinstance(x, np.ndarray):
+            a = a.astype(np.int64)
+        if a.dtype.kind not in "iu":
+            raise TypeError("vbq_b200: %s must be integers, got %s" % (name, a.dtype))
+        t = torch.from_numpy(a.astype(np.int64, copy=False))
+    if t.dtype not in (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8):
+        raise TypeError("vbq_b200: %s must be an integer tensor, got %s" % (name, t.dtype))
+    return t
+
+
+def _rank_inputs(queries, targets, metric, exclude, tail, V, device):
+    """Validates the arguments of the rank functions before any launch: returns (q (B, D) float32, t (B,) int64,
+    ex (B, E) int64) on `device`.  One host synchronisation reads the finiteness, the id ranges and the
+    target-in-its-exclude-row flag together (none for B = 0)."""
+    q = _query_matrix(queries, metric, tail)
+    B = q.shape[0]
+    t = _int_tensor(targets, "targets")
+    if tuple(t.shape) != (B,):
+        raise ValueError("vbq_b200: targets must be (%d,), got %s" % (B, tuple(t.shape)))
+    if exclude is None:
+        ex = torch.full((B, 0), -1, dtype=torch.int64)
+    else:
+        ex = _int_tensor(exclude, "exclude")
+        if ex.dim() != 2 or ex.shape[0] != B:
+            raise ValueError("vbq_b200: exclude must be (%d, E), got %s" % (B, tuple(ex.shape)))
+    q = q.to(device=device, dtype=torch.float32).contiguous()
+    t = t.to(device=device, dtype=torch.int64).contiguous()
+    ex = ex.to(device=device, dtype=torch.int64).contiguous()
+    if B == 0:
+        return q, t, ex
+    checks = [torch.isfinite(q).all().to(torch.int64), t.min(), t.max()]
+    if ex.shape[1]:
+        checks += [ex.min(), ex.max(), (ex == t[:, None]).any().to(torch.int64)]
+    got = torch.stack(checks).tolist()
+    if not got[0]:
+        raise ValueError("vbq_b200: queries must be finite")
+    if got[1] < 0 or got[2] >= V:
+        raise IndexError("vbq_b200: target %d outside [0, %d)" % (got[1] if got[1] < 0 else got[2], V))
+    if ex.shape[1]:
+        if got[3] < -1 or got[4] >= V:
+            raise IndexError("vbq_b200: exclude id %d outside [-1, %d)" % (got[3] if got[3] < -1 else got[4], V))
+        if got[5]:
+            raise ValueError("vbq_b200: a target is listed in its own exclude row")
+    return q, t, ex
+
+
+def _score_keys(s):
+    """int64 keys of float32 scores in the order of CompressedEmbedding.topk: the order-preserving map of the bits,
+    -0.0 as +0.0, NaN lowest."""
+    bits = s.view(torch.int32)
+    k = torch.where(bits < 0, bits ^ 0x7FFFFFFF, bits)
+    k = k.masked_fill(s == 0, 0).masked_fill(torch.isnan(s), -(1 << 31))
+    return k.to(torch.int64)
+
+
+def _excluded_beaters(s, ids, valid, thr, t):
+    """(B,) number of distinct excluded rows that beat the target: s (B, E) their scores, ids (B, E) their ids, valid
+    marks the first occurrence of each id >= 0, thr (B,) the targets' scores, t (B,) the targets."""
+    ks, kt = _score_keys(s), _score_keys(thr)[:, None]
+    beats = (ks > kt) | ((ks == kt) & (ids < t[:, None]))
+    return (beats & valid).sum(dim=1)
+
+
+def _distinct_excluded(ex):
+    """(sorted ids (B, E), mask of the first occurrence of every id >= 0)."""
+    srt = ex.sort(dim=1).values
+    valid = srt >= 0
+    valid[:, 1:] &= srt[:, 1:] != srt[:, :-1]
+    return srt, valid
+
+
+def _dense_rows(matrix):
+    """A (V, *tail) float32 CUDA tensor -> (V, D) contiguous; TypeError / ValueError otherwise."""
+    if not isinstance(matrix, torch.Tensor) or not matrix.is_cuda or matrix.dtype != torch.float32:
+        raise TypeError("vbq_b200: the embedding must be a float32 CUDA tensor or a CompressedEmbedding")
+    if matrix.dim() < 1 or math.prod(matrix.shape[1:]) < 1:
+        raise ValueError("vbq_b200: the embedding must be (V, *tail) with at least one coordinate per row, got %s"
+                         % (tuple(matrix.shape),))
+    return matrix.reshape(matrix.shape[0], -1).contiguous()
+
+
+def ranks(matrix, queries, targets, metric="dot", exclude=None):
+    """Exact rank of each query's target among the rows of a dense embedding: int64 (B,) tensor, 1 = the best row.
+
+    matrix: a (V, *tail) float32 CUDA tensor (`compress_coordinates` or `decompress_from_bytes` output, or any
+    matrix).  queries and metric as for `CompressedEmbedding.scores` (values must be finite).  targets: (B,) integer
+    ids in [0, V) on any device.  exclude: an optional (B, E) integer array as for `CompressedEmbedding.topk` (-1 pads,
+    duplicates count once); a target in its own exclude row is a ValueError.
+
+    Scores follow the numerics contract of include/vbq_b200.h and rows are ordered as `topk` orders them (score key
+    descending, then id ascending), so rank_i = 1 + the number of rows not excluded that beat t_i, and rank_i <= k
+    exactly when `topk(q_i, k, exclude=exclude_i)` returns t_i, at position rank_i.  The count runs in the
+    vbq_score_ranks kernel without writing a score; excluded rows are subtracted afterwards from their scores
+    (vbq_pair_scores).  A non-empty call makes one host synchronisation (the argument checks)."""
+    Z = _dense_rows(matrix)
+    V = Z.shape[0]
+    q, t, ex = _rank_inputs(queries, targets, metric, exclude, tuple(matrix.shape[1:]), V, Z.device)
+    B = q.shape[0]
+    if B == 0:
+        return torch.empty(0, dtype=torch.int64, device=Z.device)
+    ar = torch.arange(B, device=Z.device)
+    thr = ops.pair_scores(Z, q, t, ar, metric)
+    counts = torch.ones(B, dtype=torch.int64, device=Z.device)
+    if ex.shape[1]:
+        srt, valid = _distinct_excluded(ex)
+        s = ops.pair_scores(Z, q, srt.clamp_min(0).reshape(-1), ar[:, None].expand_as(srt).reshape(-1), metric)
+        counts -= _excluded_beaters(s.view(srt.shape), srt, valid, thr, t)
+    return ops.score_ranks(Z, q, metric, thr, t, counts)
+
+
+def analogy_ranks(embedding, questions, metric="cosine"):
+    """Ranks of the answers of analogy questions a : b :: c : d (3CosAdd on the stored rows): int64 (B,) tensor.
+
+    embedding: a dense (V, *tail) float32 CUDA tensor or a `CompressedEmbedding`.  questions: (B, 4) integer ids
+    a, b, c, d (any device).  The query of a question is (z_b - z_a) + z_c in float32 with round-to-nearest, its target
+    is d, and a, b and c are excluded (`ranks` / `CompressedEmbedding.ranks`), so a question whose d equals a, b or c
+    is a ValueError.  Raises TypeError / ValueError for a bad questions array and IndexError for an id outside
+    [0, V), before any launch."""
+    compressed = isinstance(embedding, CompressedEmbedding)
+    if compressed:
+        V, tail, dev = embedding.shape[0], embedding.shape[1:], embedding.device
+    else:
+        Z = _dense_rows(embedding)
+        V, tail, dev = Z.shape[0], tuple(embedding.shape[1:]), Z.device
+    qs = _int_tensor(questions, "questions")
+    if qs.dim() != 2 or qs.shape[1] != 4:
+        raise ValueError("vbq_b200: questions must be (B, 4), got %s" % (tuple(qs.shape),))
+    qs = qs.to(device=dev, dtype=torch.int64)
+    B = qs.shape[0]
+    if B:
+        lo, hi = torch.stack([qs.min(), qs.max()]).tolist()
+        if lo < 0 or hi >= V:
+            raise IndexError("vbq_b200: question id %d outside [0, %d)" % (lo if lo < 0 else hi, V))
+    abc = qs[:, :3].contiguous()
+    rows = embedding.lookup(abc).reshape(B, 3, math.prod(tail)) if compressed else Z[abc]
+    query = ((rows[:, 1] - rows[:, 0]) + rows[:, 2]).reshape((B,) + tuple(tail))
+    if compressed:
+        return embedding.ranks(query, qs[:, 3], metric, exclude=abc)
+    return ranks(embedding, query, qs[:, 3], metric, exclude=abc)
+
+
+def analogy_metrics(ranks):
+    """The quality columns of the notebook's `test_beta` from analogy ranks: {"mrr": mean(1 / rank), "acc":
+    mean(rank == 1), "hits10": mean(rank <= 10)} as float64.  ranks: a non-empty integer array (any device) of
+    values >= 1."""
+    r = (ranks.detach().cpu().numpy() if isinstance(ranks, torch.Tensor) else np.asarray(ranks)).reshape(-1)
+    if r.size and r.dtype.kind not in "iu":
+        raise TypeError("vbq_b200: ranks must be integers, got %s" % r.dtype)
+    if r.size == 0 or r.min() < 1:
+        raise ValueError("vbq_b200: ranks must be a non-empty array of values >= 1")
+    r = r.astype(np.float64)
+    return {"mrr": np.float64(np.mean(1.0 / r)), "acc": np.float64(np.mean(r == 1)),
+            "hits10": np.float64(np.mean(r <= 10))}
+
+
 class GaussianCodebook:
     """`codepoints` / `lengths` of the notebook (heap order, float64 / int64) plus the device tables."""
 
@@ -135,7 +318,7 @@ class GaussianCodebook:
         """The rate side of the notebook's beta sweep (ipynb:464-473, :1102-1103: `test_beta` for every beta of
         `np.exp(np.linspace(np.log(0.01), np.log(100000), 50))`): compresses all coordinates with every beta and
         returns the `compressed_bitlength` = `empirical_entropy(compressed)` (ipynb:452-455) of each, as a float64
-        array (the embedding-quality metrics of `test_beta` need the skip-gram model and are out of scope).
+        array (the quality columns of `test_beta` come from `analogy_sweep`, which takes its rates from this method).
 
         The coordinates are walked ONCE for all betas (sweep kernel) in row chunks of at most ``max_chunk_symbols``
         (beta, coordinate) pairs; the symbols of a chunk are counted on the device (`vbq_symbol_histogram`) and only the
@@ -198,6 +381,29 @@ class GaussianCodebook:
         if is_np:
             return out.cpu().numpy().astype(np.asarray(means).dtype), None
         return out.to(means.dtype), None
+
+    def analogy_sweep(self, means, stds, betas, questions, metric="cosine", exact=True):
+        """The notebook's `test_beta` loop (ipynb:464-473): for every beta, the analogy quality of the quantized
+        embedding and its rate.  Returns a (len(betas), 4) float64 array with the columns mrr, acc, hits10, bits.
+
+        means, stds: (V, *tail) posteriors (tensors or arrays).  questions: (B, 4) ids a, b, c, d as for
+        `analogy_ranks`.  For each beta, z_hat = `compress_coordinates(means, stds, float(beta), exact=exact)` stays on
+        the device (one at a time), `analogy_ranks(z_hat, questions, metric)` ranks the questions on it and
+        `analogy_metrics` gives the first three columns.  The bits column is one `beta_sweep(means, stds, betas,
+        exact=exact)` call, which takes every beta as a Python float too, so rate and quality come from the same
+        quantization."""
+        bits = self.beta_sweep(means, stds, betas, exact=exact)
+        m = means if isinstance(means, torch.Tensor) else torch.as_tensor(np.asarray(means))
+        s = stds if isinstance(stds, torch.Tensor) else torch.as_tensor(np.asarray(stds))
+        m = m.to(device=self.device, dtype=torch.float32).contiguous()
+        s = s.to(device=self.device, dtype=torch.float32).contiguous()
+        out = np.empty((len(betas), 4), dtype=np.float64)
+        for i, beta in enumerate(betas):
+            zhat, _ = self.compress_coordinates(m, s, float(beta), exact=exact)
+            met = analogy_metrics(analogy_ranks(zhat, questions, metric))
+            del zhat
+            out[i] = (met["mrr"], met["acc"], met["hits10"], bits[i])
+        return out
 
     def compress_to_bytes(self, means, stds, betas, exact=True, prob_bits=coding.DEFAULT_PROB_BITS, seg_rows=None):
         """Entropy-code the coordinates that `compress_coordinates(means, stds, beta, exact=exact)` chooses, for every
@@ -347,17 +553,7 @@ class CompressedEmbedding:
     def _ids(self, ids):
         """ids -> flat int64 tensor and its shape; TypeError / IndexError before anything runs on the device for
         host ids (device ids are range-checked with the work list's size)."""
-        if isinstance(ids, torch.Tensor):
-            t = ids
-        else:
-            a = np.asarray(ids)
-            if a.size == 0 and not isinstance(ids, np.ndarray):
-                a = a.astype(np.int64)
-            if a.dtype.kind not in "iu":
-                raise TypeError("vbq_b200: ids must be integers, got %s" % a.dtype)
-            t = torch.from_numpy(a.astype(np.int64, copy=False))
-        if t.dtype not in (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8):
-            raise TypeError("vbq_b200: ids must be an integer tensor, got %s" % t.dtype)
+        t = _int_tensor(ids, "ids")
         flat = t.reshape(-1)
         if not flat.is_cuda and flat.numel():
             lo, hi = int(flat.min()), int(flat.max())
@@ -435,27 +631,11 @@ class CompressedEmbedding:
 
     def _queries(self, queries, metric):
         """queries -> (B, D) on their own device; TypeError / ValueError before anything reaches this device."""
-        if metric not in ops.SCORE_METRICS:
-            raise ValueError("vbq_b200: metric must be one of %s, got %r" % (sorted(ops.SCORE_METRICS), metric))
-        if isinstance(queries, torch.Tensor):
-            if not queries.dtype.is_floating_point:
-                raise TypeError("vbq_b200: queries must be floating point, got %s" % queries.dtype)
-            t = queries
-        else:
-            a = np.asarray(queries)
-            if a.dtype.kind != "f":
-                raise TypeError("vbq_b200: queries must be floating point, got %s" % a.dtype)
-            t = torch.from_numpy(np.ascontiguousarray(a))
-        tail = self._shape[1:]
-        if tuple(t.shape) == tail:
-            t = t.reshape((1,) + tail)
-        if t.dim() != len(tail) + 1 or tuple(t.shape[1:]) != tail:
-            raise ValueError("vbq_b200: queries must have shape (B, %s) or %s, got %s"
-                             % (", ".join(map(str, tail)), tail, tuple(t.shape)))
+        t = _query_matrix(queries, metric, self._shape[1:])
         if ops.rans_shared_score_max_queries(self._D) < 1:
             raise ValueError("vbq_b200: a query of %d coordinates does not fit the scoring kernel's shared memory"
                              % self._D)
-        return t.reshape(t.shape[0], self._D)
+        return t
 
     def _upload(self, q):
         return q.to(device=self.device, dtype=torch.float32).contiguous()
@@ -585,3 +765,50 @@ class CompressedEmbedding:
         self._check_status(status)
         ids = 0xFFFFFFFF - (keys[:, :k] & 0xFFFFFFFF)
         return vals[:, :k].clone(), ids
+
+    # -- exact target ranks ----------------------------------------------------------------------------------------
+    RANKS_WORKSPACE_BYTES = 256 << 20   # ranks' decoded row block (and its work list)
+    _RANKS_ROW_EXTRA_BYTES = 128        # device bytes per block row besides its D floats: the work list's temporaries
+
+    def ranks(self, queries, targets, metric="dot", exclude=None):
+        """Exact rank of each query's target among the rows of this embedding: int64 (B,) tensor, equal to
+        `vbq_b200.ranks(decompress_from_bytes(blob), queries, targets, metric, exclude)` (arguments as there; queries as
+        for `scores`).
+
+        The target rows and the excluded rows are read with `lookup` and scored with vbq_pair_scores.  Then the plane
+        is decoded in blocks of R consecutive rows, each block straight into one buffer by the row gather, and
+        vbq_score_ranks adds each block's counts; R is chosen so that a block takes at most RANKS_WORKSPACE_BYTES
+        (256 MiB) whatever shape[0] is, so the dense matrix is never whole.  The counts are integers, so the result does
+        not depend on R.  A non-empty call makes 5 + (number of blocks) host synchronisations: the argument checks,
+        three in `lookup`, one per block for its work list and one for the decode status."""
+        V = self._shape[0]
+        q, t, ex = _rank_inputs(queries, targets, metric, exclude, self._shape[1:], V, self.device)
+        B, D, dev = q.shape[0], self._D, self.device
+        if B == 0:
+            return torch.empty(0, dtype=torch.int64, device=dev)
+        ar = torch.arange(B, device=dev)
+        srt, valid = _distinct_excluded(ex)
+        E = srt.shape[1]
+        rows = self.lookup(torch.cat([t, srt.clamp_min(0).reshape(-1)])).reshape(B + B * E, D)
+        thr = ops.pair_scores(rows, q, ar, ar, metric)
+        counts = torch.ones(B, dtype=torch.int64, device=dev)
+        if E:
+            s = ops.pair_scores(rows, q, B + torch.arange(B * E, device=dev), ar[:, None].expand(B, E).reshape(-1),
+                                metric)
+            counts -= _excluded_beaters(s.view(B, E), srt, valid, thr, t)
+        del rows
+        R = max(1, min(V, self.RANKS_WORKSPACE_BYTES // (4 * D + self._RANKS_ROW_EXTRA_BYTES)))
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        for start in range(0, V, R):
+            u = torch.arange(start, min(V, start + R), device=dev)
+            items, _ = self._work_list(u)
+            _, z, st = ops.rans_shared_decode_rows(self._words, self._bounds, self._cum, self._n, self._seg, self._N,
+                                                   self._P, self._k, self._offsets, self._states, items, u, D,
+                                                   self._code_points)
+            status.bitwise_or_(st)
+            ops.score_ranks(z, q, metric, thr, t, counts, row_offset=start)
+            del z, items, u
+        st = int(status.item())
+        if st:
+            raise RuntimeError("vbq_b200: row gather failed (status %d)" % st)
+        return counts
