@@ -274,6 +274,46 @@ int vbq_rans_decode(const unsigned short *d_payload, long long payload_words, co
                     const unsigned short *d_cum, const float *d_code_points, int *d_qidx, float *d_zhat, int *d_status,
                     void *stream);
 
+/* ---- many VBQ2 streams in one launch: the work-list decoder (DESIGN.md §8h) ------------------------------------
+ *
+ * vbq_rans_decode_batch decodes any set of groups of the layout above, from any number of streams (blobs) that share C
+ * and N but may differ in table, prob_bits, seg_rows, item_rows, n_planes and items.  Each group is a UNIT.  Inputs:
+ *   d_payload    (payload_words,) uint16: the streams' payloads back to back;
+ *   d_cum        (n_tables, C, Q) uint16 cum tables as for vbq_rans_decode, and d_prob_bits (n_tables,) int32 device
+ *                array with each table's prob_bits;
+ *   d_units      (n_units,) vbq_rans_batch_unit;
+ *   d_ctas       (n_ctas,) vbq_rans_batch_cta: CTA i decodes units [first, first + count), 1 <= count <= 8, which must
+ *                all have the descriptor's (table, cg): the CTA stages that table set once;
+ *   d_status     (n_blobs,) int32, zeroed by the call: bits 1, 2 and 4 of vbq_rans_decode for the groups of each blob,
+ *                and bit 8 for a bad unit.
+ * A unit decodes rows r = 0 .. rows - 1 of lanes j < nact = min(32, C - 32 cg) from its word range [start, end) and
+ * writes symbol (r, j) to element out + r C + j of d_qidx (int32) and/or d_zhat (float32 d_code_points[32 cg + j][q],
+ * the (C, Q) ascending code points), both flat of n_out elements; per row, the decoder is that of vbq_rans_decode.
+ * Units and descriptors come from the caller's memory, so the kernel checks each before it acts: a range inside the
+ * payload that holds at least the 2 nact state words, table and cg in range and equal to the descriptor's, rows >= 1,
+ * 0 <= out and out + (rows - 1) C + nact <= n_out, 0 <= blob < n_blobs, and the table's prob_bits valid.  A bad unit
+ * sets bit 8 of its blob (of blob 0 if the blob id itself, or the descriptor, is bad) and writes nothing.  Units
+ * whose output ranges overlap write in an undefined order.
+ * Status codes: VBQ_ERR_BAD_DEPTH for N > 10, VBQ_ERR_BAD_SHAPE for a bad count or C. */
+typedef struct {
+    long long start, end;   /* word range [start, end) of the group in d_payload: states, then words */
+    long long out;          /* output element of row 0, lane 0 */
+    long long rows;         /* rows of the segment */
+    long long table, cg;    /* table id in d_cum, 32-channel group */
+    long long blob;         /* the d_status entry this unit reports to */
+} vbq_rans_batch_unit;      /* 56 bytes: an (n_units, 7) int64 array */
+
+typedef struct {
+    long long first, count; /* units [first, first + count) */
+    long long table, cg;    /* shared by all of them */
+} vbq_rans_batch_cta;       /* 32 bytes: an (n_ctas, 4) int64 array */
+
+int vbq_rans_decode_batch(const unsigned short *d_payload, long long payload_words, const unsigned short *d_cum,
+                          const int *d_prob_bits, int n_tables, int C, int N, const vbq_rans_batch_unit *d_units,
+                          long long n_units, const vbq_rans_batch_cta *d_ctas, long long n_ctas, int n_blobs,
+                          const float *d_code_points, long long n_out, int *d_qidx, float *d_zhat, int *d_status,
+                          void *stream);
+
 /* ---- entropy coding with one shared table per plane: word embeddings (DESIGN.md §8d) ------------------------------
  *
  * All coordinates of an embedding matrix share one prior and one empirical model, so the channel axis of the layout

@@ -230,52 +230,41 @@ __device__ __forceinline__ unsigned short ld_word(const unsigned short *__restri
     return i < end ? __ldg(w + i) : (unsigned short)0;
 }
 
-// Same CTA layout as the encoder.  Shared memory: the group's cum tables [nact][Q] and the coarse index [32][257].
-// A warp keeps the next 128 words of its group in registers (4 windows of 32, one word per lane) and reads each row's
-// words with shuffles; a window is refilled 64..96 words before it is needed.
-__global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_decode_kernel(const unsigned short *__restrict__ words,
-                                                                         long long n_words,
-                                                                         const long long *__restrict__ bounds,
-                                                                         const unsigned short *__restrict__ cum,
-                                                                         RansShape s,
-                                                                         const float *__restrict__ code_points,
-                                                                         int *__restrict__ qidx,
-                                                                         float *__restrict__ zhat,
-                                                                         int *__restrict__ status) {
-    extern __shared__ unsigned short sh_cum[];   // [32][Q] then [32][kRansBuckets + 1]
-    const int cg = blockIdx.y, plane = blockIdx.z;
-    unsigned short *sh_idx = sh_cum + 32 * s.Q;
-    load_group_cum(sh_cum, cum, plane, cg, s);
+// Shared memory of the VBQ2 decoders: the 32-channel group's cum tables [nact][Q] (a linear copy of nact Q entries
+// from src) and the coarse index [32][257]: idx[j][b] = the symbol whose slot range holds b << (P - 8), and
+// idx[j][256] = Q - 1.  Every thread of the CTA takes part (two barriers).
+__device__ __forceinline__ void stage_group_table(unsigned short *sh_cum, unsigned short *sh_idx,
+                                                  const unsigned short *__restrict__ src, int nact, int Q, int P) {
+    for (int i = threadIdx.x; i < nact * Q; i += blockDim.x) sh_cum[i] = __ldg(src + i);
     __syncthreads();
-    const int nact = min(32, s.C - 32 * cg);
-    const int bshift = s.P - 8;
-    const unsigned top = 1u << s.P;
-    // idx[j][b] = the symbol whose slot range holds b << bshift: every bucket start lies in exactly one symbol
-    for (int k = threadIdx.x; k < nact * s.Q; k += blockDim.x) {
-        const int j = k / s.Q, q = k - j * s.Q;
-        const unsigned lo = sh_cum[k], hi = q + 1 < s.Q ? (unsigned)sh_cum[k + 1] : top;
+    const int bshift = P - 8;
+    const unsigned top = 1u << P;
+    // every bucket start lies in exactly one symbol
+    for (int k = threadIdx.x; k < nact * Q; k += blockDim.x) {
+        const int j = k / Q, q = k - j * Q;
+        const unsigned lo = sh_cum[k], hi = q + 1 < Q ? (unsigned)sh_cum[k + 1] : top;
         for (unsigned b = (lo + (1u << bshift) - 1) >> bshift; (b << bshift) < hi && b < kRansBuckets; ++b)
             sh_idx[j * (kRansBuckets + 1) + b] = (unsigned short)q;
     }
-    for (int j = threadIdx.x; j < nact; j += blockDim.x) sh_idx[j * (kRansBuckets + 1) + kRansBuckets] = (unsigned short)(s.Q - 1);
+    for (int j = threadIdx.x; j < nact; j += blockDim.x) sh_idx[j * (kRansBuckets + 1) + kRansBuckets] = (unsigned short)(Q - 1);
     __syncthreads();
+}
 
+// One warp decodes one VBQ2 group of len rows and nact state lanes from its word range [start, end) (err = 4 with
+// start = end = 0 for a range the caller rejected): symbol of row t, lane j goes to qidx / zhat[out0 + t C] of lane j,
+// with out0 and cp (the lane's code points) already offset to the lane's channel.  tab / cidx are the lane's table and
+// coarse index.  A warp keeps the next 128 words of its group in registers (4 windows of 32, one word per lane) and
+// reads each row's words with shuffles; a window is refilled 64..96 words before it is needed.  Returns the status
+// bits 1, 2 and 4 of vbq_rans_decode, the same on every lane.
+__device__ __forceinline__ int vbq2_decode_group(const unsigned short *__restrict__ words, long long start,
+                                                 long long end, int err, const unsigned short *tab,
+                                                 const unsigned short *cidx, int P, int Q, int nact, long long len,
+                                                 int C, long long out0, const float *__restrict__ cp,
+                                                 int *__restrict__ qidx, float *__restrict__ zhat) {
     const int lane = threadIdx.x & 31;
-    const long long unit = (long long)blockIdx.x * kRansWarps + (threadIdx.x >> 5);
-    if (unit >= (long long)s.items * s.n_segs) return;
-    const int item = (int)(unit / s.n_segs);
-    const long long r0 = (unit % s.n_segs) * s.seg_rows;
-    const long long len = min(s.seg_rows, s.item_rows - r0);
     const bool active = lane < nact;
-    const int c = 32 * cg + lane;
-    const unsigned short *tab = sh_cum + (active ? lane : 0) * s.Q;
-    const unsigned short *cidx = sh_idx + (active ? lane : 0) * (kRansBuckets + 1);
-    const long long g = (((long long)plane * s.items * s.n_segs + unit) * s.CG + cg);
-    long long start = bounds[2 * g], end = bounds[2 * g + 1];
-    int err = 0;
-    if (start < 0 || end > n_words || end - start < 2ll * nact) { err = 4; end = start = 0; }
-    const long long out0 = (((long long)plane * s.items + item) * s.item_rows + r0) * s.C + c;
-    const float *cp = code_points + (size_t)(active ? c : 0) * s.Q;
+    const int bshift = P - 8;
+    const unsigned top = 1u << P;
     const unsigned lt = lanemask_lt();
 
     unsigned x = kRansL;
@@ -297,14 +286,14 @@ __global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_decode_kernel(const 
             sy[k] = 0;
             if (t0 + k >= len) break;                      // warp-uniform
             const unsigned slot = x & (top - 1);
-            int lo = min((int)cidx[slot >> bshift], s.Q - 1), hi = min((int)cidx[(slot >> bshift) + 1], s.Q - 1);
+            int lo = min((int)cidx[slot >> bshift], Q - 1), hi = min((int)cidx[(slot >> bshift) + 1], Q - 1);
             while (lo < hi) {
                 const int mid = (lo + hi + 1) >> 1;
                 if (tab[mid] <= slot) lo = mid; else hi = mid - 1;
             }
             const unsigned c0 = tab[lo];
-            const unsigned f = (lo + 1 < s.Q ? (unsigned)tab[lo + 1] : top) - c0;
-            x = f * (x >> s.P) + slot - c0;
+            const unsigned f = (lo + 1 < Q ? (unsigned)tab[lo + 1] : top) - c0;
+            x = f * (x >> P) + slot - c0;
             const bool need = active && x < kRansL;
             const unsigned mask = __ballot_sync(0xffffffffu, need);
             const int n = __popc(mask);
@@ -323,13 +312,13 @@ __global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_decode_kernel(const 
         if (zhat && tprev >= 0) {
 #pragma unroll
             for (int k = 0; k < kDecBlock; ++k)
-                if (active) zhat[out0 + (tprev + k) * s.C] = zprev[k];   // a previous block is always full
+                if (active) zhat[out0 + (tprev + k) * C] = zprev[k];   // a previous block is always full
         }
         if (err) break;
 #pragma unroll
         for (int k = 0; k < kDecBlock; ++k) {
             if (active && t0 + k < len) {
-                if (qidx) qidx[out0 + (t0 + k) * s.C] = sy[k];
+                if (qidx) qidx[out0 + (t0 + k) * C] = sy[k];
                 if (zhat) zprev[k] = __ldg(cp + sy[k]);
             }
         }
@@ -338,10 +327,92 @@ __global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_decode_kernel(const 
     if (zhat && tprev >= 0 && !err) {
 #pragma unroll
         for (int k = 0; k < kDecBlock; ++k)
-            if (active && tprev + k < len) zhat[out0 + (tprev + k) * s.C] = zprev[k];
+            if (active && tprev + k < len) zhat[out0 + (tprev + k) * C] = zprev[k];
     }
     if (!err && (__any_sync(0xffffffffu, active && x != kRansL) || pos != end)) err |= 2;
+    return err;
+}
+
+// Same CTA layout as the encoder: CTA (x, cg, plane), one warp per (item, segment) of its channel group.
+__global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_decode_kernel(const unsigned short *__restrict__ words,
+                                                                         long long n_words,
+                                                                         const long long *__restrict__ bounds,
+                                                                         const unsigned short *__restrict__ cum,
+                                                                         RansShape s,
+                                                                         const float *__restrict__ code_points,
+                                                                         int *__restrict__ qidx,
+                                                                         float *__restrict__ zhat,
+                                                                         int *__restrict__ status) {
+    extern __shared__ unsigned short sh_cum[];   // [32][Q] then [32][kRansBuckets + 1]
+    const int cg = blockIdx.y, plane = blockIdx.z;
+    unsigned short *sh_idx = sh_cum + 32 * s.Q;
+    const int nact = min(32, s.C - 32 * cg);
+    stage_group_table(sh_cum, sh_idx, cum + ((size_t)plane * s.C + 32 * cg) * s.Q, nact, s.Q, s.P);
+
+    const int lane = threadIdx.x & 31;
+    const long long unit = (long long)blockIdx.x * kRansWarps + (threadIdx.x >> 5);
+    if (unit >= (long long)s.items * s.n_segs) return;
+    const int item = (int)(unit / s.n_segs);
+    const long long r0 = (unit % s.n_segs) * s.seg_rows;
+    const long long len = min(s.seg_rows, s.item_rows - r0);
+    const bool active = lane < nact;
+    const int c = 32 * cg + lane;
+    const long long g = (((long long)plane * s.items * s.n_segs + unit) * s.CG + cg);
+    long long start = bounds[2 * g], end = bounds[2 * g + 1];
+    int err = 0;
+    if (start < 0 || end > n_words || end - start < 2ll * nact) { err = 4; end = start = 0; }
+    err = vbq2_decode_group(words, start, end, err, sh_cum + (active ? lane : 0) * s.Q,
+                            sh_idx + (active ? lane : 0) * (kRansBuckets + 1), s.P, s.Q, nact, len, s.C,
+                            (((long long)plane * s.items + item) * s.item_rows + r0) * s.C + c,
+                            code_points + (size_t)(active ? c : 0) * s.Q, qidx, zhat);
     if (err && lane == 0) atomicOr(status, err);
+}
+
+// The work-list decoder of many VBQ2 streams (vbq_rans_decode_batch): CTA i stages the table set (table, cg) of
+// descriptor i and its warp w decodes unit first + w.  Every field of the descriptor and the unit comes from the
+// caller's memory and is checked before it is used: a bad one sets status bit 8 (of the unit's blob if its blob id is
+// in range, else of blob 0) and writes nothing.
+__global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_decode_batch_kernel(
+        const unsigned short *__restrict__ words, long long n_words, const unsigned short *__restrict__ cum,
+        const int *__restrict__ prob_bits, int n_tables, int C, int Q, const vbq_rans_batch_unit *__restrict__ units,
+        long long n_units, const vbq_rans_batch_cta *__restrict__ ctas, int n_blobs,
+        const float *__restrict__ code_points, long long n_out, int *__restrict__ qidx, float *__restrict__ zhat,
+        int *__restrict__ status) {
+    extern __shared__ unsigned short sh_cum[];   // [32][Q] then [32][kRansBuckets + 1]
+    unsigned short *sh_idx = sh_cum + 32 * Q;
+    const vbq_rans_batch_cta d = ctas[blockIdx.x];
+    const int CG = (C + 31) / 32;
+    bool ok = d.count >= 1 && d.count <= kRansWarps && d.first >= 0 && d.first <= n_units - d.count &&
+              d.table >= 0 && d.table < n_tables && d.cg >= 0 && d.cg < CG;
+    const int P = ok ? __ldg(prob_bits + d.table) : 0;
+    ok = ok && P >= 12 && P <= 16 && Q <= (1 << P);
+    if (!ok) {                                                         // CTA-uniform
+        if (threadIdx.x == 0) atomicOr(status, 8);
+        return;
+    }
+    const int cg = (int)d.cg;
+    const int nact = min(32, C - 32 * cg);
+    stage_group_table(sh_cum, sh_idx, cum + ((size_t)d.table * C + 32 * cg) * Q, nact, Q, P);
+
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (warp >= d.count) return;
+    const vbq_rans_batch_unit u = units[d.first + warp];
+    const bool blob_ok = u.blob >= 0 && u.blob < n_blobs;
+    // the word range holds the states, the rows fit the output: out + (rows - 1) C + nact <= n_out
+    const bool bad = !blob_ok || u.table != d.table || u.cg != d.cg || u.start < 0 || u.end > n_words ||
+                     u.end - u.start < 2ll * nact || u.rows < 1 || u.out < 0 || u.rows > n_out / C ||
+                     u.out > n_out - ((u.rows - 1) * C + nact);
+    int *st = status + (blob_ok ? u.blob : 0);
+    if (bad) {
+        if (lane == 0) atomicOr(st, 8);
+        return;
+    }
+    const bool active = lane < nact;
+    const int c = 32 * cg + lane;
+    const int err = vbq2_decode_group(words, u.start, u.end, 0, sh_cum + (active ? lane : 0) * Q,
+                                      sh_idx + (active ? lane : 0) * (kRansBuckets + 1), P, Q, nact, u.rows, C,
+                                      u.out + lane, code_points + (size_t)(active ? c : 0) * Q, qidx, zhat);
+    if (err && lane == 0) atomicOr(st, err);
 }
 
 // ---- the shared-table layout (vbq_rans_shared_*): one table per plane, symbols as one flat sequence ----------------
@@ -1081,6 +1152,40 @@ extern "C" int vbq_rans_decode(const unsigned short *d_payload, long long payloa
     VBQ_ENSURE_MAX_SMEM(vbq_rans_decode_kernel, dev);
     vbq_rans_decode_kernel<<<grid, kRansWarps * 32, smem, st>>>(d_payload, payload_words, d_group_bounds, d_cum, s,
                                                                 d_code_points, d_qidx, d_zhat, d_status);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+extern "C" int vbq_rans_decode_batch(const unsigned short *d_payload, long long payload_words,
+                                     const unsigned short *d_cum, const int *d_prob_bits, int n_tables, int C, int N,
+                                     const vbq_rans_batch_unit *d_units, long long n_units,
+                                     const vbq_rans_batch_cta *d_ctas, long long n_ctas, int n_blobs,
+                                     const float *d_code_points, long long n_out, int *d_qidx, float *d_zhat,
+                                     int *d_status, void *stream) {
+    if (N < 0 || N > 10) return vbq_fail(VBQ_ERR_BAD_DEPTH, "vbq_rans_decode_batch: N=%d (the coder holds N <= 10)", N);
+    if (payload_words < 0 || n_tables < 0 || C < 1 || C > 32 * 65535 || n_units < 0 || n_ctas < 0 ||
+        n_ctas > 2147483647ll || n_blobs < 0 || n_out < 0 || (n_ctas > 0 && (n_units < 1 || n_blobs < 1 || n_tables < 1)))
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "vbq_rans_decode_batch: payload_words=%lld n_tables=%d C=%d n_units=%lld "
+                        "n_ctas=%lld n_blobs=%d n_out=%lld", payload_words, n_tables, C, n_units, n_ctas, n_blobs, n_out);
+    const bool work = n_ctas > 0;
+    if ((n_blobs > 0 && !d_status) || (d_zhat && !d_code_points) ||
+        (work && (!d_payload || !d_cum || !d_prob_bits || !d_units || !d_ctas)))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_decode_batch: null pointer");
+    if (((uintptr_t)d_payload & 1) || ((uintptr_t)d_cum & 1) || ((uintptr_t)d_prob_bits & 3) ||
+        ((uintptr_t)d_units & 7) || ((uintptr_t)d_ctas & 7) || ((uintptr_t)d_code_points & 3) ||
+        ((uintptr_t)d_qidx & 3) || ((uintptr_t)d_zhat & 3) || ((uintptr_t)d_status & 3))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_decode_batch: misaligned pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (n_blobs > 0) CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int) * (size_t)n_blobs, st));
+    if (!work) return VBQ_OK;
+    int dev = 0, sms = 0;
+    RETURN_IF(vbq_current_device(&dev, &sms));
+    const int Q = (1 << (N + 1)) - 1;
+    const size_t smem = (size_t)32 * (Q + kRansBuckets + 1) * sizeof(unsigned short);
+    VBQ_ENSURE_MAX_SMEM(vbq_rans_decode_batch_kernel, dev);
+    vbq_rans_decode_batch_kernel<<<(unsigned)n_ctas, kRansWarps * 32, smem, st>>>(
+        d_payload, payload_words, d_cum, d_prob_bits, n_tables, C, Q, d_units, n_units, d_ctas, n_blobs,
+        d_code_points, n_out, d_qidx, d_zhat, d_status);
     CUDA_TRY(cudaGetLastError());
     return VBQ_OK;
 }

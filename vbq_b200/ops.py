@@ -648,6 +648,45 @@ def rans_decode(words: torch.Tensor, bounds: torch.Tensor, cum: torch.Tensor, it
     return q, z, status
 
 
+BATCH_UNIT_FIELDS = 7       # vbq_rans_batch_unit: start, end, out, rows, table, cg, blob (int64 each)
+BATCH_CTA_FIELDS = 4        # vbq_rans_batch_cta: first, count, table, cg (int64 each)
+
+
+def rans_decode_batch(words: torch.Tensor, cum: torch.Tensor, prob_bits: torch.Tensor, units: torch.Tensor,
+                      ctas: torch.Tensor, n_blobs: int, max_bits: int, n_out: int,
+                      code_points: Optional[torch.Tensor] = None, want_qidx: bool = True):
+    """The work-list decoder of many VBQ2 streams in one launch.  words: the payloads as int16 words; cum (n_tables,
+    C, Q) int16; prob_bits (n_tables,) int32; units (n_units, 7) and ctas (n_ctas, 4) int64 (vbq_rans_batch_unit /
+    vbq_rans_batch_cta).  Returns (qidx or None, zhat or None, status): flat (n_out,) int32 symbols and float32
+    code_points[c, q] (code_points (C, Q) ascending), and the (n_blobs,) int32 device status per blob (bits 1, 2, 4 of
+    rans_decode, 8 for a bad unit).  No synchronisation."""
+    for name, t, dt, nd in (("words", words, torch.int16, 1), ("cum", cum, torch.int16, 3),
+                            ("prob_bits", prob_bits, torch.int32, 1), ("units", units, torch.int64, 2),
+                            ("ctas", ctas, torch.int64, 2)):
+        _need_cuda(name, t, dt, nd)
+    if units.shape[1] != BATCH_UNIT_FIELDS or ctas.shape[1] != BATCH_CTA_FIELDS:
+        raise ValueError("vbq_b200: `units` must be (n, %d) and `ctas` (n, %d), got %s and %s" % (
+            BATCH_UNIT_FIELDS, BATCH_CTA_FIELDS, tuple(units.shape), tuple(ctas.shape)))
+    n_tables, C, _ = cum.shape
+    if prob_bits.numel() != n_tables:
+        raise ValueError("vbq_b200: %d prob_bits for %d tables" % (prob_bits.numel(), n_tables))
+    dev = words.device
+    q = torch.empty(n_out, dtype=torch.int32, device=dev) if want_qidx else None
+    z = None
+    if code_points is not None:
+        _need_cuda("code_points", code_points, torch.float32, 2)
+        if tuple(code_points.shape) != tuple(cum.shape[1:]):
+            raise ValueError("vbq_b200: code_points are %s, need (C, Q) = %s" % (tuple(code_points.shape),
+                                                                              tuple(cum.shape[1:])))
+        z = torch.empty(n_out, dtype=torch.float32, device=dev)
+    status = torch.zeros(n_blobs, dtype=torch.int32, device=dev)
+    st = _lib.load().vbq_rans_decode_batch(_ptr(words), words.numel(), _ptr(cum), _ptr(prob_bits), n_tables, C,
+                                           max_bits, _ptr(units), units.shape[0], _ptr(ctas), ctas.shape[0], n_blobs,
+                                           _ptr(code_points), n_out, _ptr(q), _ptr(z), _ptr(status), _stream(dev))
+    _lib.check(st, "vbq_rans_decode_batch")
+    return q, z, status
+
+
 # ------------------------------------------------------------------------------------------------------
 # entropy coding with one shared table per plane, symbols as one flat sequence (word embeddings; include/vbq_b200.h)
 # ------------------------------------------------------------------------------------------------------

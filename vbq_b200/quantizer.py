@@ -422,18 +422,44 @@ class ChannelwisePriorCDFQuantizer:
         """z_hat of a `compress_to_bytes` blob as a device tensor (1, H', W', C) (several items or planes stack on the
         first axis).  The blob's lambda selects the entropy model by float equality, as the dict keys do."""
         h = serialize.read_header(blob)
+        tables = self._blob_tables(h)
+        out = serialize.decode(blob, tables=tables, code_points=self.code_points_by_channel, device=self.device,
+                               want_qidx=False)
+        return out["zhat"].reshape(self._image_shape(out))
+
+    def _blob_tables(self, h):
+        """The cached rans_tables of a VBQ2 header's planes; KeyError for a lambda without an entropy model."""
         keys = []
         for lam in h["lambdas"]:
             k = [l for l in (self.entropy_models or {}) if float(l) == lam]
             if not k:
                 raise KeyError(lam)
             keys.append(k[0])
-        tables = [self.rans_tables(k, h["prob_bits"]) for k in keys]
-        out = serialize.decode(blob, tables=tables, code_points=self.code_points_by_channel, device=self.device,
-                               want_qidx=False)
-        z = out["zhat"]
-        Hp = out["height"] or out["item_rows"]
-        return z.reshape(-1, Hp, out["item_rows"] // max(1, Hp), self.num_channels)
+        return [self.rans_tables(k, h["prob_bits"]) for k in keys]
+
+    def _image_shape(self, h):
+        Hp = h["height"] or h["item_rows"]
+        return (-1, Hp, h["item_rows"] // max(1, Hp), self.num_channels)
+
+    def decompress_many(self, blobs, stack=False):
+        """`decompress_from_bytes` of every blob of a list (e.g. all the blobs of `compress_to_bytes`, any mix of
+        lambdas and shapes) in one kernel launch: a list of device tensors, each exactly what `decompress_from_bytes`
+        returns for its blob and each a view into one device buffer.  stack=True returns that buffer as one
+        (B, H', W', C) tensor, without a copy, ready for `vae.decode`; it needs every blob to have the same shape and
+        raises ValueError otherwise.  An unknown lambda raises KeyError before any launch."""
+        blobs = list(blobs)
+        if not blobs:
+            return []
+        headers = [serialize.read_header(b) for b in blobs]
+        plane_tables = [[(("obj", id(t)), t) for t in self._blob_tables(h)] for h in headers]
+        shapes = [(h["n_planes"] * h["items"],) + self._image_shape(h)[1:] for h in headers]
+        if stack and len(set(shapes)) > 1:
+            raise ValueError("vbq_b200: stack=True needs blobs of one shape, got %s" % sorted(set(shapes)))
+        outs, _, z = serialize.decode_blobs(blobs, headers, plane_tables, code_points=self.code_points_by_channel,
+                                            device=self.device, want_qidx=False)
+        if stack:
+            return z.view(self._image_shape(headers[0]))
+        return [o["zhat"].view(self._image_shape(o)) for o in outs]
 
     @property
     def lambs(self):

@@ -275,10 +275,7 @@ def decode(data: bytes, tables=None, code_points=None, device="cuda", want_qidx:
             raise ValueError("vbq_b200.serialize: the frequency table of plane %d (lambda %r) has another fingerprint "
                              "than the one the stream was coded with" % (i, h["lambdas"][i]))
     t = coding.check_tables(t, P)
-    rest = len(data) - h["payload_offset"]
-    if rest % 2:
-        raise ValueError("vbq_b200.serialize: payload of odd length")
-    words = np.frombuffer(data, dtype="<u2", count=rest // 2, offset=h["payload_offset"])
+    words = _payload_words(data, h)
     bounds = _group_bounds(words, h)
     dev = torch.device(device)
     w = torch.from_numpy(words.view(np.int16).copy()).to(dev)
@@ -288,12 +285,175 @@ def decode(data: bytes, tables=None, code_points=None, device="cuda", want_qidx:
     q, z, status = ops.rans_decode(w, b, cum, h["items"], h["item_rows"], h["seg_rows"], N, P, cp, want_qidx)
     st = int(status.item())
     if st:
-        raise ValueError("vbq_b200.serialize: corrupt VBQ2 payload (decoder status %d: %s)" % (
-            st, ", ".join(m for bit, m in ((1, "a group ran out of words"), (2, "integrity check failed"),
-                                            (4, "bad group range or initial state")) if st & bit)))
+        raise ValueError("vbq_b200.serialize: corrupt VBQ2 payload (decoder status %d: %s)" % (st, _status_text(st)))
     out = {k: v for k, v in h.items() if k not in ("tables", "payload_offset")}
     out.update(qidx=q, zhat=z)
     return out
+
+
+def _payload_words(data, h):
+    rest = len(data) - h["payload_offset"]
+    if rest % 2:
+        raise ValueError("vbq_b200.serialize: payload of odd length")
+    return np.frombuffer(data, dtype="<u2", count=rest // 2, offset=h["payload_offset"])
+
+
+_STATUS_BITS = ((1, "a group ran out of words"), (2, "integrity check failed"), (4, "bad group range or initial state"),
+                (8, "bad work unit"))
+
+
+def _status_text(st):
+    return ", ".join(m for bit, m in _STATUS_BITS if st & bit)
+
+
+# ------------------------------------------------------------------------------------------------------
+# many VBQ2 blobs in one launch (vbq_rans_decode_batch)
+# ------------------------------------------------------------------------------------------------------
+BATCH_CTA_UNITS = 8         # units per CTA descriptor: the decoder's warps per CTA
+
+
+def batch_plan(headers, payloads, table_ids):
+    """The work list of `decode_many` (host only).  headers: `read_header` dicts of blobs sharing C; payloads: each
+    blob's payload as uint16 words; table_ids: per blob, the table index of each plane.  Checks every offset table and
+    returns dict(words: the payloads back to back, units (U, 7) int64 (vbq_rans_batch_unit: start, end, out, rows,
+    table, cg, blob), ctas (K, 4) int64 (vbq_rans_batch_cta: first, count, table, cg), offsets: each blob's first output
+    element, sizes: its element count, n_out).  Blob b's output block is (n_planes, items, item_rows, C) at
+    offsets[b].  Units are ordered by (table, cg), then blob, plane, item, segment, and each descriptor takes up to
+    BATCH_CTA_UNITS consecutive units of one (table, cg)."""
+    B = len(headers)
+    C = headers[0]["C"] if B else 1
+    CG = -(-C // 32)
+    f = {k: np.array([h[k] for h in headers], dtype=np.int64) for k in ("n_planes", "items", "item_rows", "seg_rows")}
+    L, items, item_rows, seg = f["n_planes"], f["items"], f["item_rows"], f["seg_rows"]
+    n_segs = -(-item_rows // seg)
+    G = L * items * n_segs * CG
+    sizes = L * items * item_rows * C
+    offsets = np.cumsum(sizes) - sizes
+    lens = np.array([p.size for p in payloads], dtype=np.int64)
+    bases = np.cumsum(lens) - lens
+    # group ranges of every blob, in (plane, item, segment, cg) order, moved to the concatenated payload
+    bounds = [_group_bounds(p, h) + base for p, h, base in zip(payloads, headers, bases)]
+    bounds = np.concatenate(bounds) if B else np.zeros((0, 2), np.int64)
+    blob = np.repeat(np.arange(B, dtype=np.int64), G)
+    g = np.arange(int(G.sum()), dtype=np.int64) - np.repeat(np.cumsum(G) - G, G)
+    cg = g % CG
+    rest = g // CG
+    sg = rest % n_segs[blob]
+    rest //= n_segs[blob]
+    item = rest % items[blob]
+    plane = rest // items[blob]
+    r0 = sg * seg[blob]
+    rows = np.minimum(seg[blob], item_rows[blob] - r0)
+    out = offsets[blob] + ((plane * items[blob] + item) * item_rows[blob] + r0) * C + 32 * cg
+    tids = np.array([t for ids in table_ids for t in ids], dtype=np.int64)
+    table = tids[(np.cumsum(L) - L)[blob] + plane]
+    units = np.stack([bounds[:, 0], bounds[:, 1], out, rows, table, cg, blob], axis=1)
+    U = units.shape[0]
+    units = units[np.lexsort((np.arange(U), cg, table))]
+    key = units[:, 4] * CG + units[:, 5]
+    new_run = np.ones(U, bool)
+    new_run[1:] = key[1:] != key[:-1]
+    run_starts = np.flatnonzero(new_run)
+    run = np.cumsum(new_run) - 1
+    pos = np.arange(U) - run_starts[run]
+    first = np.flatnonzero(pos % BATCH_CTA_UNITS == 0)
+    run_ends = np.append(run_starts[1:], U)
+    count = np.minimum(BATCH_CTA_UNITS, run_ends[run[first]] - first)
+    ctas = np.stack([first, count, units[first, 4], units[first, 5]], axis=1).astype(np.int64)
+    words = np.concatenate(payloads) if B else np.zeros(0, np.uint16)
+    return dict(words=words, units=np.ascontiguousarray(units), ctas=ctas, offsets=offsets, sizes=sizes,
+                n_out=int(sizes.sum()))
+
+
+def _resolve_tables(h, tables, b):
+    """The tables argument of `decode_many` for blob b: per plane a (key, table) pair, where equal keys mean the same
+    table object (fingerprinted once)."""
+    L = h["n_planes"]
+    if tables is None:
+        if h["tables"] is None:
+            raise ValueError("vbq_b200.serialize: blob %d embeds no frequency tables; pass `tables`" % b)
+        return [(("blob", b, i), h["tables"][i]) for i in range(L)]
+    if isinstance(tables, dict):
+        try:
+            return [(("obj", id(tables[lam])), tables[lam]) for lam in h["lambdas"]]
+        except KeyError as e:
+            raise ValueError("vbq_b200.serialize: blob %d: no table for lambda %r" % (b, e.args[0]))
+    if isinstance(tables, (list, tuple)):
+        if len(tables) != L:
+            raise ValueError("vbq_b200.serialize: blob %d has %d planes, got %d tables" % (b, L, len(tables)))
+        return [(("obj", id(t)), t) for t in tables]
+    t = np.asarray(tables)
+    if t.ndim == 2:
+        return [(("obj", id(tables)), t)] * L
+    t = _as_tables(t, L)
+    return [(("obj", id(tables), i), t[i]) for i in range(L)]
+
+
+def decode_blobs(blobs, headers, plane_tables, code_points=None, device="cuda", want_qidx: bool = True):
+    """`decode_many` with parsed headers and resolved tables (plane_tables: per blob a list of (key, table) pairs as
+    `_resolve_tables` makes them).  Returns (list of result dicts, flat qidx or None, flat zhat or None): every result
+    tensor is a view into the flat buffers, in blob order."""
+    if not blobs:
+        return [], None, None
+    C, N = headers[0]["C"], headers[0]["max_bits"]
+    for b, h in enumerate(headers):
+        if (h["C"], h["max_bits"]) != (C, N):
+            raise ValueError("vbq_b200.serialize: blob %d has C=%d N=%d, blob 0 has C=%d N=%d; one call decodes "
+                             "blobs of one quantizer" % (b, h["C"], h["max_bits"], C, N))
+    Q = ops.num_levels(N)
+    ids, distinct, table_ids = {}, [], []
+    for b, (h, pt) in enumerate(zip(headers, plane_tables)):
+        row = []
+        for i, (key, table) in enumerate(pt):
+            if key not in ids:
+                t = np.asarray(table)
+                if t.shape != (C, Q):
+                    raise ValueError("vbq_b200.serialize: blob %d: tables are %s, the blob needs (%d, %d)"
+                                     % (b, t.shape, C, Q))
+                P = coding.prob_bits_of(t)
+                ids[key] = len(distinct)
+                distinct.append((coding.check_tables(t, P), coding.fingerprint(t), P))
+            tid = ids[key]
+            if distinct[tid][1] != h["fingerprints"][i] or distinct[tid][2] != h["prob_bits"]:
+                raise ValueError("vbq_b200.serialize: blob %d: the frequency table of plane %d (lambda %r) has another "
+                                 "fingerprint than the one the stream was coded with" % (b, i, h["lambdas"][i]))
+            row.append(tid)
+        table_ids.append(row)
+    plan = batch_plan(headers, [_payload_words(d, h) for d, h in zip(blobs, headers)], table_ids)
+    dev = torch.device(device)
+    w = torch.from_numpy(plan["words"].view(np.int16)).to(dev)
+    cum = torch.from_numpy(np.stack([coding.cum_table(t) for t, _, _ in distinct]).view(np.int16)).to(dev)
+    pb = torch.tensor([P for _, _, P in distinct], dtype=torch.int32).to(dev)
+    units = torch.from_numpy(plan["units"]).to(dev)
+    ctas = torch.from_numpy(plan["ctas"]).to(dev)
+    cp = None if code_points is None else code_points.to(device=dev, dtype=torch.float32).contiguous()
+    q, z, status = ops.rans_decode_batch(w, cum, pb, units, ctas, len(blobs), N, plan["n_out"], cp, want_qidx)
+    st = status.cpu().numpy()
+    bad = np.flatnonzero(st)
+    if bad.size:
+        raise ValueError("vbq_b200.serialize: corrupt VBQ2 payload in blob%s %s (%s)" % (
+            "s" if bad.size > 1 else "", ", ".join(str(b) for b in bad),
+            "; ".join("blob %d: decoder status %d: %s" % (b, st[b], _status_text(int(st[b]))) for b in bad)))
+    outs = []
+    for h, o, n in zip(headers, plan["offsets"].tolist(), plan["sizes"].tolist()):
+        shape = (h["n_planes"], h["items"], h["item_rows"], C)
+        r = {k: v for k, v in h.items() if k not in ("tables", "payload_offset")}
+        r.update(qidx=None if q is None else q[o:o + n].view(shape), zhat=None if z is None else z[o:o + n].view(shape))
+        outs.append(r)
+    return outs, q, z
+
+
+def decode_many(blobs, tables=None, code_points=None, device="cuda", want_qidx: bool = True) -> list:
+    """`decode` of every blob of a list in one kernel launch: a list of dicts, one per blob, each equal to what
+    `decode` returns for that blob (qidx / zhat are views into one device buffer each).  The blobs may differ in
+    lambda, prob_bits, seg_rows, item_rows, height, n_planes and items, and must share C and N.  tables: as for
+    `decode`, applied to every blob.  Every header, table fingerprint and offset table is checked before anything is
+    uploaded; a payload that fails the decoder's integrity check raises ValueError naming the failing blobs and their
+    status bits, and no result is returned."""
+    blobs = list(blobs)
+    headers = [read_header(d) for d in blobs]
+    plane_tables = [_resolve_tables(h, tables, b) for b, h in enumerate(headers)]
+    return decode_blobs(blobs, headers, plane_tables, code_points, device, want_qidx)[0]
 
 
 # ------------------------------------------------------------------------------------------------------
