@@ -314,6 +314,58 @@ int vbq_rans_decode_batch(const unsigned short *d_payload, long long payload_wor
                           const float *d_code_points, long long n_out, int *d_qidx, float *d_zhat, int *d_status,
                           void *stream);
 
+/* ---- many images in one launch: the work-list encoder (DESIGN.md §8i) --------------------------------------------
+ *
+ * vbq_rans_encode_batch codes any set of groups of the layout above, from any number of images that share C and N but
+ * may differ in rows, table, prob_bits and seg_rows, into n_blobs BLOBS back to back in d_payload.  Each blob is one
+ * plane of one item: exactly the payload vbq_rans_encode writes for that item alone (its group end offset table, then
+ * its groups).  Each group is a UNIT.  Inputs:
+ *   d_in         (n_in,) int32 symbols; a unit codes rows r = 0 .. rows - 1 of lanes j < nact = min(32, C - 32 cg),
+ *                symbol (r, j) at element in + r C + j;
+ *   d_cum, d_prob_bits, n_tables: as for vbq_rans_decode_batch;
+ *   d_units      (n_units,) vbq_rans_encode_unit;
+ *   d_ctas       (n_ctas,) vbq_rans_batch_cta: CTA i codes units [first, first + count), 1 <= count <= 8, which must all
+ *                have the descriptor's (table, cg): the CTA stages that table set once;
+ *   d_blob_groups (n_blobs + 1,) int64: the first group of each blob in blob-major group order, [n_blobs] = n_groups;
+ *   d_workspace  vbq_rans_encode_batch_workspace_bytes(n_groups, scratch_words) bytes: three int64 arrays of n_groups
+ *                entries, then the scratch, in which unit u writes at most nact (rows + 2) words from word u.scratch on
+ *                (the Python planner gives every unit its own range).
+ * Outputs (no host synchronisation):
+ *   d_payload    (payload_words,) uint16: blob b occupies words [d_blob_starts[b], d_blob_starts[b + 1]);
+ *                2 n_groups + scratch_words words always suffice;
+ *   d_blob_starts (n_blobs + 1,) int64, [n_blobs] = the payload size in words;
+ *   d_status     (n_blobs,) int32, zeroed by the call: bit 1 if a symbol of the blob's groups lies outside [0, Q), bit 8
+ *                for a bad unit or descriptor (of blob 0 if no valid blob id names the fault, as in
+ *                vbq_rans_decode_batch), and bit 8 of blob 0 if d_blob_groups does not run from 0 to n_groups without
+ *                decreasing (then every blob start is 0 and nothing is moved to the payload).
+ * Units and descriptors come from the caller's memory, so the kernel checks each before it acts: 0 <= in and
+ * in + (rows - 1) C + nact <= n_in, rows >= 1, table and cg in range and equal to the descriptor's, the table's
+ * prob_bits valid, 0 <= group < n_groups, 0 <= blob < n_blobs, and 0 <= scratch with scratch + nact (rows + 2) inside
+ * the workspace's scratch.  A bad unit writes no scratch and leaves its group's size 0.  Every write of the scan and the
+ * compaction stays inside d_payload and the workspace whatever the units say; units that name one group twice, or
+ * whose scratch ranges overlap, give an unspecified payload but no access out of bounds.  A blob's group data must stay
+ * below 2^32 words (its offset table is 32-bit); the caller checks this from the worst case, nact (rows + 2) words per
+ * group.  The scan is one CTA of 1,024 threads that walks the groups 1,024 at a time, so its time grows linearly with
+ * n_groups (n_groups < 2^31).
+ * Status codes: VBQ_ERR_BAD_DEPTH for N > 10, VBQ_ERR_BAD_SHAPE for a bad count or C, VBQ_ERR_WORKSPACE for a workspace
+ * smaller than the three index arrays. */
+typedef struct {
+    long long in;           /* element of row 0, lane 0 in d_in */
+    long long rows;         /* rows of the segment */
+    long long table, cg;    /* table id in d_cum, 32-channel group */
+    long long group;        /* the group's index in blob-major order */
+    long long scratch;      /* first word of the unit's scratch range */
+    long long blob;         /* the d_status entry this unit reports to */
+} vbq_rans_encode_unit;     /* 56 bytes: an (n_units, 7) int64 array */
+
+long long vbq_rans_encode_batch_workspace_bytes(long long n_groups, long long scratch_words);
+int vbq_rans_encode_batch(const int *d_in, long long n_in, const unsigned short *d_cum, const int *d_prob_bits,
+                          int n_tables, int C, int N, const vbq_rans_encode_unit *d_units, long long n_units,
+                          const vbq_rans_batch_cta *d_ctas, long long n_ctas, const long long *d_blob_groups,
+                          int n_blobs, long long n_groups, unsigned short *d_payload, long long payload_words,
+                          long long *d_blob_starts, int *d_status, void *d_workspace, long long workspace_bytes,
+                          void *stream);
+
 /* ---- entropy coding with one shared table per plane: word embeddings (DESIGN.md §8d) ------------------------------
  *
  * All coordinates of an embedding matrix share one prior and one empirical model, so the channel axis of the layout

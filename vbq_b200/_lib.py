@@ -84,6 +84,9 @@ SIGNATURES = {
     "vbq_rans_encode": (_i, [_p, _i, _i, _ll, _i, _ll, _i, _i, _p, _p, _ll, _p, _p, _p, _ll, _p]),
     "vbq_rans_decode": (_i, [_p, _ll, _p, _i, _i, _ll, _i, _ll, _i, _i, _p, _p, _p, _p, _p, _p]),
     "vbq_rans_decode_batch": (_i, [_p, _ll, _p, _p, _i, _i, _i, _p, _ll, _p, _ll, _i, _p, _ll, _p, _p, _p, _p]),
+    "vbq_rans_encode_batch_workspace_bytes": (_ll, [_ll, _ll]),
+    "vbq_rans_encode_batch": (_i, [_p, _ll, _p, _p, _i, _i, _i, _p, _ll, _p, _ll, _p, _i, _ll, _p, _ll, _p, _p, _p,
+                                   _ll, _p]),
     "vbq_rans_shared_workspace_bytes": (_ll, [_i, _ll, _p]),
     "vbq_rans_shared_payload_bound": (_ll, [_i, _ll, _p]),
     "vbq_rans_shared_encode": (_i, [_p, _i, _ll, _p, _i, _i, _p, _p, _ll, _p, _p, _p, _ll, _p]),

@@ -75,8 +75,63 @@ __device__ __forceinline__ unsigned lanemask_lt() {
 
 constexpr int kEncBlock = 16;   // rows whose symbols are loaded together (the next block's loads overlap the coding)
 
-// One warp per (item, segment) of the CTA's channel group: rows last to first, lanes high to low, words written back
-// to front into the group's scratch region [base, base + nact (seg_rows + 2)).
+// One warp encodes one group of len rows and nact lanes: rows last to first, lanes high to low, words written back to
+// front into scratch below `end`, then the lanes' final states.  src (already offset to the lane's channel) + t C is
+// the lane's symbol of row t, tab the lane's cum table.  Returns the group's first word (its states, then its words);
+// `bad` becomes 1 on a lane that met a symbol outside [0, Q) (coded as symbol 0).
+__device__ __forceinline__ long long rans_encode_group(const int *__restrict__ src, int C, long long len, int nact,
+                                                       const unsigned short *tab, int P, int Q,
+                                                       unsigned short *__restrict__ scratch, long long end,
+                                                       int &bad) {
+    const int lane = threadIdx.x & 31;
+    const bool active = lane < nact;
+    const unsigned top = 1u << P;
+    const int fshift = 32 - P;
+    long long pos = end;
+    unsigned x = kRansL;
+    const unsigned lt = lanemask_lt();
+
+    int cur[kEncBlock], nxt[kEncBlock];
+#pragma unroll
+    for (int k = 0; k < kEncBlock; ++k) {
+        const long long t = len - 1 - k;
+        cur[k] = (active && t >= 0) ? __ldg(src + t * C) : 0;
+    }
+    for (long long t0 = len - 1; t0 >= 0; t0 -= kEncBlock) {
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) {
+            const long long t = t0 - kEncBlock - k;
+            nxt[k] = (active && t >= 0) ? __ldg(src + t * C) : 0;
+        }
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) {
+            if (t0 - k < 0) break;                         // warp-uniform
+            int sym = cur[k];
+            if (sym < 0 || sym >= Q) { bad = 1; sym = 0; }
+            const unsigned lo = tab[sym];
+            const unsigned f = (sym + 1 < Q ? (unsigned)tab[sym + 1] : top) - lo;
+            const bool emit = active && (unsigned long long)x >= ((unsigned long long)f << fshift);
+            const unsigned mask = __ballot_sync(0xffffffffu, emit);
+            pos -= __popc(mask);
+            if (emit) {
+                scratch[pos + __popc(mask & lt)] = (unsigned short)(x & 0xffffu);
+                x >>= 16;
+            }
+            if (active) x = ((x / f) << P) + (x % f) + lo;
+        }
+#pragma unroll
+        for (int k = 0; k < kEncBlock; ++k) cur[k] = nxt[k];
+    }
+    pos -= 2 * nact;
+    if (active) {
+        scratch[pos + 2 * lane] = (unsigned short)(x & 0xffffu);
+        scratch[pos + 2 * lane + 1] = (unsigned short)(x >> 16);
+    }
+    return pos;
+}
+
+// One warp per (item, segment) of the CTA's channel group, coded into the group's scratch region
+// [base, base + nact (seg_rows + 2)).
 __global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_encode_kernel(const int *__restrict__ qidx,
                                                                          const unsigned short *__restrict__ cum,
                                                                          RansShape s,
@@ -97,56 +152,67 @@ __global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_encode_kernel(const 
     const bool active = lane < nact;
     const int c = 32 * cg + lane;
     const int *src = qidx + (((long long)plane * s.items + item) * s.item_rows + r0) * s.C + c;
-    const unsigned short *tab = sh_cum + (active ? lane : 0) * s.Q;
-    const unsigned top = 1u << s.P;
-    const int fshift = 32 - s.P;
     const long long base = ((long long)plane * s.items * s.n_segs + unit) * s.C * (s.seg_rows + 2) +
                            32ll * cg * (s.seg_rows + 2);
     const long long end = base + (long long)nact * (s.seg_rows + 2);
-    long long pos = end;
-    unsigned x = kRansL;
     int bad = 0;
-    const unsigned lt = lanemask_lt();
-
-    int cur[kEncBlock], nxt[kEncBlock];
-#pragma unroll
-    for (int k = 0; k < kEncBlock; ++k) {
-        const long long t = len - 1 - k;
-        cur[k] = (active && t >= 0) ? __ldg(src + t * s.C) : 0;
-    }
-    for (long long t0 = len - 1; t0 >= 0; t0 -= kEncBlock) {
-#pragma unroll
-        for (int k = 0; k < kEncBlock; ++k) {
-            const long long t = t0 - kEncBlock - k;
-            nxt[k] = (active && t >= 0) ? __ldg(src + t * s.C) : 0;
-        }
-#pragma unroll
-        for (int k = 0; k < kEncBlock; ++k) {
-            if (t0 - k < 0) break;                         // warp-uniform
-            int sym = cur[k];
-            if (sym < 0 || sym >= s.Q) { bad = 1; sym = 0; }
-            const unsigned lo = tab[sym];
-            const unsigned f = (sym + 1 < s.Q ? (unsigned)tab[sym + 1] : top) - lo;
-            const bool emit = active && (unsigned long long)x >= ((unsigned long long)f << fshift);
-            const unsigned mask = __ballot_sync(0xffffffffu, emit);
-            pos -= __popc(mask);
-            if (emit) {
-                scratch[pos + __popc(mask & lt)] = (unsigned short)(x & 0xffffu);
-                x >>= 16;
-            }
-            if (active) x = ((x / f) << s.P) + (x % f) + lo;
-        }
-#pragma unroll
-        for (int k = 0; k < kEncBlock; ++k) cur[k] = nxt[k];
-    }
-    pos -= 2 * nact;
-    if (active) {
-        scratch[pos + 2 * lane] = (unsigned short)(x & 0xffffu);
-        scratch[pos + 2 * lane + 1] = (unsigned short)(x >> 16);
-    }
+    const long long pos = rans_encode_group(src, s.C, len, nact, sh_cum + (active ? lane : 0) * s.Q, s.P, s.Q, scratch,
+                                            end, bad);
     const long long g = (((long long)plane * s.items * s.n_segs + unit) * s.CG + cg);
     if (lane == 0) sizes[g] = end - pos;
     if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(status, 1);
+}
+
+// The work-list encoder of many images (vbq_rans_encode_batch): CTA i stages the table set (table, cg) of descriptor i
+// and its warp w codes unit first + w into the unit's scratch range, then records the group's size and scratch end.
+// Every field of the descriptor and the unit comes from the caller's memory and is checked before it is used: a bad
+// one sets status bit 8 (of the unit's blob if its blob id is in range, else of blob 0) and writes nothing.
+__global__ void __launch_bounds__(kRansWarps * 32) vbq_rans_encode_batch_kernel(
+        const int *__restrict__ in, long long n_in, const unsigned short *__restrict__ cum,
+        const int *__restrict__ prob_bits, int n_tables, int C, int Q, const vbq_rans_encode_unit *__restrict__ units,
+        long long n_units, const vbq_rans_batch_cta *__restrict__ ctas, int n_blobs, long long n_groups,
+        unsigned short *__restrict__ scratch, long long scratch_words, long long *__restrict__ sizes,
+        long long *__restrict__ ends, int *__restrict__ status) {
+    extern __shared__ unsigned short sh_cum[];   // [nact][Q]
+    const vbq_rans_batch_cta d = ctas[blockIdx.x];
+    const int CG = (C + 31) / 32;
+    bool ok = d.count >= 1 && d.count <= kRansWarps && d.first >= 0 && d.first <= n_units - d.count &&
+              d.table >= 0 && d.table < n_tables && d.cg >= 0 && d.cg < CG;
+    const int P = ok ? __ldg(prob_bits + d.table) : 0;
+    ok = ok && P >= 12 && P <= 16 && Q <= (1 << P);
+    if (!ok) {                                                         // CTA-uniform
+        if (threadIdx.x == 0) atomicOr(status, 8);
+        return;
+    }
+    const int cg = (int)d.cg;
+    const int nact = min(32, C - 32 * cg);
+    const unsigned short *src_cum = cum + ((size_t)d.table * C + 32 * cg) * Q;
+    for (int i = threadIdx.x; i < nact * Q; i += blockDim.x) sh_cum[i] = __ldg(src_cum + i);
+    __syncthreads();
+
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (warp >= d.count) return;
+    const vbq_rans_encode_unit u = units[d.first + warp];
+    const bool blob_ok = u.blob >= 0 && u.blob < n_blobs;
+    // the rows lie in the input (in + (rows - 1) C + nact <= n_in) and the worst case in the scratch
+    const bool bad = !blob_ok || u.table != d.table || u.cg != d.cg || u.rows < 1 || u.in < 0 || u.rows > n_in / C ||
+                     u.in > n_in - ((u.rows - 1) * C + nact) || u.group < 0 || u.group >= n_groups ||
+                     u.scratch < 0 || u.scratch > scratch_words - nact * (u.rows + 2);
+    int *st = status + (blob_ok ? u.blob : 0);
+    if (bad) {
+        if (lane == 0) atomicOr(st, 8);
+        return;
+    }
+    const bool active = lane < nact;
+    const long long end = u.scratch + nact * (u.rows + 2);
+    int sym_bad = 0;
+    const long long pos = rans_encode_group(in + u.in + lane, C, u.rows, nact, sh_cum + (active ? lane : 0) * Q, P, Q,
+                                            scratch, end, sym_bad);
+    if (lane == 0) {
+        sizes[u.group] = end - pos;
+        ends[u.group] = end;
+    }
+    if (__any_sync(0xffffffffu, sym_bad) && lane == 0) atomicOr(st, 1);
 }
 
 // Block-wide inclusive sum of one value per thread (blockDim.x a multiple of 32, at most 1024).
@@ -222,6 +288,81 @@ __global__ void vbq_rans_compact_kernel(const unsigned short *__restrict__ scrat
     const unsigned short *src = scratch + end - n;
     unsigned short *d = out + dst[g];
     for (long long i = threadIdx.x; i < n; i += blockDim.x) d[i] = src[i];
+}
+
+// One CTA: the blobs of vbq_rans_encode_batch back to back.  blob_groups (n_blobs + 1) gives each blob's first group
+// in blob-major order; it comes from the caller's memory, so unless it runs from 0 to n_groups without decreasing the
+// kernel sets bit 8 of blob 0, zeroes blob_starts and marks every group as not to be moved (dst = -1).  Otherwise:
+// dst[g] = the exclusive prefix of the sizes (first pass), blob_starts[b] = 2 (first group) + prefix at the first group
+// (second pass), then each group's offset-table entry and its destination word (third pass; a group finds its blob by
+// binary search).  Table words that would fall outside the payload are not written.
+__global__ void __launch_bounds__(1024) vbq_rans_encode_batch_scan_kernel(
+        const long long *__restrict__ sizes, long long *__restrict__ dst, long long n_groups,
+        const long long *__restrict__ blob_groups, int n_blobs, unsigned short *__restrict__ out, long long out_words,
+        long long *__restrict__ blob_starts, int *__restrict__ status) {
+    __shared__ long long sh_warp[32];
+    bool bad = false;
+    for (int b = threadIdx.x; b <= n_blobs; b += blockDim.x) {
+        const long long g = blob_groups[b];
+        bad = bad || (b == 0 ? g != 0 : g < blob_groups[b - 1]) || (b == n_blobs && g != n_groups);
+    }
+    if (__syncthreads_or(bad)) {
+        for (int b = threadIdx.x; b <= n_blobs; b += blockDim.x) blob_starts[b] = 0;
+        for (long long g = threadIdx.x; g < n_groups; g += blockDim.x) dst[g] = -1;
+        if (threadIdx.x == 0) atomicOr(status, 8);
+        return;
+    }
+    long long total = 0;
+    for (long long c0 = 0; c0 < n_groups; c0 += blockDim.x) {
+        const long long i = c0 + threadIdx.x;
+        const long long v = i < n_groups ? sizes[i] : 0;
+        long long chunk;
+        const long long incl = block_inclusive_sum(v, sh_warp, &chunk);
+        if (i < n_groups) dst[i] = total + incl - v;
+        total += chunk;
+    }
+    __syncthreads();
+    for (int b = threadIdx.x; b <= n_blobs; b += blockDim.x) {
+        const long long g = blob_groups[b];
+        blob_starts[b] = 2 * g + (g < n_groups ? dst[g] : total);
+    }
+    __syncthreads();
+    for (long long g = threadIdx.x; g < n_groups; g += blockDim.x) {
+        int lo = 0, hi = n_blobs - 1;                      // the last blob whose first group is <= g holds g
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (blob_groups[mid] <= g) lo = mid; else hi = mid - 1;
+        }
+        const long long g0 = blob_groups[lo], start = blob_starts[lo];
+        const long long data = start + 2 * (blob_groups[lo + 1] - g0);   // the blob's group data
+        const long long excl = dst[g] - (start - 2 * g0);                // words of the blob's groups before g
+        const unsigned long long e = (unsigned long long)(excl + sizes[g]);
+        const long long w = start + 2 * (g - g0);
+        if (w + 1 < out_words) {
+            out[w] = (unsigned short)(e & 0xffffu);
+            out[w + 1] = (unsigned short)(e >> 16);
+        }
+        dst[g] = data + excl;
+    }
+}
+
+// One CTA per group of vbq_rans_encode_batch: move its words from the end of its scratch range to their place in the
+// payload.  A group of size 0 (no unit, or a bad one) moves nothing; the clamps keep every access inside the scratch
+// and the payload even when duplicate units of one group left the size of one and the scratch end of another.
+__global__ void vbq_rans_encode_batch_compact_kernel(const unsigned short *__restrict__ scratch,
+                                                     const long long *__restrict__ sizes,
+                                                     const long long *__restrict__ ends,
+                                                     const long long *__restrict__ dst,
+                                                     unsigned short *__restrict__ out, long long out_words) {
+    const long long g = blockIdx.x;
+    const long long size = sizes[g];
+    if (size <= 0) return;                           // ends[g] is written together with a nonzero size
+    const long long end = ends[g], d = dst[g];
+    const long long n = min(size, end);
+    if (d < 0) return;
+    const unsigned short *src = scratch + end - n;
+    const long long m = min(n, out_words - d);
+    for (long long i = threadIdx.x; i < m; i += blockDim.x) out[d + i] = src[i];
 }
 
 constexpr int kDecBlock = 8;   // rows per unrolled block; z_hat gathers of a block are stored one block later
@@ -1186,6 +1327,70 @@ extern "C" int vbq_rans_decode_batch(const unsigned short *d_payload, long long 
     vbq_rans_decode_batch_kernel<<<(unsigned)n_ctas, kRansWarps * 32, smem, st>>>(
         d_payload, payload_words, d_cum, d_prob_bits, n_tables, C, Q, d_units, n_units, d_ctas, n_blobs,
         d_code_points, n_out, d_qidx, d_zhat, d_status);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+extern "C" long long vbq_rans_encode_batch_workspace_bytes(long long n_groups, long long scratch_words) {
+    if (n_groups < 0 || n_groups > 2147483647ll || scratch_words < 0 || scratch_words > (1ll << 60)) return -1;
+    return 3 * align256(8 * n_groups) + align256(2 * scratch_words);
+}
+
+extern "C" int vbq_rans_encode_batch(const int *d_in, long long n_in, const unsigned short *d_cum,
+                                     const int *d_prob_bits, int n_tables, int C, int N,
+                                     const vbq_rans_encode_unit *d_units, long long n_units,
+                                     const vbq_rans_batch_cta *d_ctas, long long n_ctas,
+                                     const long long *d_blob_groups, int n_blobs, long long n_groups,
+                                     unsigned short *d_payload, long long payload_words, long long *d_blob_starts,
+                                     int *d_status, void *d_workspace, long long workspace_bytes, void *stream) {
+    if (N < 0 || N > 10) return vbq_fail(VBQ_ERR_BAD_DEPTH, "vbq_rans_encode_batch: N=%d (the coder holds N <= 10)", N);
+    if (n_in < 0 || n_tables < 0 || C < 1 || C > 32 * 65535 || n_units < 0 || n_ctas < 0 || n_ctas > 2147483647ll ||
+        n_blobs < 0 || n_groups < 0 || n_groups > 2147483647ll || payload_words < 0 || workspace_bytes < 0 ||
+        (n_groups > 0 && n_blobs < 1) || (n_ctas > 0 && (n_units < 1 || n_tables < 1 || n_groups < 1)))
+        return vbq_fail(VBQ_ERR_BAD_SHAPE, "vbq_rans_encode_batch: n_in=%lld n_tables=%d C=%d n_units=%lld n_ctas=%lld "
+                        "n_blobs=%d n_groups=%lld payload_words=%lld workspace_bytes=%lld", n_in, n_tables, C, n_units,
+                        n_ctas, n_blobs, n_groups, payload_words, workspace_bytes);
+    const bool work = n_ctas > 0, groups = n_groups > 0;
+    if (!d_blob_starts || (n_blobs > 0 && !d_status) || (groups && (!d_blob_groups || !d_payload || !d_workspace)) ||
+        (work && (!d_in || !d_cum || !d_prob_bits || !d_units || !d_ctas)))
+        return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_rans_encode_batch: null pointer");
+    if (((uintptr_t)d_in & 3) || ((uintptr_t)d_cum & 1) || ((uintptr_t)d_prob_bits & 3) || ((uintptr_t)d_units & 7) ||
+        ((uintptr_t)d_ctas & 7) || ((uintptr_t)d_blob_groups & 7) || ((uintptr_t)d_payload & 1) ||
+        ((uintptr_t)d_blob_starts & 7) || ((uintptr_t)d_status & 3) || ((uintptr_t)d_workspace & 7))
+        return vbq_fail(VBQ_ERR_MISALIGNED, "vbq_rans_encode_batch: misaligned pointer");
+    const long long index_bytes = 3 * align256(8 * n_groups);
+    if (groups && workspace_bytes < index_bytes)
+        return vbq_fail(VBQ_ERR_WORKSPACE, "vbq_rans_encode_batch: workspace %lld < %lld bytes for %lld groups",
+                        workspace_bytes, index_bytes, n_groups);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (n_blobs > 0) CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int) * (size_t)n_blobs, st));
+    if (!groups) {
+        CUDA_TRY(cudaMemsetAsync(d_blob_starts, 0, sizeof(long long) * ((size_t)n_blobs + 1), st));
+        return VBQ_OK;
+    }
+    char *ws = (char *)d_workspace;
+    long long *sizes = (long long *)ws;
+    long long *ends = (long long *)(ws + align256(8 * n_groups));
+    long long *dst = (long long *)(ws + 2 * align256(8 * n_groups));
+    unsigned short *scratch = (unsigned short *)(ws + index_bytes);
+    const long long scratch_words = (workspace_bytes - index_bytes) / 2;
+    CUDA_TRY(cudaMemsetAsync(sizes, 0, 8 * (size_t)n_groups, st));
+    if (work) {
+        int dev = 0, sms = 0;
+        RETURN_IF(vbq_current_device(&dev, &sms));
+        const int Q = (1 << (N + 1)) - 1;
+        const size_t smem = (size_t)32 * Q * sizeof(unsigned short);
+        VBQ_ENSURE_MAX_SMEM(vbq_rans_encode_batch_kernel, dev);
+        vbq_rans_encode_batch_kernel<<<(unsigned)n_ctas, kRansWarps * 32, smem, st>>>(
+            d_in, n_in, d_cum, d_prob_bits, n_tables, C, Q, d_units, n_units, d_ctas, n_blobs, n_groups, scratch,
+            scratch_words, sizes, ends, d_status);
+        CUDA_TRY(cudaGetLastError());
+    }
+    vbq_rans_encode_batch_scan_kernel<<<1, 1024, 0, st>>>(sizes, dst, n_groups, d_blob_groups, n_blobs, d_payload,
+                                                          payload_words, d_blob_starts, d_status);
+    CUDA_TRY(cudaGetLastError());
+    vbq_rans_encode_batch_compact_kernel<<<(unsigned)n_groups, 256, 0, st>>>(scratch, sizes, ends, dst, d_payload,
+                                                                             payload_words);
     CUDA_TRY(cudaGetLastError());
     return VBQ_OK;
 }

@@ -687,6 +687,47 @@ def rans_decode_batch(words: torch.Tensor, cum: torch.Tensor, prob_bits: torch.T
     return q, z, status
 
 
+def rans_encode_batch(symbols: torch.Tensor, cum: torch.Tensor, prob_bits: torch.Tensor, units: torch.Tensor,
+                      ctas: torch.Tensor, blob_groups: torch.Tensor, n_groups: int, max_bits: int, scratch_words: int):
+    """The work-list encoder of many images in one launch each of encode, scan and compaction.  symbols: contiguous
+    int32 (read flat); cum (n_tables, C, Q) int16; prob_bits (n_tables,) int32; units (n_units, 7) int64
+    (vbq_rans_encode_unit: in, rows, table, cg, group, scratch, blob), ctas (n_ctas, 4) int64 (vbq_rans_batch_cta) and
+    blob_groups (n_blobs + 1,) int64 (each blob's first group; [n_blobs] = n_groups); scratch_words: the scratch the
+    units' ranges lie in.  Returns (payload, meta): the int16 payload of 2 n_groups + scratch_words words, and one int64
+    device tensor meta holding the n_blobs + 1 blob starts (blob b is payload words [meta[b], meta[b + 1])) followed by
+    the (n_blobs,) int32 status per blob (bit 1: a symbol outside [0, Q), bit 8: a bad unit), so that one copy brings
+    both to the host.  No synchronisation."""
+    for name, t, dt, nd in (("symbols", symbols, torch.int32, None), ("cum", cum, torch.int16, 3),
+                            ("prob_bits", prob_bits, torch.int32, 1), ("units", units, torch.int64, 2),
+                            ("ctas", ctas, torch.int64, 2), ("blob_groups", blob_groups, torch.int64, 1)):
+        _need_cuda(name, t, dt, nd)
+    if units.shape[1] != BATCH_UNIT_FIELDS or ctas.shape[1] != BATCH_CTA_FIELDS:
+        raise ValueError("vbq_b200: `units` must be (n, %d) and `ctas` (n, %d), got %s and %s" % (
+            BATCH_UNIT_FIELDS, BATCH_CTA_FIELDS, tuple(units.shape), tuple(ctas.shape)))
+    n_tables, C, _ = cum.shape
+    if prob_bits.numel() != n_tables:
+        raise ValueError("vbq_b200: %d prob_bits for %d tables" % (prob_bits.numel(), n_tables))
+    n_blobs = blob_groups.numel() - 1
+    if n_blobs < 0:
+        raise ValueError("vbq_b200: `blob_groups` needs n_blobs + 1 >= 1 entries")
+    lib = _lib.load()
+    dev = symbols.device
+    ws_bytes = lib.vbq_rans_encode_batch_workspace_bytes(n_groups, scratch_words)
+    if ws_bytes < 0:
+        raise ValueError("vbq_b200: bad batch encode size: %d groups, %d scratch words" % (n_groups, scratch_words))
+    payload_words = 2 * n_groups + scratch_words
+    payload = torch.empty(max(1, payload_words), dtype=torch.int16, device=dev)
+    meta = torch.empty(n_blobs + 1 + (n_blobs + 1) // 2, dtype=torch.int64, device=dev)
+    status = meta[n_blobs + 1:].view(torch.int32)
+    ws = torch.empty(max(1, ws_bytes), dtype=torch.uint8, device=dev)
+    st = lib.vbq_rans_encode_batch(_ptr(symbols), symbols.numel(), _ptr(cum), _ptr(prob_bits), n_tables, C, max_bits,
+                                   _ptr(units), units.shape[0], _ptr(ctas), ctas.shape[0], _ptr(blob_groups), n_blobs,
+                                   n_groups, payload.data_ptr(), payload_words, meta.data_ptr(), _ptr(status),
+                                   ws.data_ptr(), ws_bytes, _stream(dev))
+    _lib.check(st, "vbq_rans_encode_batch")
+    return payload, meta
+
+
 # ------------------------------------------------------------------------------------------------------
 # entropy coding with one shared table per plane, symbols as one flat sequence (word embeddings; include/vbq_b200.h)
 # ------------------------------------------------------------------------------------------------------

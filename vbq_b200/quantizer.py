@@ -418,6 +418,50 @@ class ChannelwisePriorCDFQuantizer:
                                        lambdas=lambs, height=height)
         return {lamb: blobs[i] for i, lamb in enumerate(lambs)}
 
+    def compress_many(self, posterior_means, posterior_logvars, lambs, prob_bits=coding.DEFAULT_PROB_BITS,
+                      seg_rows=None):
+        """`compress_to_bytes` of many images of any shapes in one quantize call and one `serialize.encode_many`:
+        posterior_means / posterior_logvars are lists of (H'_b, W'_b, C) or (1, H'_b, W'_b, C) arrays or tensors, on
+        the host or the device.  Returns {lambda: [bytes of image b]}, each blob byte-identical to
+        `compress_to_bytes(means[b][None], logvars[b][None], lambs, prob_bits, seg_rows)[lambda][0]`, so
+        `decompress_many` of the blobs gives each image's `compress_latents` z_hat.  An empty list gives
+        {lambda: []}; a wrong C raises ValueError."""
+        if self.entropy_models is None:
+            raise TypeError("'NoneType' object is not subscriptable: entropy_models not built "
+                            "(call build_entropy_models first)")
+        means, logvars = list(posterior_means), list(posterior_logvars)
+        if len(means) != len(logvars):
+            raise ValueError("vbq_b200: %d means for %d logvars" % (len(means), len(logvars)))
+        if not means:
+            return {lamb: [] for lamb in lambs}
+        C = self.num_channels
+        shapes = []
+        image = lambda s: s[1:] if len(s) == 4 and s[0] == 1 else s
+        for b, (m, v) in enumerate(zip(means, logvars)):
+            s = image(tuple(m.shape))
+            if len(s) != 3 or s[-1] != C or image(tuple(v.shape)) != s:
+                raise ValueError("vbq_b200: image %d has means %s and logvars %s, need (H', W', %d) or (1, H', W', %d)"
+                                 % (b, tuple(m.shape), tuple(v.shape), C, C))
+            shapes.append(s)
+        qidx = self.quantize(self._rows_of(means), self._rows_of(logvars), lambs, logvar=True,
+                             outputs=ops.OUT_QIDX)['qidx']
+        tables = [self.rans_tables(l, prob_bits) for l in lambs]
+        blobs = serialize.encode_many(qidx, tables, self.max_bits_per_coord, [h * w for h, w, _ in shapes],
+                                      seg_rows=seg_rows, lambdas=lambs, heights=[h for h, _, _ in shapes])
+        return {lamb: blobs[i] for i, lamb in enumerate(lambs)}
+
+    def _rows_of(self, xs):
+        """Latents of many images as one (rows, C) float32 device tensor, their rows back to back: each image is
+        copied straight into its rows (no host-side concatenation)."""
+        C = self.num_channels
+        parts = [torch.as_tensor(x).reshape(-1, C) for x in xs]
+        out = torch.empty((sum(p.shape[0] for p in parts), C), dtype=torch.float32, device=self.device)
+        r = 0
+        for p in parts:
+            out[r:r + p.shape[0]].copy_(p)
+            r += p.shape[0]
+        return out
+
     def decompress_from_bytes(self, blob):
         """z_hat of a `compress_to_bytes` blob as a device tensor (1, H', W', C) (several items or planes stack on the
         first axis).  The blob's lambda selects the entropy model by float equality, as the dict keys do."""

@@ -31,7 +31,7 @@ import struct
 import numpy as np
 import torch
 
-from . import coding, ops
+from . import coding, ops, utils
 
 MAGIC = b"VBQ1"
 _HDR = struct.Struct("<4sIIIIQ")
@@ -348,9 +348,18 @@ def batch_plan(headers, payloads, table_ids):
     tids = np.array([t for ids in table_ids for t in ids], dtype=np.int64)
     table = tids[(np.cumsum(L) - L)[blob] + plane]
     units = np.stack([bounds[:, 0], bounds[:, 1], out, rows, table, cg, blob], axis=1)
+    units, ctas = _into_ctas(units, table, cg, CG)
+    words = np.concatenate(payloads) if B else np.zeros(0, np.uint16)
+    return dict(words=words, units=units, ctas=ctas, offsets=offsets, sizes=sizes, n_out=int(sizes.sum()))
+
+
+def _into_ctas(units, table, cg, CG):
+    """Units (rows of an int64 array) sorted stably by (table, cg), and the CTA descriptors (K, 4) int64 (first, count,
+    table, cg) that take up to BATCH_CTA_UNITS consecutive units of one (table, cg) each."""
     U = units.shape[0]
-    units = units[np.lexsort((np.arange(U), cg, table))]
-    key = units[:, 4] * CG + units[:, 5]
+    order = np.lexsort((np.arange(U), cg, table))
+    units, table, cg = units[order], table[order], cg[order]
+    key = table * CG + cg
     new_run = np.ones(U, bool)
     new_run[1:] = key[1:] != key[:-1]
     run_starts = np.flatnonzero(new_run)
@@ -359,10 +368,8 @@ def batch_plan(headers, payloads, table_ids):
     first = np.flatnonzero(pos % BATCH_CTA_UNITS == 0)
     run_ends = np.append(run_starts[1:], U)
     count = np.minimum(BATCH_CTA_UNITS, run_ends[run[first]] - first)
-    ctas = np.stack([first, count, units[first, 4], units[first, 5]], axis=1).astype(np.int64)
-    words = np.concatenate(payloads) if B else np.zeros(0, np.uint16)
-    return dict(words=words, units=np.ascontiguousarray(units), ctas=ctas, offsets=offsets, sizes=sizes,
-                n_out=int(sizes.sum()))
+    ctas = np.stack([first, count, table[first], cg[first]], axis=1).astype(np.int64)
+    return np.ascontiguousarray(units), ctas
 
 
 def _resolve_tables(h, tables, b):
@@ -454,6 +461,137 @@ def decode_many(blobs, tables=None, code_points=None, device="cuda", want_qidx: 
     headers = [read_header(d) for d in blobs]
     plane_tables = [_resolve_tables(h, tables, b) for b, h in enumerate(headers)]
     return decode_blobs(blobs, headers, plane_tables, code_points, device, want_qidx)[0]
+
+
+# ------------------------------------------------------------------------------------------------------
+# many images in one launch (vbq_rans_encode_batch)
+# ------------------------------------------------------------------------------------------------------
+def encode_plan(item_rows, seg_rows, C: int, table_ids) -> dict:
+    """The work list of `encode_many` (host only), the mirror of `batch_plan`.  item_rows: (B,) rows of each image, the
+    images back to back in each of the L = len(table_ids) planes; seg_rows: rows per segment (None: the whole image);
+    table_ids: the table index of each plane.  Blob p B + b is image b of plane p, its groups in (segment, cg) order.
+    Returns dict(units (U, 7) int64 (vbq_rans_encode_unit: in, rows, table, cg, group, scratch, blob) sorted stably by
+    (table, cg), ctas (K, 4) int64 (vbq_rans_batch_cta), blob_groups (L B + 1,) int64, seg (B,) the seg_rows each blob
+    records, n_groups, scratch_words (every unit its own range of nact (rows + 2) words) and payload_words, the
+    payload bound 2 n_groups + scratch_words).  Raises ValueError for an image whose worst case exceeds the 32-bit
+    offset table."""
+    R = np.asarray(item_rows, dtype=np.int64).reshape(-1)
+    tids = np.asarray(table_ids, dtype=np.int64).reshape(-1)
+    B, L, CG = R.size, tids.size, -(-C // 32)
+    seg = np.maximum(1, R if seg_rows is None else np.full(B, int(seg_rows), np.int64))
+    n_segs = -(-R // seg)
+    worst = C * (R + 2 * n_segs)                   # an image's group data if every lane emitted a word on every row
+    if (worst >= 2 ** 32).any():
+        b = int(np.flatnonzero(worst >= 2 ** 32)[0])
+        raise ValueError("vbq_b200.serialize: image %d of %d rows x %d channels in segments of %d rows exceeds the "
+                         "32-bit offset table" % (b, R[b], C, seg[b]))
+    row0 = np.cumsum(R) - R
+    G = np.tile(n_segs * CG, L)                    # groups of blob p B + b
+    blob_groups = np.concatenate([[0], np.cumsum(G)]).astype(np.int64)
+    n_groups = int(blob_groups[-1])
+    blob = np.repeat(np.arange(L * B, dtype=np.int64), G)
+    g = np.arange(n_groups, dtype=np.int64)
+    local = g - blob_groups[blob]
+    cg = local % CG
+    plane, b = blob // max(B, 1), blob % max(B, 1)
+    r0 = (local // CG) * seg[b]
+    rows = np.minimum(seg[b], R[b] - r0)
+    nact = np.minimum(32, C - 32 * cg)
+    words = nact * (rows + 2)
+    scratch = np.cumsum(words) - words
+    table = tids[plane]
+    units = np.stack([(plane * int(R.sum()) + row0[b] + r0) * C + 32 * cg, rows, table, cg, g, scratch, blob], axis=1)
+    units, ctas = _into_ctas(units.astype(np.int64), table, cg, CG)
+    scratch_words = int(words.sum())
+    return dict(units=units, ctas=ctas, blob_groups=blob_groups, seg=seg, n_groups=n_groups,
+                scratch_words=scratch_words, payload_words=2 * n_groups + scratch_words)
+
+
+def encode_many(qidx, tables, max_bits: int, item_rows, seg_rows=None, lambdas=None, heights=None) -> list:
+    """Entropy-code many images of different shapes in one launch each of encode, scan and compaction: one VBQ2 blob
+    per (plane, image), as a list over planes of lists over images of bytes.
+
+    qidx: (L, total_rows, C) int32 CUDA tensor (what `quantize` returns for images concatenated row-wise).  tables: one
+    (C, Q) integer table per plane (an (L, C, Q) array, a (C, Q) array for every plane, or a sequence); planes may
+    differ in prob_bits.  item_rows: each image's row count.  seg_rows: rows per coded segment (default: the whole
+    image).  lambdas: the plane labels (default 0.0).  heights: each image's H' (default 0, unknown).  Blob [p][b] is
+    byte-identical to `encode_items(qidx[p:p+1, rows of image b], tables[p], max_bits, items=1, seg_rows=seg_rows,
+    lambdas=[lambdas[p]], height=heights[b])[0][0]`.
+
+    Every table is checked and fingerprinted once.  Item rows that do not sum to the rows, a height that does not
+    divide its image's rows and tables of the wrong shape raise ValueError before any launch.  The call synchronises
+    with the host twice: once for one copy of the blob starts and statuses, and once for the copy of the payload.  A
+    symbol outside [0, Q) raises ValueError naming the images it lies in."""
+    q = qidx if qidx.dim() == 3 else qidx.unsqueeze(0)
+    L, rows, C = q.shape
+    R = np.asarray(item_rows, dtype=np.int64).reshape(-1)
+    B = R.size
+    if (R < 0).any() or int(R.sum()) != rows:
+        raise ValueError("vbq_b200.serialize: item_rows %s do not sum to the %d rows" % (R.tolist(), rows))
+    hs = np.zeros(B, np.int64) if heights is None else np.asarray(heights, dtype=np.int64).reshape(-1)
+    if hs.size != B:
+        raise ValueError("vbq_b200.serialize: %d heights for %d images" % (hs.size, B))
+    for b in np.flatnonzero((hs < 0) | ((hs > 0) & (R % np.maximum(hs, 1) != 0))):
+        raise ValueError("vbq_b200.serialize: height %d does not divide the %d rows of image %d" % (hs[b], R[b], b))
+    lam = _lambdas(lambdas, L)
+    Q = ops.num_levels(max_bits)
+    if isinstance(tables, (list, tuple)):
+        if len(tables) != L:
+            raise ValueError("vbq_b200.serialize: %d tables for %d planes" % (len(tables), L))
+        keyed = [(id(t), t) for t in tables]
+    elif np.ndim(tables) == 2:
+        keyed = [(id(tables), tables)] * L
+    else:
+        t = _as_tables(tables, L)
+        keyed = [((id(tables), p), t[p]) for p in range(L)]
+    ids, distinct, table_ids = {}, [], []
+    for p, (key, table) in enumerate(keyed):
+        if key not in ids:
+            t = np.asarray(table)
+            if t.shape != (C, Q):
+                raise ValueError("vbq_b200.serialize: the table of plane %d is %s, need (C, Q) = (%d, %d)"
+                                 % (p, t.shape, C, Q))
+            P = coding.prob_bits_of(t)
+            ids[key] = len(distinct)
+            distinct.append((coding.check_tables(t, P), coding.fingerprint(t), P))
+        table_ids.append(ids[key])
+    plan = encode_plan(R, seg_rows, C, table_ids)
+    if B == 0:
+        return [[] for _ in range(L)]
+    dev = q.device
+    U, K, LB = plan["units"].shape[0], plan["ctas"].shape[0], L * B
+    index = torch.from_numpy(np.concatenate([plan["units"].reshape(-1), plan["ctas"].reshape(-1),
+                                             plan["blob_groups"]])).to(dev)      # one upload for the work list
+    units = index[:7 * U].view(U, 7)
+    ctas = index[7 * U:7 * U + 4 * K].view(K, 4)
+    cum = torch.from_numpy(np.stack([coding.cum_table(t) for t, _, _ in distinct]).view(np.int16)).to(dev)
+    pb = torch.tensor([P for _, _, P in distinct], dtype=torch.int32).to(dev)
+    payload, meta = ops.rans_encode_batch(q.contiguous(), cum, pb, units, ctas, index[7 * U + 4 * K:],
+                                          plan["n_groups"], max_bits, plan["scratch_words"])
+    m = utils.to_host_numpy(meta)
+    starts, status = m[:LB + 1], m[LB + 1:].view(np.int32)[:LB]
+    bad = np.flatnonzero(status)
+    if bad.size:
+        where = "; ".join("image %d of plane %d (lambda %r): %s" % (i % B, i // B, lam[i // B],
+                                                                   _encode_status_text(int(status[i]))) for i in bad)
+        raise ValueError("vbq_b200.serialize: cannot encode image%s %s for max_bits=%d (%s)" % (
+            "s" if len(set((bad % B).tolist())) > 1 else "", ", ".join(str(b) for b in sorted(set((bad % B).tolist()))),
+            max_bits, where))
+    words = utils.to_host_numpy(payload[:int(starts[-1])]).view(np.uint16).astype("<u2", copy=False)
+    out = []
+    for p in range(L):
+        _, fp, P = distinct[table_ids[p]]
+        blobs = []
+        for b in range(B):
+            f = dict(N=max_bits, C=C, P=P, n_planes=1, items=1, item_rows=int(R[b]), seg_rows=int(plan["seg"][b]))
+            i = p * B + b
+            blobs.append(b"".join(_header(f, [lam[p]], [fp], int(hs[b]))) + words[starts[i]:starts[i + 1]].tobytes())
+        out.append(blobs)
+    return out
+
+
+def _encode_status_text(st):
+    return ", ".join(m for bit, m in ((1, "a symbol lies outside [0, Q)"), (8, "bad work unit")) if st & bit)
 
 
 # ------------------------------------------------------------------------------------------------------
