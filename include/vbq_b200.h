@@ -513,6 +513,25 @@ int vbq_pair_scores(const float *d_rows, long long n_rows, long long row_size, c
                     long long n_queries, const long long *d_pair_rows, const long long *d_pair_queries,
                     long long n_pairs, int metric, float *d_scores, void *stream);
 
+/* ---- image quality: exact SSE and MS-SSIM levels (DESIGN.md §8j) -------------------------------------------------
+ *
+ * d_x (N, H, W, C) uint8 are N originals and d_y (M, N, H, W, C) uint8 are M reconstructions of each (1 <= C <= 4).
+ * For every pair (m, n), vbq_image_metrics writes d_sse[m, n] (M, N) int64 = the exact sum over H W C of
+ * (x - y)^2, and d_ssim[m, n, k] / d_cs[m, n, k] (M, N, 5) float64 = the means of ssim and cs at pyramid level k of
+ * TF models' MultiScaleSSIM with max_val 255 (k1 = 0.01, k2 = 0.03): level k + 1 is the 2 x 2 mean of level k with
+ * the last row or column repeated at an odd size; at each level the window is _FSpecialGauss(s, 1.5 s / 11) with
+ * s = min(11, h, w), the moments are filtered over the valid positions, and the means run over all valid positions
+ * and all channels.  The moments are computed in float64 with a separable window (agreeing with the reference's FFT
+ * filtering to about 1e-14 relative); the sums over positions run in a fixed order, so two calls give the same bits.
+ * MS-SSIM = prod_k<4 cs[k]^w[k] * ssim[4]^w[4] and PSNR are left to the caller.
+ * d_workspace: vbq_image_metrics_workspace_bytes(N, M, H, W, C) bytes, 16-byte aligned (-1 for a bad shape).
+ * N = 0 or M = 0 is no work.  Status codes: VBQ_ERR_BAD_SHAPE for a bad size, VBQ_ERR_WORKSPACE for a workspace
+ * missing or too small. */
+long long vbq_image_metrics_workspace_bytes(long long N, long long M, int H, int W, int C);
+int vbq_image_metrics(const unsigned char *d_x, const unsigned char *d_y, long long N, long long M, int H, int W,
+                      int C, void *d_workspace, long long workspace_bytes, long long *d_sse, double *d_ssim,
+                      double *d_cs, void *stream);
+
 /* ---- stand-alone operator forms------------------------------------------------------------------------------- */
 
 /* ChannelwisePriorCDFQuantizer.get_all_N_bit_intervals (quantizer.py:65-80): d_mu (rows, C) -> d_left, d_right

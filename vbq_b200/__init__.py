@@ -12,8 +12,9 @@ from .learned_prior import BMSHJ2018Prior                            # noqa: E40
 from .vae_models import StandardGaussianPrior, FactoredGaussianPrior, GaussianVAE   # noqa: E402
 from .word_embeddings import GaussianCodebook, CompressedEmbedding   # noqa: E402
 from .word_embeddings import ranks, analogy_ranks, analogy_metrics   # noqa: E402
-from .evaluation import evaluate_compression_quantizer               # noqa: E402
+from .evaluation import evaluate_compression_quantizer, image_metrics  # noqa: E402
 
 __all__ = ["ops", "utils", "sharding", "serialize", "ChannelwisePriorCDFQuantizer", "BMSHJ2018Prior",
            "StandardGaussianPrior", "FactoredGaussianPrior", "GaussianVAE", "GaussianCodebook", "CompressedEmbedding",
-           "ranks", "analogy_ranks", "analogy_metrics", "evaluate_compression_quantizer"]
+           "ranks", "analogy_ranks", "analogy_metrics", "evaluate_compression_quantizer",
+           "image_metrics"]

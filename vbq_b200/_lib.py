@@ -29,6 +29,8 @@ MAX_DEPTH = 20
 RANS_SHARED_MAX_PLANES = 64
 SCORE_DOT = 0
 SCORE_COSINE = 1
+IMAGE_METRICS_LEVELS = 5
+IMAGE_METRICS_MAX_CHANNELS = 4
 
 
 class VbqError(RuntimeError):
@@ -100,6 +102,8 @@ SIGNATURES = {
                                         _p, _p, _p]),
     "vbq_score_ranks": (_i, [_p, _ll, _ll, _ll, _p, _ll, _i, _p, _p, _p, _p]),
     "vbq_pair_scores": (_i, [_p, _ll, _ll, _p, _ll, _p, _p, _ll, _i, _p, _p]),
+    "vbq_image_metrics_workspace_bytes": (_ll, [_ll, _ll, _i, _i, _i]),
+    "vbq_image_metrics": (_i, [_p, _p, _ll, _ll, _i, _i, _i, _p, _ll, _p, _p, _p, _p]),
 }
 
 _lib = None

@@ -8,7 +8,7 @@ import subprocess
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 REPO_DIR = os.path.dirname(PKG_DIR)
 SOURCES = [os.path.join(PKG_DIR, "csrc", f) for f in ("api.cu", "priors.cu", "quantize.cu", "quantize_strict.cu", "quantize_reference.cu", "quantize_fast.cu", "quantize_bisect.cu", "quantize_tma.cu", "quantize_tma_both.cu", "sweep_bisect.cu", "sweep_both.cu",
-            "sweep.cu", "host_pipeline.cu", "operators.cu", "embeddings.cu", "serialize.cu", "rans.cu", "ranks.cu", "peer.cu")]
+            "sweep.cu", "host_pipeline.cu", "operators.cu", "embeddings.cu", "serialize.cu", "rans.cu", "ranks.cu", "image_metrics.cu", "peer.cu")]
 HEADERS = [os.path.join(REPO_DIR, "include", "vbq_b200.h"), os.path.join(PKG_DIR, "csrc", "common.h"),
            os.path.join(PKG_DIR, "csrc", "tree.cuh"),
            os.path.join(PKG_DIR, "csrc", "quantize_kernel.cuh"), os.path.join(PKG_DIR, "csrc", "bisect.cuh"), os.path.join(PKG_DIR, "csrc", "tma.cuh"), os.path.join(PKG_DIR, "csrc", "quantize_tma.cuh")]

@@ -942,3 +942,36 @@ def pair_scores(rows: torch.Tensor, queries: torch.Tensor, pair_rows: torch.Tens
                                      _ptr(out), _stream(rows.device))
     _lib.check(st, "vbq_pair_scores")
     return out
+
+
+# image quality: exact SSE and the MS-SSIM levels (include/vbq_b200.h, vbq_image_metrics)
+# ---------------------------------------------------------------------------------------
+def image_metrics(originals: torch.Tensor, reconstructions: torch.Tensor):
+    """originals (N, H, W, C) uint8 and reconstructions (M, N, H, W, C) uint8 on one CUDA device ->
+    (sse (M, N) int64, ssim (M, N, 5) float64, cs (M, N, 5) float64): the exact sum of squared errors and the per-level
+    means of MultiScaleSSIM's ssim and cs.  No synchronisation."""
+    _need_cuda("originals", originals, torch.uint8, 4)
+    _need_cuda("reconstructions", reconstructions, torch.uint8, 5)
+    if tuple(reconstructions.shape[1:]) != tuple(originals.shape) or reconstructions.device != originals.device:
+        raise ValueError("vbq_b200: image_metrics shapes: originals %s on %s, reconstructions %s on %s"
+                         % (tuple(originals.shape), originals.device, tuple(reconstructions.shape),
+                            reconstructions.device))
+    N, H, W, C = originals.shape
+    M = reconstructions.shape[0]
+    lib = _lib.load()
+    nbytes = lib.vbq_image_metrics_workspace_bytes(N, M, H, W, C)
+    if nbytes < 0:
+        raise ValueError("vbq_b200: image_metrics cannot take images of shape %s (1 <= C <= %d, H W C < 2^31)"
+                         % (tuple(originals.shape), _lib.IMAGE_METRICS_MAX_CHANNELS))
+    dev = originals.device
+    L = _lib.IMAGE_METRICS_LEVELS
+    sse = torch.empty((M, N), dtype=torch.int64, device=dev)
+    ssim = torch.empty((M, N, L), dtype=torch.float64, device=dev)
+    cs = torch.empty((M, N, L), dtype=torch.float64, device=dev)
+    if M * N == 0:
+        return sse, ssim, cs
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    st = lib.vbq_image_metrics(_ptr(originals), _ptr(reconstructions), N, M, H, W, C, _ptr(ws), nbytes, _ptr(sse),
+                               _ptr(ssim), _ptr(cs), _stream(dev))
+    _lib.check(st, "vbq_image_metrics")
+    return sse, ssim, cs
