@@ -552,6 +552,10 @@ int vbq_argmax_candidates(const float *d_P, const void *d_L, int l_is_float, int
  * compare it with IEEE division bit for bit. */
 int vbq_selftest_divide(const float *d_a, const float *d_b, long long n, float *d_out, void *stream);
 
+/* Self-test helper: out[i] = the sigma every search kernel derives from a log-variance input lv[i] under
+ * VBQ_FLAG_LOGVAR (sqrt(exp(lv)) with CUDA's expf and sqrtf), so that tests can hand the oracle the kernels' sigma. */
+int vbq_selftest_sigma_from_logvar(const float *d_lv, long long n, float *d_out, void *stream);
+
 /* Self-test helper (host only): out[b] .. out[b+1] is the range of 4-row x 16-channel tiles, in (channel group, row)
  * order, that CTA b of a `grid`-CTA launch of the bisection kernels processes; out has grid+1 entries. */
 int vbq_selftest_span_cuts(long long rows, int C, int grid, long long *out);

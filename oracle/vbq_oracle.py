@@ -391,11 +391,20 @@ class QuantizerNP:
             I[:, c] = np.searchsorted(self.code_points_by_channel[c], Z_hat[:, c], side="left")
         return I
 
+    def _stds(self, posterior_logvars, posterior_stds):
+        """(rows, C) float32 sigma: exp(logvar) ** 0.5 in float32 (quantizer.py:93, :198), or the given stds."""
+        if posterior_stds is not None:
+            return np.asarray(posterior_stds, dtype=F32).reshape(-1, self.C)
+        return np.exp(np.asarray(posterior_logvars, dtype=F32)).reshape(-1, self.C) ** F32(0.5)
+
     # quantizer.py:82-150, given latents instead of (X, vae)
-    def build_entropy_models_from_latents(self, posterior_means, posterior_logvars, lambs, add_n_smoothing):
+    def build_entropy_models_from_latents(self, posterior_means, posterior_logvars, lambs, add_n_smoothing,
+                                          posterior_stds=None):
+        """``posterior_stds`` (optional) replaces ``posterior_logvars`` by ready-made standard deviations, as the
+        facade's parameter of the same name does (e.g. the sigma the kernels derive from the log-variances)."""
         N, C = self.N, self.C
         means = np.asarray(posterior_means, dtype=F32).reshape(-1, C)
-        stds = np.exp(np.asarray(posterior_logvars, dtype=F32)).reshape(-1, C) ** F32(0.5)
+        stds = self._stds(posterior_logvars, posterior_stds)
         self.raw_code_length_entropy_models = None
         _, raw_bits = self.compress_batch_channel_latents(means, stds, lambs)
         rcl = {}
@@ -417,12 +426,13 @@ class QuantizerNP:
         self.entropy_models = em
 
     # quantizer.py:190-240
-    def compress_latents(self, posterior_means, posterior_logvars, lambs):
+    def compress_latents(self, posterior_means, posterior_logvars, lambs, posterior_stds=None):
+        """``posterior_stds``: as in `build_entropy_models_from_latents`."""
         C = self.C
         pm = np.asarray(posterior_means, dtype=F32)
         assert pm.shape[-1] == C
         means = pm.reshape(-1, C)
-        stds = np.exp(np.asarray(posterior_logvars, dtype=F32)).reshape(-1, C) ** F32(0.5)
+        stds = self._stds(posterior_logvars, posterior_stds)
         Z_hat_dict, raw_dict = self.compress_batch_channel_latents(means, stds, lambs)
         keys = ("Z_hat", "raw_num_bits", "num_bits_cl", "num_bits")
         out = {k: {} for k in keys}

@@ -69,6 +69,19 @@ def test_argument_validation_needs_no_gpu():
     assert lib.vbq_pack_code_points(one, 0, 10, one, None) == 2
 
 
+def test_sigma_selftest_validates_without_gpu():
+    """vbq_selftest_sigma_from_logvar rejects null pointers and negative counts, and an empty call is a no-op: all
+    before any device work."""
+    from vbq_b200 import _lib
+    lib = _lib.load()
+    one = ctypes.c_void_p(16)
+    assert lib.vbq_selftest_sigma_from_logvar(None, 8, one, None) == 1
+    assert lib.vbq_selftest_sigma_from_logvar(one, 8, None, None) == 1
+    assert b"vbq_selftest_sigma_from_logvar" in lib.vbq_last_error()
+    assert lib.vbq_selftest_sigma_from_logvar(one, -1, one, None) == 2 and b"n=-1" in lib.vbq_last_error()
+    assert lib.vbq_selftest_sigma_from_logvar(None, 0, None, None) == 0
+
+
 def test_no_cpu_fallback():
     import vbq_b200
     from vbq_b200 import ops

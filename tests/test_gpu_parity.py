@@ -162,15 +162,21 @@ def test_prune_equals_no_prune_large():
 
 
 def test_host_pipeline_matches_device_path():
-    """vbq_quantize_host (chunked upload/kernel/download) == vbq_quantize on the same data, incl. ragged last chunk."""
+    """vbq_quantize_host (chunked upload/kernel/download) == vbq_quantize on the same data, incl. ragged last chunk; with
+    3 lambdas (penalties also on the host) and with 16 lambdas (more than the pipeline's 64 host penalty floats)."""
     import vbq_b200
     from vbq_b200 import ops
     C, N, rows = 40, 10, 5000
-    lambs = [2.0 ** -5, 0.5, 16.0]
     pr = H.make_prior(C, seed=5)
     q = vbq_b200.ChannelwisePriorCDFQuantizer(C, N)
     q.set_code_points(ops.build_code_points_learned(_dev(pr.packed()), N))
     mu, sigma, _ = H.make_latents(pr, rows, 6, table=q.all_code_points.cpu().numpy())
+    for lambs in ([2.0 ** -5, 0.5, 16.0], [float(l) for l in 2.0 ** np.linspace(-8, 6, 16)]):
+        _host_pipeline_case(q, C, N, rows, mu, sigma, lambs)
+
+
+def _host_pipeline_case(q, C, N, rows, mu, sigma, lambs):
+    from vbq_b200 import ops
     want = q.quantize(_dev(mu), _dev(sigma), lambs,
                       outputs=ops.OUT_ZHAT | ops.OUT_QIDX | ops.OUT_LEVEL | ops.OUT_BITS | ops.OUT_TOTALS)
     pen, length = q._length_tables(lambs)

@@ -95,6 +95,32 @@ def test_search_raw_and_corrected_lengths(name):
         assert np.array_equal(np.take_along_axis(q.code_points_by_channel.T, I, axis=0), Zh[l])
 
 
+@pytest.mark.parametrize("name", LEARNED)
+def test_posterior_stds_replace_logvars(name):
+    """posterior_stds= hands the oracle a sigma directly (the GPU tests pass it the kernels' sigma of the log-variances):
+    given the reference's own exp(logvar) ** 0.5 it reproduces the reference bit for bit without the log-variances, and
+    any other sigma is searched as given."""
+    g = load(name)
+    lambs = lambs_of(g)
+    C = int(g["C"])
+    stds = np.exp(g["logvars"].astype(np.float32)) ** np.float32(0.5)
+    q = quantizer_of(g)
+    q.build_entropy_models_from_latents(g["means"], None, lambs, add_n_smoothing=1, posterior_stds=stds)
+    for i, l in enumerate(lambs):
+        assert np.array_equal(q.raw_code_length_entropy_models[l], g["rcl_%d" % i])
+        assert np.array_equal(q.entropy_models[l], g["em_%d" % i])
+    out = q.compress_latents(g["means"], None, lambs, posterior_stds=stds)
+    for i, l in enumerate(lambs):
+        for key in ("Z_hat", "raw_num_bits", "num_bits_cl", "num_bits"):
+            assert np.array_equal(out[key][l], g["compress_%s_%d" % (key, i)]), key
+    wide = (stds * np.float32(3.0)).astype(np.float32)
+    out = q.compress_latents(g["means"], g["logvars"], lambs, posterior_stds=wide)
+    Zh, nb = q.compress_batch_channel_latents(g["means"].reshape(-1, C), wide.reshape(-1, C), lambs)
+    assert any(not np.array_equal(Zh[l], g["cl_zhat_%d" % i]) for i, l in enumerate(lambs))
+    for l in lambs:
+        assert np.array_equal(out["Z_hat"][l].reshape(-1, C), Zh[l]) and np.array_equal(out["raw_num_bits"][l].reshape(-1, C), nb[l])
+
+
 def test_sorted_rank_formula():
     g = load("learned_c6_n10")
     N = int(g["N"])

@@ -76,6 +76,7 @@ SIGNATURES = {
     "vbq_intervals": (_i, [_p, _ll, _i, _p, _i, _p, _p, _p]),
     "vbq_argmax_candidates": (_i, [_p, _p, _i, _i, _p, _p, _p, _p, _i, _i, _ll, _p, _p, _p, _p]),
     "vbq_selftest_divide": (_i, [_p, _p, _ll, _p, _p]),
+    "vbq_selftest_sigma_from_logvar": (_i, [_p, _ll, _p, _p]),
     "vbq_selftest_span_cuts": (_i, [_ll, _i, _i, _p]),
     "vbq_packed_index_words": (_ll, [_ll, _i]),
     "vbq_pack_indices": (_i, [_p, _ll, _i, _p, _p]),

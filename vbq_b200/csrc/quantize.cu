@@ -89,6 +89,11 @@ __global__ void selftest_divide_kernel(const float *__restrict__ x, const float 
         out[t] = div_rn(x[t], y[t], rcp_rn(y[t]));
 }
 
+__global__ void selftest_sigma_kernel(const float *__restrict__ lv, long long n, float *__restrict__ out) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) out[t] = sigma_of_logvar(lv[t]);
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // C ABI
 // ------------------------------------------------------------------------------------------------------------
@@ -275,6 +280,17 @@ extern "C" int vbq_selftest_divide(const float *d_a, const float *d_b, long long
     int grid;
     RETURN_IF(vbq_grid_for(n, 256, &grid));
     selftest_divide_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_a, d_b, n, d_out);
+    CUDA_TRY(cudaGetLastError());
+    return VBQ_OK;
+}
+
+extern "C" int vbq_selftest_sigma_from_logvar(const float *d_lv, long long n, float *d_out, void *stream) {
+    if (n > 0 && (!d_lv || !d_out)) return vbq_fail(VBQ_ERR_NULL_POINTER, "vbq_selftest_sigma_from_logvar: null pointer");
+    if (n < 0) return vbq_fail(VBQ_ERR_BAD_SHAPE, "vbq_selftest_sigma_from_logvar: n=%lld", n);
+    if (n == 0) return VBQ_OK;
+    int grid;
+    RETURN_IF(vbq_grid_for(n, 256, &grid));
+    selftest_sigma_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_lv, n, d_out);
     CUDA_TRY(cudaGetLastError());
     return VBQ_OK;
 }

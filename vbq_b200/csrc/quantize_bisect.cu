@@ -188,7 +188,7 @@ __global__ void __launch_bounds__(kThreads, 1) vbq_bisect_kernel(const QArgs a) 
                 ok[u] = !CHECK || (c_ok && row + 2 * u < rows);
                 mu[u] = ok[u] ? myStage[slot * kTileFloats + u * 2 * VBQ_GROUP] : 0.0f;
                 float s = ok[u] ? myStage[slot * kTileFloats + kTileRows * VBQ_GROUP + u * 2 * VBQ_GROUP] : 1.0f;
-                if (logvar) s = sqrtf(expf(s));
+                if (logvar) s = sigma_of_logvar(s);
                 sg[u] = s;
             }
 #pragma unroll

@@ -170,7 +170,7 @@ __global__ void __launch_bounds__(kThreads, 1) vbq_quantize_kernel(const QArgs a
                 const bool ok = row + u * RP < row_end;
                 mu[u] = ok ? myStage[((slot * 2 + 0) * U + u) * kThreads] : 0.0f;
                 float s = ok ? myStage[((slot * 2 + 1) * U + u) * kThreads] : 1.0f;
-                if (logvar) s = sqrtf(expf(s));
+                if (logvar) s = sigma_of_logvar(s);
                 sg[u] = s;
             }
             {   // refill the slot consumed in the previous iteration

@@ -896,7 +896,7 @@ __global__ void __launch_bounds__(32 * (W + 1), 1)
             for (int u = 0; u < U; ++u) {
                 const bool ok = full || (c_ok && par + 2 * u < my_rows);
                 float m = lds_u32(mine + u * 128), sd = lds_u32(mine + 4 * kSgOff + u * 128);
-                if (logvar) sd = sqrtf(expf(sd));
+                if (logvar) sd = sigma_of_logvar(sd);
                 if (!ok) { m = 0.0f; sd = 1.0f; }
                 sts_u32(mine + u * 128, __float_as_uint(m));
                 sts_u32(mine + 4 * kSgOff + u * 128, __float_as_uint(sd));

@@ -115,7 +115,7 @@ __global__ void __launch_bounds__(kThreads, 1) vbq_sweep_kernel(const QArgs a) {
                 ok[u] = row + u * RP < row_end;
                 mu[u] = ok[u] ? myStage[((slot * 2 + 0) * U + u) * kThreads] : 0.0f;
                 float s = ok[u] ? myStage[((slot * 2 + 1) * U + u) * kThreads] : 1.0f;
-                if (logvar) s = sqrtf(expf(s));
+                if (logvar) s = sigma_of_logvar(s);
                 sg[u] = s;
             }
             {

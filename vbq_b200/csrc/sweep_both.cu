@@ -172,7 +172,7 @@ __global__ void __launch_bounds__(kThreads, 1) vbq_both_sweep_kernel(const QArgs
                 ok[u] = !check || (c_ok && row + 2 * u < rows);
                 mu[u] = ok[u] ? myStage[slot * kTileFloats + u * 2 * VBQ_GROUP] : 0.0f;
                 float s = ok[u] ? myStage[slot * kTileFloats + kTileRows * VBQ_GROUP + u * 2 * VBQ_GROUP] : 1.0f;
-                if (logvar) s = sqrtf(expf(s));
+                if (logvar) s = sigma_of_logvar(s);
                 sg[u] = s;
             }
             const float2 nmu2 = make_float2(-mu[0], -mu[1]);

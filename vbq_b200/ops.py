@@ -402,6 +402,15 @@ def selftest_divide(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def selftest_sigma_from_logvar(lv: torch.Tensor) -> torch.Tensor:
+    """The sigma the search kernels derive from log-variances `lv` (FLAG_LOGVAR), bit for bit."""
+    _need_cuda("lv", lv, torch.float32)
+    out = torch.empty_like(lv)
+    st = _lib.load().vbq_selftest_sigma_from_logvar(_ptr(lv), lv.numel(), _ptr(out), _stream(lv.device))
+    _lib.check(st, "vbq_selftest_sigma_from_logvar")
+    return out
+
+
 # ------------------------------------------------------------------------------------------------------
 # host-resident latents: chunked upload / kernel / download pipeline (vbq_quantize_host)
 # ------------------------------------------------------------------------------------------------------
